@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the fp64 UKF + URTSS hot path on synthetic ship tracks (BASELINE.json configs 3-5).
 
-    python bench.py [--config c5|c3|c4] [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--config c5|c3|c4] [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 ``--config c5`` (default; BASELINE.json configs[4], the one the metric is quoted on): 16 M tracks x
@@ -18,7 +18,9 @@ ragged tracks of 100-5000 fixes, gaps drawn from {1,2,3,6,12,24} h, k = 2 sub-st
 2, 1 % displaced fixes, Mahalanobis gating + URTSS, processed as length-sorted tiles
 (``sharding.plan_ragged_tiles``, dealt round-robin to the ranks).
 
-One JSON line is printed by rank 0; see README / DESIGN.md for the keys.  ``--impl reference``
+One JSON line is printed by rank 0; see README / DESIGN.md for the keys.  ``--dump-outputs DIR`` also writes the
+results of the last timed step (a seeded sample of its tracks) as ``DIR/*.npy``: the inputs are seeded, so two builds
+run with the same arguments can be compared output for output.  ``--impl reference``
 times the reference's own CPU implementation of the same path (the unmodified reference installed
 under ``baseline/_ref`` when present, else the numpy oracle port) on all host cores of the box.
 """
@@ -317,6 +319,47 @@ def workload_config(args, per_gpu_tracks):
     return out
 
 
+# --dump-outputs: a fixed, seeded sample of the track columns of the last timed step's results, at most this many bytes
+DUMP_BYTES = 60 * 1000 * 1000
+DUMP_SEED = 20251020
+
+
+def sample_results(res, budget=DUMP_BYTES, prefix=""):
+    """Host float64 copies of every result array of a TrackResults (its kernels' layout, tracks last), restricted to a
+    seeded sample of track columns sized to ``budget`` bytes; ``<prefix>columns`` holds the sampled column indices."""
+    import numpy as np
+    import torch
+
+    arrays, seen = {}, set()
+    for name in res._TENSORS:
+        t = getattr(res, name)
+        if t is None or t.data_ptr() in seen:      # smoothed in place: mean_s / cov_s are mean_f / cov_f
+            continue
+        seen.add(t.data_ptr())
+        arrays[name] = t
+    T = res.status.shape[0]
+    per_track = 8 * sum(t.numel() // T for t in arrays.values()) + 8
+    n = min(T, budget // per_track)
+    cols = np.sort(np.random.default_rng(DUMP_SEED).choice(T, size=n, replace=False))
+    idx = torch.from_numpy(cols).to(res.status.device)
+    out = {prefix + "columns": cols.astype(np.float64)}
+    for name, t in arrays.items():
+        a = t.index_select(t.dim() - 1, idx).to(torch.float64).cpu().numpy()
+        if name in ("mean_f", "cov_f", "mean_s", "cov_s") and res.n_steps_host is not None:
+            past = np.arange(a.shape[0])[:, None] > res.n_steps_host[cols][None, :]   # past a ragged track's end: never written
+            a = np.where(past[:, None, :], 0.0, a)
+        out[prefix + name] = a
+    return out
+
+
+def write_dump(directory, arrays):
+    import numpy as np
+
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 class ClockSampler:
     """nvidia-smi clocks / throttle reasons sampled DURING the timed region (one background
     `nvidia-smi -lms 50` process, read when the region ends)."""
@@ -548,6 +591,8 @@ def run_uniform(args, D):
         marks = [step(args.warmup + i, True) for i in range(args.steps)]
         t_end.record()
         D.barrier()
+    if args.dump_outputs and rank == 0:   # before the passes below reuse the buffers
+        write_dump(args.dump_outputs, sample_results(res))
     total_ms = D.reduce(t_start.elapsed_time(t_end), "max")
     f_ms = statistics.mean(m[0].elapsed_time(m[1]) for m in marks)
     b_ms = statistics.mean(m[1].elapsed_time(m[2]) for m in marks) if smoother else None
@@ -794,7 +839,7 @@ def run_ragged(args, D):
         pick, n_warm = list(mine), 0
     else:
         warm = [mine[i] for i in spaced(len(mine), args.warmup)]
-        pick, n_warm = warm + [mine[i] for i in spaced(len(mine), min(args.steps, len(mine)))], len(warm)
+        pick, n_warm = warm + [mine[i] for i in spaced(len(mine), args.steps)], len(warm)   # more steps than tiles: tiles repeat
     ev = lambda: torch.cuda.Event(enable_timing=True)  # noqa: E731
 
     def make_tile(ti):
@@ -823,6 +868,8 @@ def run_ragged(args, D):
                 recs.append((b.track_steps(), e0.elapsed_time(e1), e1.elapsed_time(e2), b.n_tracks, b.max_steps))
                 gated += int((r.gate_iters > 0).sum())
                 flagged += int(((r.status & ~nat.STE_STATUS_SMOOTH_RECOMPUTE) != 0).sum())
+            if args.dump_outputs and rank == 0 and n == len(pick) - 1:
+                write_dump(args.dump_outputs, sample_results(r))
             del b, r
             torch.cuda.empty_cache()
         D.barrier()
@@ -934,6 +981,9 @@ def run_fleet(args, D):
             if i >= args.warmup:
                 conc.append(e0.elapsed_time(e1))
         D.barrier()
+    if args.dump_outputs and rank == 0:
+        for _, _, r, group, _ in tiles:
+            write_dump(args.dump_outputs, sample_results(r, DUMP_BYTES // len(tiles), prefix=group[0]["fixture"] + "_"))
     # parity against the reference's own outputs stored with the inputs (what tests/test_gpu_golden.py asserts)
     for ukf, b, r, group, _ in tiles:
         r.check_status()
@@ -1005,8 +1055,12 @@ def main():
     ap.add_argument("--full-cov", action="store_true", help="store full 4x4 covariances (default: the 10 unique entries)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-tracks-per-core", type=int, default=16)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step as DIR/<name>.npy (float64; a fixed, "
+                                                          f"seeded sample of track columns, at most {DUMP_BYTES // 10**6} MB)")
     args = ap.parse_args()
     args.state_budget = int(args.state_budget)
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the GPU path computed (--impl b200)")
     if args.impl == "reference":
         run_reference_arm(args)
         return

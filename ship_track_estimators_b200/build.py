@@ -14,7 +14,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB_PATH = os.environ.get("STE_UKF_LIB") or os.path.join(CSRC, "libste_ukf.so")  # env override: developer A/B builds
 SOURCES = ["ste_ukf.cu"]
-HEADERS = ["ste_fastmath.cuh", "ste_math.cuh", "ste_filter.cuh", "ste_tracks.cuh", os.path.join("..", "..", "include", "ste_ukf.h")]
+HEADERS = ["ste_fastmath.cuh", "ste_math.cuh", "ste_filter.cuh", "ste_tracks.cuh", "ste_generic.cuh", "ste_ingest.cuh",
+           os.path.join("..", "..", "include", "ste_ukf.h")]
 
 NVCC_FLAGS = [
     "-O3",

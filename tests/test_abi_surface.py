@@ -40,6 +40,23 @@ def test_library_is_sm100a_only(native_lib):
     assert archs == {"sm_100a"}, archs
 
 
+def test_staleness_check_watches_every_included_file():
+    """build.is_stale() must see an edit to any file the compile reads: every local #include reachable from the sources."""
+    from ship_track_estimators_b200 import build
+
+    todo = [os.path.join(build.CSRC, s) for s in build.SOURCES]
+    seen = set()
+    while todo:
+        path = os.path.normpath(todo.pop())
+        if path in seen:
+            continue
+        seen.add(path)
+        for inc in re.findall(r'^\s*#\s*include\s+"([^"]+)"', open(path).read(), flags=re.M):
+            todo.append(os.path.join(os.path.dirname(path), inc))
+    watched = {os.path.normpath(os.path.join(build.CSRC, f)) for f in build.SOURCES + build.HEADERS}
+    assert seen <= watched, sorted(seen - watched)
+
+
 def test_ctypes_structs_match_c_layout():
     from ship_track_estimators_b200 import _native as nat
 

@@ -6,7 +6,7 @@ from types import SimpleNamespace
 import numpy as np
 import pytest
 
-from _helpers import GOLDEN, TOL, assert_track_close, cov_err, load_golden, mean_err
+from _helpers import GOLDEN, REPO, TOL, assert_track_close, cov_err, load_golden, mean_err
 
 pytestmark = pytest.mark.gpu
 
@@ -864,6 +864,38 @@ def test_bench_shape_tile_against_c_oracle(cuda, native_lib):
                 err = float(np.max(np.max(np.abs(g - r), axis=1) / np.max(np.abs(r), axis=1)))
             print(f"bench-shape tile packed={packed} smoother={smoother} {key}: worst error {err:.2e}")
             assert err <= TOL, (key, packed, smoother, err)
+
+
+def test_bench_dump_outputs_are_the_last_timed_step(cuda, native_lib, tmp_path):
+    """bench.py --dump-outputs: the sampled tracks of the last timed step, equal bit for bit to the same seeded tile run
+    directly through BatchedUKF, within the size limit, and --steps timed steps in the line."""
+    import json
+    import subprocess
+    import sys
+
+    import bench
+    from ship_track_estimators_b200.batch import BatchedUKF, TrackBatch
+    from ship_track_estimators_b200.synthetic import make_tracks
+
+    T, steps, warmup = 1184, 2, 3
+    out = subprocess.run([sys.executable, os.path.join(REPO, "bench.py"), "--tracks", str(T), "--steps", str(steps), "--warmup", str(warmup),
+                          "--no-job", "--no-partitioned", "--no-cpu-baseline", "--e2e-tracks", "128", "--e2e-headline-only",
+                          "--dump-outputs", str(tmp_path / "dump")], capture_output=True, text=True, timeout=900, cwd=REPO)
+    assert out.returncode == 0, out.stderr[-2000:]
+    line = json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][-1])
+    assert line["steps"] == steps and line["gpu_launches"] == 2 * steps
+    files = sorted(os.listdir(tmp_path / "dump"))
+    assert files == sorted(n + ".npy" for n in ("columns", "mean_f", "cov_f", "mean_s", "cov_s", "status", "n_updates"))
+    assert sum(os.path.getsize(tmp_path / "dump" / f) for f in files) <= 64 * 1000 * 1000
+    got = {f[:-4]: np.load(tmp_path / "dump" / f) for f in files}
+    assert all(a.dtype == np.float64 for a in got.values())
+    cols = got["columns"].astype(np.int64)
+    assert 0 < len(cols) < T and np.all(np.diff(cols) > 0) and cols[-1] < T    # a seeded sample of the tile's tracks
+    syn = make_tracks(T, 1024 + 1, seed=1000 + (warmup + steps - 1) % 2, device=str(cuda))   # the tile of the last timed step
+    H, R, Q, P = bench.np_model()
+    res = BatchedUKF(H, Q, R, P, packed_cov=True, long_steps=False).run(TrackBatch.from_synthetic(syn, substeps=1), smoother=True)
+    for name in ("mean_f", "cov_f", "mean_s", "cov_s", "status", "n_updates"):
+        assert np.array_equal(got[name], getattr(res, name)[..., cols].double().cpu().numpy()), name
 
 
 def _c4_shape_fleet(T, nobs_max, seed):

@@ -154,19 +154,47 @@ def test_bulk_csv_ingest_matches_per_ship_reader(tmp_path, string_labels):
         fleet.to_batch(device="cpu")
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/data/historical_ships/historical_ship_data.csv"),
-                    reason="reference data only exists in the build container")
-def test_bulk_csv_ingest_on_the_historical_file():
+def _historical_csv(path, tracks, ids, seed=5):
+    """The layout of the reference's data/historical_ships file (a leading row-label column that pandas turns into the
+    index, ships interleaved, an embedded repeated header row whose id is "id.tidy", ``lon2`` beside ``lon``) holding
+    the fixes of the committed real ships."""
+    rng = np.random.default_rng(seed)
+    rows = []
+    for s, (tr, sid) in enumerate(zip(tracks, ids)):
+        when = pd.Timestamp("1880-01-01") + pd.Timedelta(hours=24 * s) + pd.to_timedelta(np.concatenate(([0.0], np.cumsum(tr["dts"]))), unit="h")
+        rows += [(sid, d, float(lo), float(la)) for d, lo, la in zip(when, tr["z"][0], tr["z"][1])]
+    order = rng.permutation(len(rows))
+    # labels follow file order; zero-padded, so their string order (the header row makes them strings) is their number order
+    order = order[np.argsort([rows[k][1] for k in order], kind="stable")]
+    lines = ["primary.id,yr,mo,dy,hr,lat,lon,lon2"]
+    for lab, k in enumerate(order):
+        sid, d, lo, la = rows[k]
+        lines.append(f"{lab:05d},{sid},{d.year},{d.month},{d.day},{d.hour},{la!r},{lo!r},{lo!r}")
+        if lab == 1:
+            lines.append("row,id.tidy,yr,mo,dy,hr,lat,lon,lon2")
+    with open(path, "w") as fh:
+        fh.write("\n".join(lines) + "\n")
+
+
+def test_bulk_csv_ingest_on_the_historical_file(tmp_path):
+    """The 71 runnable ships of the reference's historical file (fixture c2_historical_batch: fixes and gaps as the
+    reference's ShipTrack read them) written back in that file's layout: the bulk reader, the per-ship reader and the
+    reference's own readings agree ship by ship."""
     from ship_track_estimators_b200.ingest import read_csv_fleet
 
-    csv = "/root/reference/data/historical_ships/historical_ship_data.csv"
+    tracks, extra = load_golden("c2_historical_batch")
+    ids = [str(i) for i in extra["ids"]]
+    csv = str(tmp_path / "historical_ship_data.csv")
+    _historical_csv(csv, tracks, ids)
     kw = dict(id_col="primary.id", lat_col="lat", lon_col="lon2")
     fleet = read_csv_fleet(csv, on_bad_rows="skip", **kw)
-    assert fleet.n_tracks == 116
-    for i in range(0, fleet.n_tracks, 5):
+    assert fleet.n_tracks == len(ids) == 71 and sorted(fleet.ids) == sorted(ids)
+    for i in range(fleet.n_tracks):
         lat, lon, dts = ShipTrack().read_csv(csv, ship_id=fleet.ids[i], **kw)
         a, b, c = fleet.track(i)
         assert np.array_equal(a, lat) and np.array_equal(b, lon) and np.array_equal(c, dts)
+        tr = tracks[ids.index(fleet.ids[i])]
+        assert np.array_equal(b, tr["z"][0]) and np.array_equal(a, tr["z"][1]) and np.array_equal(c, tr["dts"])
 
 
 def test_reference_import_name_is_an_alias():
