@@ -32,10 +32,12 @@
 extern "C" {
 #endif
 
-#define STE_ABI_VERSION 5   /* 2: ste_ukf_fused_f64, ste_track_metrics_f64, geodesy argument of ste_derive_inputs_f64, STE_FLAG_LONG_STEPS */
+#define STE_ABI_VERSION 6   /* 2: ste_ukf_fused_f64, ste_track_metrics_f64, geodesy argument of ste_derive_inputs_f64, STE_FLAG_LONG_STEPS */
                             /* 3: smooth_stats holds STE_STATS_PLANES = 15 planes per step (was 30)                                          */
                             /* 4: SteInputs.R_tracks, dimension-generic steps (ste_ukf_*_n_f64, ste_process_f64), ste_gate_terms_f64          */
                             /* 5: ste_urtss_backward_n_f64 (dimension-generic smoother); ld < 2^29                                            */
+                            /* 6: fleet path of the five-state model: SteProblemN / SteInputsN / SteOutputsN, ste_ukf_forward_n_f64,      */
+                            /*    ste_urtss_backward_tracks_n_f64                                                                          */
 #define STE_STATS_PLANES 15
 #define STE_DIM 4
 #define STE_NSIGMA 9
@@ -202,6 +204,61 @@ int ste_urtss_backward_n_f64(int32_t n, int32_t model, int32_t n_tracks, int64_t
                              double *cov_s, int32_t *status, void *stream);
 int ste_process_f64(int32_t model, int32_t n, int32_t n_tracks, int64_t ld, const double *x_in, const double *dt,
                     const double *sog_rate, const double *cog_rate, double *x_out, void *stream);
+
+/* Fleet path of the dimension-generic model (ABI 6): the n = 4 trio above for n = 5, STE_MODEL_GEODETIC_TURN.  Layout as
+ * everywhere else (element (plane, t) at base[plane * ld + t]); matrices are row-major n x n planes.  The arithmetic is
+ * that of ste_ukf_predict_n_f64 / ste_ukf_update_n_f64 / ste_urtss_backward_n_f64: every track is bit-identical to those
+ * single-step kernels driven step by step.  No gating, full (not packed) covariances.  H, Q, R, P0: reference
+ * UnscentedKalmanFilter.__init__ (unscented.py:20-74), row-major n x n in the first n*n entries; Q, R, P0 symmetric. */
+typedef struct SteProblemN {
+    int32_t n;             /* state dimension: 5                                            */
+    int32_t model;         /* STE_MODEL_GEODETIC_TURN                                       */
+    int32_t n_tracks;      /* T                                                             */
+    int32_t max_steps;     /* N_max: filter steps of the longest track (states = N_max + 1) */
+    int32_t max_obs;       /* rows available in the observation arrays                      */
+    int32_t reserved;      /* must be 0                                                     */
+    int64_t ld;            /* leading dimension of every SoA array (>= n_tracks)            */
+    double H[64];
+    double Q[64];
+    double R[64];
+    double P0[64];
+} SteProblemN;
+
+typedef struct SteInputsN {
+    const double *x0;         /* [n][ld] initial state                                                   */
+    const double *P0;         /* [n*n][ld] per-track prior covariance, or NULL -> SteProblemN.P0         */
+    const double *dt;         /* [max_steps][ld] step lengths (hours)                                    */
+    const uint8_t *upd_mask;  /* [max_steps][ld] 1 = step ends exactly on an observation time (forward) */
+    const int32_t *n_steps;   /* [T] steps per track, or NULL -> max_steps for all                       */
+    const double *z[8];       /* [max_obs][ld] observation rows 0 .. n-1; a NULL row is read as 0        */
+    const double *sog_rate;   /* [max_obs][ld]                                                           */
+    const double *cog_rate;   /* [max_obs][ld] or NULL (geodetic_dynamics_turn takes the turn rate from  */
+                              /* the state)                                                              */
+    const int32_t *rate_repeat; /* [T] backward-pass rate repeat per track (required by the backward)   */
+    /* optional noise tapes of UNIT normals (NULL = zero noise), scaled by sqrt(diag Q) / sqrt(diag R)   */
+    const double *noise_pred; /* [max_steps][n][ld]  unscented.py:198-202, row = step                    */
+    const double *noise_upd;  /* [max_obs][n][ld]    unscented.py:232-236, row = update index            */
+    const double *noise_bwd;  /* [max_steps][n][ld]  unscented.py:320-323, row = backward step           */
+} SteInputsN;
+
+typedef struct SteOutputsN {
+    double *mean_f;      /* [max_steps+1][n][ld]   filtered means; row 0 = prior (kalman_filter.py:76)   */
+    double *cov_f;       /* [max_steps+1][n*n][ld] filtered covariances                                  */
+    double *mean_s;      /* smoothed, same shapes; distinct arrays (no in-place smoothing)              */
+    double *cov_s;
+    int32_t *status;     /* [T] OR-ed STE_STATUS_* (the forward pass overwrites, the backward ORs)      */
+    int32_t *n_updates;  /* [T] observations assimilated incl. the initial one, or NULL                 */
+} SteOutputsN;
+
+/* KalmanFilterBase.run (kalman_filter.py:36-117) with UnscentedKalmanFilter.predict / update (unscented.py:144-265)
+ * for T tracks of the five-state model: row 0 the prior, the initial update with observation 0, predict step s with
+ * sog_rate / cog_rate at the current update index, an update with the next observation where upd_mask[s] is set
+ * (more matches than max_obs rows: STE_STATUS_OBS_OVERRUN, update skipped).  n = 4 geodetic: ste_ukf_forward_f64. */
+int ste_ukf_forward_n_f64(const SteProblemN *prob, const SteInputsN *in, SteOutputsN *out, void *stream);
+
+/* UnscentedKalmanFilter.rts_step (unscented.py:267-351) for T ragged tracks: track t has n_steps[t] + 1 states and
+ * reads rate[step / rate_repeat[t]]; reads mean_f / cov_f, writes mean_s / cov_s. */
+int ste_urtss_backward_tracks_n_f64(const SteProblemN *prob, const SteInputsN *in, SteOutputsN *out, void *stream);
 
 /* UnscentedKalmanFilter.criterion_index and the denominator of update_lambda_factor
  * (unscented.py:389-483) for T filters: with y = z - x (not z - Hx, no angle wrap) and

@@ -9,4 +9,4 @@ unscented Rauch-Tung-Striebel smoother, behind the reference's own Python surfac
 """
 __version__ = "0.1.0"
 
-__all__ = ["__version__", "kalman_filters", "utils", "constants", "ship_track", "performance_metrics", "batch", "synthetic", "sharding", "cli"]
+__all__ = ["__version__", "kalman_filters", "utils", "constants", "ship_track", "performance_metrics", "batch", "batch_n", "synthetic", "sharding", "cli"]

@@ -13,7 +13,7 @@ from typing import Optional
 from . import build as _build
 
 # --- mirror of include/ste_ukf.h ------------------------------------------------------------ #
-STE_ABI_VERSION = 5
+STE_ABI_VERSION = 6
 STE_OK, STE_ERR_INVALID_ARG, STE_ERR_CUDA, STE_ERR_UNSUPPORTED = 0, -1, -2, -3
 STE_FLAG_GATING, STE_FLAG_FORCE_GENERIC, STE_FLAG_PACKED_COV, STE_FLAG_LONG_STEPS = 0x1, 0x2, 0x4, 0x8
 STE_STATUS_NONFINITE = 0x1
@@ -81,6 +81,50 @@ class SteOutputs(C.Structure):
     ]
 
 
+class SteProblemN(C.Structure):
+    _fields_ = [
+        ("n", C.c_int32),
+        ("model", C.c_int32),
+        ("n_tracks", C.c_int32),
+        ("max_steps", C.c_int32),
+        ("max_obs", C.c_int32),
+        ("reserved", C.c_int32),
+        ("ld", C.c_int64),
+        ("H", C.c_double * 64),
+        ("Q", C.c_double * 64),
+        ("R", C.c_double * 64),
+        ("P0", C.c_double * 64),
+    ]
+
+
+class SteInputsN(C.Structure):
+    _fields_ = [
+        ("x0", _dptr),
+        ("P0", _dptr),
+        ("dt", _dptr),
+        ("upd_mask", _dptr),
+        ("n_steps", _dptr),
+        ("z", _dptr * 8),
+        ("sog_rate", _dptr),
+        ("cog_rate", _dptr),
+        ("rate_repeat", _dptr),
+        ("noise_pred", _dptr),
+        ("noise_upd", _dptr),
+        ("noise_bwd", _dptr),
+    ]
+
+
+class SteOutputsN(C.Structure):
+    _fields_ = [
+        ("mean_f", _dptr),
+        ("cov_f", _dptr),
+        ("mean_s", _dptr),
+        ("cov_s", _dptr),
+        ("status", _dptr),
+        ("n_updates", _dptr),
+    ]
+
+
 class NativeError(RuntimeError):
     """A non-zero return code of the C ABI."""
 
@@ -101,6 +145,8 @@ _PROTOTYPES = {
     "ste_ukf_update_n_f64": (C.c_int, [C.c_int32, C.c_int32, C.c_int64, C.POINTER(C.c_double), C.POINTER(C.c_double)] + [_dptr] * 5 + [C.c_void_p]),
     "ste_urtss_backward_n_f64": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_double)]
                                  + [_dptr] * 9 + [C.c_void_p]),
+    "ste_ukf_forward_n_f64": (C.c_int, [C.POINTER(SteProblemN), C.POINTER(SteInputsN), C.POINTER(SteOutputsN), C.c_void_p]),
+    "ste_urtss_backward_tracks_n_f64": (C.c_int, [C.POINTER(SteProblemN), C.POINTER(SteInputsN), C.POINTER(SteOutputsN), C.c_void_p]),
     "ste_process_f64": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int64] + [_dptr] * 5 + [C.c_void_p]),
     "ste_csv_parse_rows": (C.c_int, [_dptr, _dptr, C.c_int64, C.POINTER(C.c_int32)] + [_dptr] * 9 + [C.c_void_p]),
     "ste_gate_terms_f64": (C.c_int, [C.POINTER(SteProblem)] + [_dptr] * 5 + [C.c_void_p]),

@@ -87,6 +87,42 @@ def exact_update_mask(dt_array: np.ndarray, dts: np.ndarray, time0: float = 0.0)
     return np.isin(times, np.cumsum(np.asarray(dts, dtype=np.float64)))
 
 
+def length_order(lengths) -> Optional[np.ndarray]:
+    """Packing order of a ragged fleet: decreasing length, stable (equal lengths keep the caller's
+    order); None when the tracks are already in that order."""
+    lengths = np.asarray(lengths)
+    if len(lengths) > 1 and np.any(lengths[:-1] < lengths[1:]):
+        return np.argsort(-lengths, kind="stable")
+    return None
+
+
+def track_update_mask(i: int, tr, dt_array: np.ndarray, m: int, time0: float = 0.0) -> np.ndarray:
+    """``exact_update_mask`` of track ``i`` with ``m`` observations; ``IndexError`` where the reference
+    raises it: more matched observation times than observations (``kalman_filter.py:101-108``)."""
+    mk = exact_update_mask(dt_array, tr.dts, time0)
+    if 1 + int(mk.sum()) > m:
+        raise IndexError(f"track {i}: {1 + int(mk.sum())} update times matched but only {m} observations")
+    return mk
+
+
+def track_rates(i: int, tr, m: int):
+    """The first ``m`` entries of the track's ``sog_rate`` / ``cog_rate`` (``IndexError`` if shorter)."""
+    sri, cri = np.asarray(tr.sog_rate, dtype=np.float64), np.asarray(tr.cog_rate, dtype=np.float64)
+    if len(sri) < m or len(cri) < m:
+        raise IndexError(f"track {i}: sog_rate/cog_rate shorter than the observations")
+    return sri[:m], cri[:m]
+
+
+def track_rate_repeat(i: int, tr, n: int, m: int) -> int:
+    """The smoother's ``int(nstates / len(dts))`` rate repeat of a track of ``n`` steps and ``m``
+    observations (reference ``unscented.py:287-292``); ``IndexError`` when a rate index runs past the
+    repeated arrays (``:287-311``)."""
+    r = int((n + 1) / max(len(np.asarray(tr.dts)), 1)) if len(np.asarray(tr.dts)) else 0
+    if r < 1 or (n > 0 and (n - 1) // r >= m):
+        raise IndexError(f"track {i}: smoother rate index out of range (repeat {r})")
+    return r
+
+
 @dataclass
 class TrackBatch:
     """Device-resident inputs of one tile of ``n_tracks`` tracks (all tensors ``[plane][track]``)."""
@@ -306,10 +342,8 @@ class TrackBatch:
         if T == 0:
             raise ValueError("empty batch")
         dt_arrays = [np.asarray(d, dtype=np.float64).reshape(-1) for d in dt_arrays]
-        order = None
-        lengths = np.array([len(d) for d in dt_arrays])
-        if sort_by_length and T > 1 and np.any(lengths[:-1] < lengths[1:]):
-            order = np.argsort(-lengths, kind="stable")
+        order = length_order([len(d) for d in dt_arrays]) if sort_by_length else None
+        if order is not None:
             tracks = [tracks[j] for j in order]
             dt_arrays = [dt_arrays[j] for j in order]
             x0 = None if x0 is None else [x0[j] for j in order]
@@ -330,22 +364,13 @@ class TrackBatch:
             if zi.shape[0] != 4:
                 raise NotImplementedError("the CUDA path needs the 4-row measurement z = [lon; lat; sog; cog]")
             n, m = int(nsteps[i]), int(nobs[i])
-            mk = exact_update_mask(dt_arrays[i], tr.dts, time0)
-            if 1 + int(mk.sum()) > m:
-                raise IndexError(f"track {i}: {1 + int(mk.sum())} update times matched but only {m} observations")
             dt[:n, i] = dt_arrays[i]
-            mask[:n, i] = mk
+            mask[:n, i] = track_update_mask(i, tr, dt_arrays[i], m, time0)
             z[:, :m, i] = zi
-            sri, cri = np.asarray(tr.sog_rate, dtype=np.float64), np.asarray(tr.cog_rate, dtype=np.float64)
-            if len(sri) < m or len(cri) < m:
-                raise IndexError(f"track {i}: sog_rate/cog_rate shorter than the observations")
-            sr[:m, i], cr[:m, i] = sri[:m], cri[:m]
+            sr[:m, i], cr[:m, i] = track_rates(i, tr, m)
             x0a[:, i] = zi[:, 0] if x0 is None else np.asarray(x0[i], dtype=np.float64).reshape(-1)
             if smoother:
-                r = int((n + 1) / max(len(np.asarray(tr.dts)), 1)) if len(np.asarray(tr.dts)) else 0
-                if r < 1 or (n > 0 and (n - 1) // r >= m):
-                    raise IndexError(f"track {i}: smoother rate index out of range (repeat {r})")
-                rep[i] = r
+                rep[i] = track_rate_repeat(i, tr, n, m)
         dev = torch.device(device)
 
         def up(a):

@@ -481,8 +481,84 @@ __global__ void __launch_bounds__(64) urtss_backward_n_kernel(const __grid_const
                                                              const double *sog_rate, const double *cog_rate, const double *noise,
                                                              double *mean_s, double *cov_s, int32_t *status) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t < p.n_tracks) rts_n(p, t, n_states, rate_repeat, n_rates, mean_f, cov_f, dt, sog_rate, cog_rate, noise, mean_s, cov_s, status);
+    if (t >= p.n_tracks) return;
+    const int st = rts_n<0>(p, t, n_states, rate_repeat, n_rates, mean_f, cov_f, dt, sog_rate, cog_rate, noise, mean_s, cov_s);
+    if (status) status[t] = st;
 }
+
+// ------------------------------------------------------------------------------------------ //
+// Whole-track fleet kernels at a compile-time dimension (NC = 5: geodetic_dynamics_turn).  One thread
+// per track, the state thread-local across the time loop; the arithmetic is the single-step kernels'
+// (predict_core / update_core / rts_n of ste_generic.cuh), so every track is bit-identical to the
+// class API's step-by-step route.
+// ------------------------------------------------------------------------------------------ //
+#ifndef STE_N5_THREADS
+#define STE_N5_THREADS 64
+#endif
+constexpr int kThreadsN = STE_N5_THREADS;
+
+struct FleetArgsN {
+    ProblemN p;
+    double P0[kMaxN * kMaxN];   // shared prior, row-major n x n
+    int32_t max_steps, max_obs;
+    SteInputsN in;
+    SteOutputsN out;
+};
+
+// KalmanFilterBase.run (kalman_filter.py:36-117): row 0 the prior, the initial update with observation 0, then per step
+// a predict with the rates of the current update index and, where upd_mask is set, an update with the next observation.
+template <int NC>
+__global__ void __launch_bounds__(kThreadsN) ukf_forward_n_kernel(const __grid_constant__ FleetArgsN a) {
+    constexpr int D = DimN<NC>::LD, n = NC;
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= a.p.n_tracks) return;
+    const SteInputsN &in = a.in;
+    const int64_t ld = a.p.ld;
+    const int nt = in.n_steps ? min(in.n_steps[t], a.max_steps) : a.max_steps;
+    double x[D], P[D * D], z[D];
+    for (int r = 0; r < n; ++r) x[r] = in.x0[r * ld + t];
+    for (int i = 0; i < n; ++i)
+        for (int j = 0; j < n; ++j) P[i * D + j] = in.P0 ? in.P0[(i * n + j) * ld + t] : a.P0[i * n + j];
+    auto store = [&](int s) {
+        for (int r = 0; r < n; ++r) {
+            a.out.mean_f[((int64_t)s * n + r) * ld + t] = x[r];
+            for (int q = 0; q < n; ++q) a.out.cov_f[((int64_t)s * n * n + r * n + q) * ld + t] = P[r * D + q];
+        }
+    };
+    auto update = [&](int u) {   // observation row u; rows the caller left NULL read as 0
+        for (int r = 0; r < n; ++r) z[r] = in.z[r] ? in.z[r][(int64_t)u * ld + t] : 0.0;
+        return update_core<NC>(a.p, x, P, z, in.noise_upd ? in.noise_upd + (int64_t)u * n * ld + t : nullptr, ld);
+    };
+    store(0);                      // :76-81
+    int status = update(0), ui = 0;
+    for (int s = 0; s < nt; ++s) {
+        const double d = in.dt[(int64_t)s * ld + t], sr = in.sog_rate[(int64_t)ui * ld + t],
+                     cr = in.cog_rate ? in.cog_rate[(int64_t)ui * ld + t] : 0.0;
+        status |= predict_core<NC>(a.p, x, P, d, sr, cr, in.noise_pred ? in.noise_pred + (int64_t)s * n * ld + t : nullptr, ld,
+                                   nullptr, nullptr, 0);
+        if (in.upd_mask[(int64_t)s * ld + t]) {   // :101-108
+            if (ui + 1 < a.max_obs) status |= update(++ui);
+            else status |= STE_STATUS_OBS_OVERRUN;
+        }
+        store(s + 1);
+    }
+    a.out.status[t] = status;
+    if (a.out.n_updates) a.out.n_updates[t] = ui + 1;
+}
+
+// UnscentedKalmanFilter.rts_step (unscented.py:267-351) over ragged tracks: n_states = n_steps[t] + 1 and rate_repeat[t]
+// per track; the status bits are OR-ed into the forward pass's.
+template <int NC>
+__global__ void __launch_bounds__(kThreadsN) urtss_backward_n_tracks_kernel(const __grid_constant__ FleetArgsN a) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= a.p.n_tracks) return;
+    const SteInputsN &in = a.in;
+    const int nt = in.n_steps ? min(in.n_steps[t], a.max_steps) : a.max_steps;
+    const int rep = max(in.rate_repeat[t], 1);
+    a.out.status[t] |= rts_n<NC>(a.p, t, nt + 1, rep, a.max_obs, a.out.mean_f, a.out.cov_f, in.dt, in.sog_rate, in.cog_rate,
+                                 in.noise_bwd, a.out.mean_s, a.out.cov_s);
+}
+
 __global__ void __launch_bounds__(64) process_n_kernel(int model, int n, int T, int64_t ld, const double *xin, const double *dt,
                                                         const double *sog_rate, const double *cog_rate, double *xout) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
@@ -819,6 +895,63 @@ int ste_urtss_backward_n_f64(int32_t n, int32_t model, int32_t n_tracks, int64_t
     urtss_backward_n_kernel<<<(n_tracks + 63) / 64, 64, 0, (cudaStream_t)stream>>>(p, n_states, rate_repeat, n_rates, mean_f, cov_f, dt,
                                                                                   sog_rate, cog_rate, noise, mean_s, cov_s, status);
     return check_launch("urtss_backward_n_kernel");
+}
+
+static bool is_symmetric_n(int n, const double *M) {
+    for (int i = 0; i < n; ++i)
+        for (int j = 0; j < i; ++j)
+            if (M[i * n + j] != M[j * n + i]) return false;
+    return true;
+}
+
+static int validate_fleet_n(const SteProblemN *p, const SteInputsN *in, const SteOutputsN *out, bool backward) {
+    if (!p || !in || !out) return fail(STE_ERR_INVALID_ARG, "null SteProblemN / SteInputsN / SteOutputsN");
+    if (p->model == STE_MODEL_GEODETIC && p->n == 4)
+        return fail(STE_ERR_UNSUPPORTED, "n = 4 geodetic_dynamics runs on the batched n = 4 path: ste_ukf_forward_f64 / ste_urtss_backward_f64");
+    if (int rc = model_dim_ok(p->n, p->model)) return rc;
+    if (p->n != 5) return fail(STE_ERR_UNSUPPORTED, "the fleet kernels are built for n = 5 (geodetic_dynamics_turn)");
+    if (p->n_tracks < 0 || p->max_steps < 0 || p->max_obs < 1) return fail(STE_ERR_INVALID_ARG, "negative sizes");
+    if (p->ld < p->n_tracks) return fail(STE_ERR_INVALID_ARG, "ld < n_tracks");
+    if (!is_symmetric_n(p->n, p->Q) || !is_symmetric_n(p->n, p->R) || !is_symmetric_n(p->n, p->P0))
+        return fail(STE_ERR_UNSUPPORTED, "Q, R and P0 must be symmetric");
+    if (!in->dt || !in->sog_rate || (!backward && (!in->x0 || !in->upd_mask)) || (backward && !in->rate_repeat))
+        return fail(STE_ERR_INVALID_ARG, "missing input array");
+    if (!out->mean_f || !out->cov_f || !out->status || (backward && (!out->mean_s || !out->cov_s)))
+        return fail(STE_ERR_INVALID_ARG, "missing output array");
+    if ((out->mean_s && (out->mean_s == out->mean_f || out->mean_s == out->cov_f)) ||
+        (out->cov_s && (out->cov_s == out->cov_f || out->cov_s == out->mean_f)))
+        return fail(STE_ERR_INVALID_ARG, "mean_s / cov_s must not alias the filtered arrays");
+    return STE_OK;
+}
+
+static FleetArgsN fleet_args(const SteProblemN *prob, const SteInputsN *in, const SteOutputsN *out) {
+    FleetArgsN a{};
+    const int n = prob->n;
+    a.p.n = n; a.p.model = prob->model; a.p.n_tracks = prob->n_tracks; a.p.ld = prob->ld;
+    memcpy(a.p.H, prob->H, sizeof(double) * n * n);
+    memcpy(a.p.Q, prob->Q, sizeof(double) * n * n);
+    memcpy(a.p.R, prob->R, sizeof(double) * n * n);
+    memcpy(a.P0, prob->P0, sizeof(double) * n * n);
+    a.max_steps = prob->max_steps; a.max_obs = prob->max_obs;
+    a.in = *in;
+    a.out = *out;
+    return a;
+}
+
+int ste_ukf_forward_n_f64(const SteProblemN *prob, const SteInputsN *in, SteOutputsN *out, void *stream) {
+    if (int rc = validate_fleet_n(prob, in, out, false)) return rc;
+    if (prob->n_tracks == 0) return STE_OK;
+    const FleetArgsN a = fleet_args(prob, in, out);
+    ukf_forward_n_kernel<5><<<(prob->n_tracks + kThreadsN - 1) / kThreadsN, kThreadsN, 0, (cudaStream_t)stream>>>(a);
+    return check_launch("ukf_forward_n_kernel");
+}
+
+int ste_urtss_backward_tracks_n_f64(const SteProblemN *prob, const SteInputsN *in, SteOutputsN *out, void *stream) {
+    if (int rc = validate_fleet_n(prob, in, out, true)) return rc;
+    if (prob->n_tracks == 0) return STE_OK;
+    const FleetArgsN a = fleet_args(prob, in, out);
+    urtss_backward_n_tracks_kernel<5><<<(prob->n_tracks + kThreadsN - 1) / kThreadsN, kThreadsN, 0, (cudaStream_t)stream>>>(a);
+    return check_launch("urtss_backward_n_tracks_kernel");
 }
 
 int ste_process_f64(int32_t model, int32_t n, int32_t n_tracks, int64_t ld, const double *x_in, const double *dt,

@@ -374,7 +374,7 @@ class UnscentedKalmanFilter(KalmanFilterBase):
 
         self._resolve_process(None)
         if self.n != 4:
-            return self._run_generic(int(nsteps), dt, ship_track)
+            return self._run_fleet_n(int(nsteps), dt, ship_track)
         N = int(nsteps)
         mask = exact_update_mask(dt, ship_track.dts, self.time)
         tape = None
@@ -414,28 +414,51 @@ class UnscentedKalmanFilter(KalmanFilterBase):
             self.gate_iters.extend(out["gate_iters"].tolist())
             self.gate_lambda.extend(out["gate_lambda"].tolist())
 
-    def _run_generic(self, N, dt, ship_track):
-        """The reference's time loop (``kalman_filter.py:76-111``) around the dimension-generic single-step
-        kernels: for states other than the batched n = 4 layout, one predict (and update) launch per step."""
-        from ..batch import exact_update_mask
+    def _run_fleet_n(self, N, dt, ship_track):
+        """``run`` at n = 5 (``geodetic_dynamics_turn``): one launch of the five-state fleet kernel on a tile of one
+        track (``batch_n.BatchedUKFN``), bit-identical to the reference's time loop (``kalman_filter.py:76-111``)
+        driven through ``predict`` / ``update``.  With ``noise="numpy"`` the same normals are drawn in the same
+        order - n for the initial update, then per step n for the predict and n more when it updates - and
+        replayed through the kernel's noise tapes."""
+        from types import SimpleNamespace
 
-        mask = exact_update_mask(dt, ship_track.dts, self.time)
+        from ..batch import exact_update_mask
+        from ..batch_n import BatchedUKFN, TrackBatchN
+
+        n = self.n
         z = np.asarray(ship_track.z, dtype=np.float64)
-        if z.shape[0] > self.n:
+        if z.shape[0] > n:
             raise ValueError("the measurement has more rows than the state")
-        pad = lambda col: np.concatenate([col, np.zeros(self.n - z.shape[0])])   # noqa: E731
-        ui = 0
-        self.means.append(self.x.reshape(self.n, 1).copy())
-        self.covariances.append(np.array(self.P, dtype=np.float64))
-        self.update(pad(z[:, 0]))
-        for s in range(N):
-            self.predict(dt=dt[s], c=None, sog_rate=ship_track.sog_rate[ui], cog_rate=ship_track.cog_rate[ui])
-            self.time = self.time + dt[s]
-            if mask[s]:
-                ui += 1   # IndexError past the last observation, as in the reference (:101-108)
-                self.update(pad(z[:, ui]))
-            self.means.append(self.x.reshape(self.n, 1).copy())
-            self.covariances.append(np.array(self.P, dtype=np.float64))
+        # the prior travels as a per-track P0: after a first run it is a filtered covariance, not exactly symmetric
+        engine = BatchedUKFN(self.H, self.Q, self.R, measurement_model=self.measurement_model, gating=self.gating)
+        track = SimpleNamespace(dts=ship_track.dts, z=np.concatenate([z, np.zeros((n - z.shape[0], z.shape[1]))]),
+                                sog_rate=ship_track.sog_rate, cog_rate=ship_track.cog_rate)
+        tape = None
+        if self._noise_on():
+            mask = exact_update_mask(dt, ship_track.dts, self.time)
+            draws = _unit_normals(1 + N + int(mask.sum()), n)
+            pred, upd = np.zeros((N, n)), [draws[0]]
+            k = 1
+            for s in range(N):   # reference call order: predict, then update when the step matches
+                pred[s] = draws[k]
+                k += 1
+                if mask[s]:
+                    upd.append(draws[k])
+                    k += 1
+            tape = [dict(pred=pred, upd=np.asarray(upd))]
+        # IndexError past the last observation, as in the reference (:101-108)
+        batch = TrackBatchN.from_tracks([track], [dt], x0=[np.asarray(self.x).reshape(-1)], time0=self.time, noise=tape,
+                                        smoother=False, device="cuda", P0=[np.asarray(self.P, dtype=np.float64)])
+        self.compute_weights()
+        out = engine.run(batch, smoother=False).track(0)
+        self.status |= out["status"]
+        for s in range(N + 1):
+            self.means.append(out["means"][s].reshape(n, 1).copy())
+            self.covariances.append(out["covs"][s].copy())
+        self.x = self.means[-1]
+        self.P = self.covariances[-1]
+        if N > 0:
+            self.time = np.cumsum(np.concatenate(([np.float64(self.time)], dt)))[-1]
 
     def rts_step(self, fwd_means, fwd_vars, ship_track, *args, **kwargs):
         """Unscented RTS smoother over explicit filtered states (reference ``:267-351``).
