@@ -5,6 +5,7 @@
     python examples/fleet_from_csv.py <tracks.csv> <input.json> [--out-dir results --id-col primary.id --device-parse]
 
 Writes the CLI's five text files per ship (output_<id>_predictions.txt, ...) and prints a per-fleet summary.
+An input.json with "dim": 5 (5 x 5 H, Q, R, P) runs the five-state turn-rate model (geodetic_dynamics_turn) instead.
 """
 import argparse
 import json

@@ -32,12 +32,13 @@
 extern "C" {
 #endif
 
-#define STE_ABI_VERSION 6   /* 2: ste_ukf_fused_f64, ste_track_metrics_f64, geodesy argument of ste_derive_inputs_f64, STE_FLAG_LONG_STEPS */
+#define STE_ABI_VERSION 7   /* 2: ste_ukf_fused_f64, ste_track_metrics_f64, geodesy argument of ste_derive_inputs_f64, STE_FLAG_LONG_STEPS */
                             /* 3: smooth_stats holds STE_STATS_PLANES = 15 planes per step (was 30)                                          */
                             /* 4: SteInputs.R_tracks, dimension-generic steps (ste_ukf_*_n_f64, ste_process_f64), ste_gate_terms_f64          */
                             /* 5: ste_urtss_backward_n_f64 (dimension-generic smoother); ld < 2^29                                            */
                             /* 6: fleet path of the five-state model: SteProblemN / SteInputsN / SteOutputsN, ste_ukf_forward_n_f64,      */
                             /*    ste_urtss_backward_tracks_n_f64                                                                          */
+                            /* 7: ste_track_metrics_n_f64 (fit metrics of the five-state fleet path)                                      */
 #define STE_STATS_PLANES 15
 #define STE_DIM 4
 #define STE_NSIGMA 9
@@ -320,6 +321,14 @@ int ste_csv_parse_rows(const uint8_t *bytes, const int64_t *row_start, int64_t n
  * abs_diff [max_obs][4][ld] or NULL receives every |x - xref|; n_pairs [T] or NULL the pair count. */
 int ste_track_metrics_f64(const SteProblem *prob, const SteInputs *in, const double *mean, double *rmse,
                           double *cum_abs, double *max_abs, double *abs_diff, int32_t *n_pairs, void *stream);
+
+/* ste_track_metrics_f64 for a tile of the five-state fleet path (ABI 7): the same pairs and reductions over observation
+ * rows r < 5 (rows with in->z[r] == NULL are skipped and left untouched), the cadence from in->upd_mask (required) and
+ * in->n_steps.  prob and in are checked as for ste_ukf_forward_n_f64 (x0, dt, sog_rate and the outputs are not read).
+ * mean [max_steps+1][5][ld]; rmse, cum_abs, max_abs each [5][ld] or NULL; abs_diff [max_obs][5][ld] or NULL; n_pairs
+ * [T] or NULL. */
+int ste_track_metrics_n_f64(const SteProblemN *prob, const SteInputsN *in, const double *mean, double *rmse,
+                            double *cum_abs, double *max_abs, double *abs_diff, int32_t *n_pairs, void *stream);
 
 /* Test hook: evaluates the library's own fp64 elementary functions (csrc/ste_fastmath.cuh) on n
  * arguments.  kind 0 sincos(a), |a| <= 105615 -> (out0, out1); 1 atan2(a, b); 2 sqrt(a); 3 rsqrt(a); 4 1/a; 5 a/b;

@@ -13,7 +13,7 @@ from typing import Optional
 from . import build as _build
 
 # --- mirror of include/ste_ukf.h ------------------------------------------------------------ #
-STE_ABI_VERSION = 6
+STE_ABI_VERSION = 7
 STE_OK, STE_ERR_INVALID_ARG, STE_ERR_CUDA, STE_ERR_UNSUPPORTED = 0, -1, -2, -3
 STE_FLAG_GATING, STE_FLAG_FORCE_GENERIC, STE_FLAG_PACKED_COV, STE_FLAG_LONG_STEPS = 0x1, 0x2, 0x4, 0x8
 STE_STATUS_NONFINITE = 0x1
@@ -154,6 +154,7 @@ _PROTOTYPES = {
     "ste_geodetic_f64": (C.c_int, [C.c_int32, C.c_int64, _dptr, _dptr, _dptr, _dptr, _dptr, C.c_void_p]),
     "ste_derive_inputs_f64": (C.c_int, [C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_int32] + [_dptr] * 8 + [C.c_void_p]),
     "ste_track_metrics_f64": (C.c_int, [C.POINTER(SteProblem), C.POINTER(SteInputs)] + [_dptr] * 6 + [C.c_void_p]),
+    "ste_track_metrics_n_f64": (C.c_int, [C.POINTER(SteProblemN), C.POINTER(SteInputsN)] + [_dptr] * 6 + [C.c_void_p]),
     "ste_probe_fastmath": (C.c_int, [C.c_int32, C.c_int32, _dptr, _dptr, _dptr, _dptr, C.c_void_p]),
     "ste_probe_fp64_latency": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, _dptr, _dptr, C.c_void_p]),
     "ste_probe_fp64_fma": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, _dptr, C.c_void_p]),

@@ -808,14 +808,7 @@ class BatchedUKF:
     }
 
     def _output_names(self, outputs, smoother: bool):
-        names = self.OUTPUT_SETS[outputs] if isinstance(outputs, str) else tuple(outputs)
-        known = {"mean_f", "cov_f", "mean_s", "cov_s", "diag_f", "diag_s", "final", "metrics"}
-        for n in names:
-            if n not in known:
-                raise ValueError(f"unknown output {n!r}; choose from {sorted(known)} or a set name {sorted(self.OUTPUT_SETS)}")
-            if not smoother and n.endswith("_s"):
-                raise ValueError(f"output {n!r} needs the smoother")
-        return names
+        return output_names(self.OUTPUT_SETS, outputs, smoother)
 
     def host_outputs(self, b: TrackBatch, outputs="all", smoother: bool = True, pinned: bool = True) -> Dict[str, torch.Tensor]:
         """Host buffers (page-locked by default) for the selected outputs of a tile shaped like ``b``,
@@ -861,17 +854,6 @@ class BatchedUKF:
                 out[n] = torch.cat([m["rmse"], m["cum_abs"], m["max_abs"]], dim=0)
         return out
 
-    @staticmethod
-    def _copy_out(dev_out: Dict[str, torch.Tensor], host_out) -> int:
-        moved = 0
-        for n, src in dev_out.items():
-            dst = host_out.get(n) if isinstance(host_out, dict) else getattr(host_out, n, None)
-            if dst is None:
-                continue
-            dst.copy_(src, non_blocking=True)
-            moved += src.numel() * src.element_size()
-        return moved
-
     def run_host(self, host_batch: TrackBatch, host_out, dev_res: Optional[TrackResults] = None, smoother: bool = True,
                  device="cuda", outputs="all") -> Dict[str, int]:
         """End-to-end call on HOST buffers: pinned inputs -> device, forward (+ backward), the selected
@@ -881,7 +863,7 @@ class BatchedUKF:
         names = self._output_names(outputs, smoother)
         dev_batch = host_batch.to(device, non_blocking=True)
         dev_res = self.run(dev_batch, smoother=smoother, res=dev_res)
-        d2h = self._copy_out(self._extract(dev_batch, dev_res, names, smoother, {}), host_out)
+        d2h = copy_out(self._extract(dev_batch, dev_res, names, smoother, {}), host_out)
         return {"h2d_bytes": host_batch.input_bytes(), "d2h_bytes": d2h}
 
     def run_host_pipelined(self, host_batches: Sequence[TrackBatch], host_outs: Sequence, smoother: bool = True,
@@ -894,59 +876,8 @@ class BatchedUKF:
         ``outputs="all"``); all tiles must share one shape.  ``outputs`` selects what is copied back
         (``OUTPUT_SETS``): PCIe carries ~50 GB/s, so the bytes per state decide the end-to-end rate.
         Returns the bytes copied over all tiles in each direction; synchronise before reading ``host_outs``."""
-        dev = torch.device(device)
-        names = self._output_names(outputs, smoother)
-        n = len(host_batches)
-        if n != len(host_outs):
-            raise ValueError("one host output set per tile")
-        shape0 = (host_batches[0].n_tracks, host_batches[0].max_steps, host_batches[0].max_obs) if n else None
-        for hb in host_batches:
-            if (hb.n_tracks, hb.max_steps, hb.max_obs) != shape0:
-                raise ValueError("run_host_pipelined: all tiles must share one shape (n_tracks, max_steps, max_obs); "
-                                 f"got {(hb.n_tracks, hb.max_steps, hb.max_obs)} after {shape0}")
-        cur = torch.cuda.current_stream(dev)
-        if self._pipe is None or self._pipe["device"] != dev:
-            self._pipe = {"device": dev, "streams": [torch.cuda.Stream(dev) for _ in range(3)], "res": [None, None],
-                          "in": [None, None], "scratch": [{}, {}], "shape": None}
-        pipe = self._pipe
-        key = (shape0, smoother, self.packed_cov)
-        if pipe["shape"] != key:                 # device input and result buffers are kept across calls of one shape
-            pipe["res"], pipe["in"], pipe["scratch"], pipe["shape"] = [None, None], [None, None], [{}, {}], key
-        s_in, s_run, s_out = pipe["streams"]
-        for s_ in (s_in, s_run, s_out):
-            s_.wait_stream(cur)
-        dev_in: List[Optional[TrackBatch]] = pipe["in"]    # two resident input tiles, overwritten in place (no allocation in the loop)
-        in_done = [torch.cuda.Event() for _ in range(n)]
-        run_done = [torch.cuda.Event() for _ in range(n)]
-        out_done = [torch.cuda.Event() for _ in range(n)]
-        moved = {"h2d_bytes": 0, "d2h_bytes": 0}
-        for i in range(n):
-            k = i % 2
-            with torch.cuda.stream(s_in):
-                if i >= 2:
-                    s_in.wait_event(run_done[i - 2])        # the kernels that read this input slot are done
-                if dev_in[k] is None or not dev_in[k].copy_from(host_batches[i]):
-                    dev_in[k] = host_batches[i].to(dev, non_blocking=True)
-                in_done[i].record(s_in)
-            with torch.cuda.stream(s_run):
-                s_run.wait_event(in_done[i])
-                if i >= 2:
-                    s_run.wait_event(out_done[i - 2])       # this result slot has been copied out
-                if pipe["res"][k] is None:
-                    pipe["res"][k] = self.allocate(dev_in[k], smoother=smoother)
-                res = pipe["res"][k]
-                res.n_steps_host, res.order = dev_in[k].n_steps_host, dev_in[k].order
-                self.run(dev_in[k], smoother=smoother, res=res)
-                dev_out = self._extract(dev_in[k], res, names, smoother, pipe["scratch"][k])
-                run_done[i].record(s_run)
-            with torch.cuda.stream(s_out):
-                s_out.wait_event(run_done[i])
-                moved["d2h_bytes"] += self._copy_out(dev_out, host_outs[i])
-                out_done[i].record(s_out)
-            moved["h2d_bytes"] += host_batches[i].input_bytes()
-        for s_ in (s_in, s_run, s_out):
-            cur.wait_stream(s_)
-        return moved
+        return run_host_pipelined(self, host_batches, host_outs, self._output_names(outputs, smoother), smoother, device,
+                                  layout=self.packed_cov)
 
     def run(self, b: TrackBatch, smoother: bool = True, res: Optional[TrackResults] = None, in_place: bool = False) -> TrackResults:
         res = res if res is not None else self.allocate(b, smoother=smoother, in_place=in_place)
@@ -954,3 +885,91 @@ class BatchedUKF:
         if smoother:
             self.backward(b, res)
         return res
+
+
+# ---------------------------------------------------------------------- #
+# host-buffer entry points shared by BatchedUKF and batch_n.BatchedUKFN   #
+# ---------------------------------------------------------------------- #
+def output_names(output_sets: Dict[str, tuple], outputs, smoother: bool) -> tuple:
+    """The output names of a set name of ``output_sets`` or an explicit list; unknown names and smoothed outputs
+    without the smoother raise ``ValueError``."""
+    names = output_sets[outputs] if isinstance(outputs, str) else tuple(outputs)
+    known = {"mean_f", "cov_f", "mean_s", "cov_s", "diag_f", "diag_s", "final", "metrics"}
+    for n in names:
+        if n not in known:
+            raise ValueError(f"unknown output {n!r}; choose from {sorted(known)} or a set name {sorted(output_sets)}")
+        if not smoother and n.endswith("_s"):
+            raise ValueError(f"output {n!r} needs the smoother")
+    return names
+
+
+def copy_out(dev_out: Dict[str, torch.Tensor], host_out) -> int:
+    """Asynchronous device->host copies of ``dev_out`` into the same names of ``host_out`` (a dict or a host results
+    object); returns the bytes moved."""
+    moved = 0
+    for n, src in dev_out.items():
+        dst = host_out.get(n) if isinstance(host_out, dict) else getattr(host_out, n, None)
+        if dst is None:
+            continue
+        dst.copy_(src, non_blocking=True)
+        moved += src.numel() * src.element_size()
+    return moved
+
+
+def run_host_pipelined(engine, host_batches: Sequence, host_outs: Sequence, names: tuple, smoother: bool, device,
+                       layout=None) -> Dict[str, int]:
+    """The three-stream loop of ``run_host_pipelined`` for an engine with ``allocate`` / ``run`` / ``_extract`` and a
+    ``_pipe`` slot, over tiles with ``copy_from`` / ``to`` / ``input_bytes``.  ``layout``: whatever else decides the
+    shape of the engine's result buffers (kept with the tile shape to reuse them across calls)."""
+    dev = torch.device(device)
+    n = len(host_batches)
+    if n != len(host_outs):
+        raise ValueError("one host output set per tile")
+    shape0 = (host_batches[0].n_tracks, host_batches[0].max_steps, host_batches[0].max_obs) if n else None
+    for hb in host_batches:
+        if (hb.n_tracks, hb.max_steps, hb.max_obs) != shape0:
+            raise ValueError("run_host_pipelined: all tiles must share one shape (n_tracks, max_steps, max_obs); "
+                             f"got {(hb.n_tracks, hb.max_steps, hb.max_obs)} after {shape0}")
+    cur = torch.cuda.current_stream(dev)
+    if engine._pipe is None or engine._pipe["device"] != dev:
+        engine._pipe = {"device": dev, "streams": [torch.cuda.Stream(dev) for _ in range(3)], "res": [None, None],
+                        "in": [None, None], "scratch": [{}, {}], "shape": None}
+    pipe = engine._pipe
+    key = (shape0, smoother, layout)
+    if pipe["shape"] != key:                 # device input and result buffers are kept across calls of one shape
+        pipe["res"], pipe["in"], pipe["scratch"], pipe["shape"] = [None, None], [None, None], [{}, {}], key
+    s_in, s_run, s_out = pipe["streams"]
+    for s_ in (s_in, s_run, s_out):
+        s_.wait_stream(cur)
+    dev_in: List = pipe["in"]    # two resident input tiles, overwritten in place (no allocation in the loop)
+    in_done = [torch.cuda.Event() for _ in range(n)]
+    run_done = [torch.cuda.Event() for _ in range(n)]
+    out_done = [torch.cuda.Event() for _ in range(n)]
+    moved = {"h2d_bytes": 0, "d2h_bytes": 0}
+    for i in range(n):
+        k = i % 2
+        with torch.cuda.stream(s_in):
+            if i >= 2:
+                s_in.wait_event(run_done[i - 2])        # the kernels that read this input slot are done
+            if dev_in[k] is None or not dev_in[k].copy_from(host_batches[i]):
+                dev_in[k] = host_batches[i].to(dev, non_blocking=True)
+            in_done[i].record(s_in)
+        with torch.cuda.stream(s_run):
+            s_run.wait_event(in_done[i])
+            if i >= 2:
+                s_run.wait_event(out_done[i - 2])       # this result slot has been copied out
+            if pipe["res"][k] is None:
+                pipe["res"][k] = engine.allocate(dev_in[k], smoother=smoother)
+            res = pipe["res"][k]
+            res.n_steps_host, res.order = dev_in[k].n_steps_host, dev_in[k].order
+            engine.run(dev_in[k], smoother=smoother, res=res)
+            dev_out = engine._extract(dev_in[k], res, names, smoother, pipe["scratch"][k])
+            run_done[i].record(s_run)
+        with torch.cuda.stream(s_out):
+            s_out.wait_event(run_done[i])
+            moved["d2h_bytes"] += copy_out(dev_out, host_outs[i])
+            out_done[i].record(s_out)
+        moved["h2d_bytes"] += host_batches[i].input_bytes()
+    for s_ in (s_in, s_run, s_out):
+        cur.wait_stream(s_)
+    return moved

@@ -21,9 +21,18 @@ import numpy as np
 import torch
 
 from . import _native as nat
-from .batch import TrackBatch, TrackResults, length_order, track_rate_repeat, track_rates, track_update_mask
+from .batch import (BatchedUKF, TrackBatch, TrackResults, copy_out, length_order, output_names, run_host_pipelined,
+                    track_rate_repeat, track_rates, track_update_mask)
 
 NS = 5   # state dimension of geodetic_dynamics_turn
+
+#: default stored-state budget of a five-state tile (``sharding.plan_ragged_tiles``).  A stored state costs 480 B of
+#: results (mean 5 + covariance 25 doubles, filtered and smoothed), and at most 65 B of inputs (dt and update flag per
+#: step, five observation rows and two rates per fix; 120 B more with noise tapes).  The pipelined host path keeps two
+#: input and two result sets resident, plus 80 B of diagonal scratch per state and set for ``outputs="cli"``:
+#: 1e8 states take 2 x 48 GB + 2 x 6.5 GB (+ 24 GB with tapes) + 16 GB = 125 GB (149 GB) of a B200's 180 GB.
+#: The n = 4 budget, 4e8 states, would need 384 GB for the two result sets alone.
+STATE_BUDGET = 100_000_000
 
 
 def _as55(name: str, M) -> np.ndarray:
@@ -109,8 +118,58 @@ class TrackBatchN:
         return self._map(lambda t: t.to(device, non_blocking=non_blocking))
 
     def pin_memory(self) -> "TrackBatchN":
-        """Host tile in page-locked memory."""
+        """Host tile in page-locked memory (the staging form for :meth:`BatchedUKFN.run_host`)."""
         return self._map(lambda t: t.cpu().pin_memory())
+
+    def copy_from(self, other: "TrackBatchN", non_blocking: bool = True) -> bool:
+        """Overwrite this tile's tensors with ``other``'s (same shapes and the same optional tensors present; e.g.
+        pinned host tile -> resident device tile, no allocation).  Returns False, with nothing copied, when the
+        layouts differ."""
+        pairs = [(getattr(self, n), getattr(other, n)) for n in self._TENSORS] + list(zip(self.z, other.z))
+        if len(self.z) != len(other.z):
+            return False
+        for dst, src in pairs:
+            if (dst is None) != (src is None) or (dst is not None and (dst.shape != src.shape or dst.dtype != src.dtype)):
+                return False
+        for dst, src in pairs:
+            if dst is not None:
+                dst.copy_(src, non_blocking=non_blocking)
+        self.n_steps_host, self.order = other.n_steps_host, other.order
+        if hasattr(self, "_z_model"):
+            del self._z_model
+        return True
+
+    def input_bytes(self) -> int:
+        """Bytes of every tensor of the tile (what one host->device upload moves)."""
+        tensors = [getattr(self, n) for n in self._TENSORS] + list(self.z)
+        return int(sum(t.numel() * t.element_size() for t in tensors if t is not None))
+
+    @classmethod
+    def fleet_tiles(cls, tracks: Sequence, dt_arrays: Sequence[np.ndarray], x0: Optional[Sequence[np.ndarray]] = None,
+                    time0: float = 0.0, noise: Optional[Sequence[Optional[Dict[str, np.ndarray]]]] = None, smoother: bool = True,
+                    device="cuda", P0: Optional[Sequence[np.ndarray]] = None, state_budget: Optional[int] = None,
+                    **plan) -> List["TrackBatchN"]:
+        """A fleet too large for one tile, as tiles of :meth:`from_tracks` (same arguments): the tracks are sorted once
+        by decreasing length and cut by ``sharding.plan_ragged_tiles`` (``state_budget`` stored states per tile,
+        default :data:`STATE_BUDGET`; ``plan``: its ``granule`` / ``max_tracks``).  Column j of a tile holds the
+        caller's track ``tile.order[j]``, and its results' ``track(i)`` takes that caller index."""
+        from .sharding import plan_ragged_tiles
+
+        if len(tracks) == 0:
+            raise ValueError("empty batch")
+        dt_arrays = [np.asarray(d, dtype=np.float64).reshape(-1) for d in dt_arrays]
+        order = length_order([len(d) for d in dt_arrays])
+        order = np.arange(len(tracks)) if order is None else order
+        budget = STATE_BUDGET if state_budget is None else int(state_budget)
+        tiles = []
+        for lo, hi in plan_ragged_tiles([len(dt_arrays[j]) for j in order], budget, **plan):
+            idx = order[lo:hi]
+            pick = lambda seq: None if seq is None else [seq[j] for j in idx]   # noqa: E731
+            tile = cls.from_tracks(pick(tracks), pick(dt_arrays), x0=pick(x0), time0=time0, noise=pick(noise), smoother=smoother,
+                                   sort_by_length=False, device=device, P0=pick(P0))
+            tile.order = np.array(idx)
+            tiles.append(tile)
+        return tiles
 
     # ------------------------------------------------------------------ #
     @classmethod
@@ -215,12 +274,36 @@ class TrackResultsN:
 
     _TENSORS = ("mean_f", "cov_f", "mean_s", "cov_s", "status", "n_updates")
 
-    def to_host(self) -> "TrackResultsN":
-        """Host copy of every buffer; ``track(i)`` on it costs no further transfers."""
+    def host_like(self, pinned: bool = True) -> "TrackResultsN":
+        """Empty host buffers of the same shapes (page-locked by default) for device->host copies."""
+        def mk(t):
+            if t is None:
+                return None
+            h = torch.empty(t.shape, dtype=t.dtype, device="cpu")
+            return h.pin_memory() if pinned else h
+        return TrackResultsN(n_steps_host=self.n_steps_host, order=self.order, **{n: mk(getattr(self, n)) for n in self._TENSORS})
+
+    def copy_to(self, other: "TrackResultsN", non_blocking: bool = True) -> int:
+        """Copy every buffer into ``other`` (e.g. device -> pinned host); returns the bytes moved."""
+        moved = 0
+        for n in self._TENSORS:
+            src, dst = getattr(self, n), getattr(other, n)
+            if src is None or dst is None:
+                continue
+            dst.copy_(src, non_blocking=non_blocking)
+            moved += src.numel() * src.element_size()
+        return moved
+
+    def to_host(self, pinned: bool = False) -> "TrackResultsN":
+        """Host copy of every buffer (one device->host transfer per array); ``track(i)`` on it costs no further
+        transfers - the form the fleet writers use."""
         if not self.mean_f.is_cuda:
             return self
-        kw = {n: (None if getattr(self, n) is None else getattr(self, n).cpu()) for n in self._TENSORS}
-        return TrackResultsN(n_steps_host=self.n_steps_host, order=self.order, **kw)
+        host = self.host_like(pinned=pinned)
+        self.copy_to(host, non_blocking=pinned)
+        if pinned:
+            torch.cuda.current_stream(self.mean_f.device).synchronize()
+        return host
 
     def check_status(self, raise_on: int = nat.STE_STATUS_NONFINITE | nat.STE_STATUS_OBS_OVERRUN) -> Dict[str, int]:
         """Per-track status bits as counts; raises ``IndexError`` for an observation overrun and
@@ -228,13 +311,17 @@ class TrackResultsN:
         return TrackResults.check_status(self, raise_on)   # reads only .status
 
     def column(self, i: int) -> int:
-        """Column of the caller's track ``i``."""
+        """Column of the caller's track ``i`` (a tile of :meth:`TrackBatchN.fleet_tiles` holds some of the caller's
+        tracks: ``IndexError`` for one it does not hold)."""
         if self.order is None:
             return int(i)
         if self._column_of is None:
-            self._column_of = np.empty(len(self.order), dtype=np.int64)
+            self._column_of = np.full(int(np.max(self.order)) + 1 if len(self.order) else 0, -1, dtype=np.int64)
             self._column_of[self.order] = np.arange(len(self.order))
-        return int(self._column_of[i])
+        j = int(self._column_of[i]) if 0 <= i < len(self._column_of) else -1
+        if j < 0:
+            raise IndexError(f"track {i} is not in this tile")
+        return j
 
     def track(self, i: int) -> Dict[str, np.ndarray]:
         """Host copies for the caller's track ``i``: means (N_i+1, 5), covs (N_i+1, 5, 5)[, means_s, covs_s]."""
@@ -282,6 +369,7 @@ class BatchedUKFN:
                 raise ValueError(f"{name} must be symmetric")
         self.measurement_model = measurement_model
         self._lib = nat.load()
+        self._pipe = None   # streams and resident buffers of run_host_pipelined, created once
 
     def _problem(self, b: TrackBatchN) -> nat.SteProblemN:
         p = nat.SteProblemN()
@@ -367,3 +455,87 @@ class BatchedUKFN:
         if smoother:
             self.backward(b, res)
         return res
+
+    def run_many(self, batches: Sequence[TrackBatchN], results: Sequence[TrackResultsN]) -> None:
+        """Filter and smooth a sequence of resident tiles (e.g. :meth:`TrackBatchN.fleet_tiles`): two launches per tile,
+        on the current stream."""
+        if len(batches) != len(results):
+            raise ValueError("one result set per tile")
+        for b, r in zip(batches, results):
+            self.forward(b, r)
+            self.backward(b, r)
+
+    # ------------------------------------------------------------------ #
+    # host-buffer (end-to-end) entry points, as BatchedUKF's              #
+    # ------------------------------------------------------------------ #
+    #: named selections of what travels back to the host per tile (the names of ``BatchedUKF.OUTPUT_SETS``).  Per
+    #: stored state: "all" 480 B, "cli" 160 B (means and diag(P) of both passes, what the CLI writes), "filtered" and
+    #: "smoothed" 80 B each, "summary" nothing per state: per track the last filtered state (5 + 25) and the fit
+    #: metrics of ``performance_metrics.track_metrics`` (3 x 5).
+    OUTPUT_SETS = BatchedUKF.OUTPUT_SETS
+    _DIAG = [r * NS + r for r in range(NS)]   # planes 0, 6, 12, 18, 24
+
+    def _output_names(self, outputs, smoother: bool):
+        return output_names(self.OUTPUT_SETS, outputs, smoother)
+
+    def host_outputs(self, b: TrackBatchN, outputs="all", smoother: bool = True, pinned: bool = True) -> Dict[str, torch.Tensor]:
+        """Host buffers (page-locked by default) for the selected outputs of a tile shaped like ``b``, plus the
+        always-returned per-track ``status`` and ``n_updates``."""
+        T, S = b.n_tracks, b.max_steps + 1
+        shapes = {"mean_f": (S, NS, T), "mean_s": (S, NS, T), "cov_f": (S, NS * NS, T), "cov_s": (S, NS * NS, T),
+                  "diag_f": (S, NS, T), "diag_s": (S, NS, T), "final": (NS + NS * NS, T), "metrics": (3 * NS, T)}
+        out = {}
+        for n in self._output_names(outputs, smoother) + ("status", "n_updates"):
+            t = torch.empty(shapes.get(n, (T,)), dtype=torch.int32 if n in ("status", "n_updates") else torch.float64)
+            out[n] = t.pin_memory() if pinned else t
+        return out
+
+    def _extract(self, b: TrackBatchN, res: TrackResultsN, names, smoother: bool, scratch: Dict[str, torch.Tensor]) -> Dict[str, torch.Tensor]:
+        """Device tensors for the selected outputs (views where the result buffers already hold them, small gathers
+        into ``scratch`` otherwise)."""
+        dev = b.device
+        dsel = scratch.get("_diag_idx")
+        if dsel is None:
+            dsel = scratch["_diag_idx"] = torch.tensor(self._DIAG, device=dev)
+        out = {"status": res.status, "n_updates": res.n_updates}
+        for n in names:
+            if n in ("mean_f", "cov_f", "mean_s", "cov_s"):
+                out[n] = getattr(res, n)
+            elif n in ("diag_f", "diag_s"):
+                cov = res.cov_f if n == "diag_f" else res.cov_s
+                buf = scratch.get(n)
+                if buf is None or buf.shape != (cov.shape[0], NS, cov.shape[2]):
+                    buf = scratch[n] = torch.empty(cov.shape[0], NS, cov.shape[2], dtype=torch.float64, device=dev)
+                torch.index_select(cov, 1, dsel, out=buf)
+                out[n] = buf
+            elif n == "final":
+                last = b.n_steps.to(torch.int64)[None, None, :]
+                out[n] = torch.cat([torch.gather(res.mean_f, 0, last.expand(1, NS, -1))[0],
+                                    torch.gather(res.cov_f, 0, last.expand(1, NS * NS, -1))[0]], dim=0)
+            elif n == "metrics":
+                from .performance_metrics import track_metrics
+
+                m = track_metrics(self, b, res, which="smoothed" if smoother else "filtered")
+                out[n] = torch.cat([m["rmse"], m["cum_abs"], m["max_abs"]], dim=0)
+        return out
+
+    def run_host(self, host_batch: TrackBatchN, host_out, dev_res: Optional[TrackResultsN] = None, smoother: bool = True,
+                 device="cuda", outputs="all") -> Dict[str, int]:
+        """End-to-end call on HOST buffers: pinned inputs -> device, forward (+ backward), the selected ``outputs`` ->
+        pinned ``host_out`` (a dict from :meth:`host_outputs`, or a host ``TrackResultsN`` for ``outputs="all"``).
+        Asynchronous on the current stream; synchronise before reading ``host_out``.  Returns the bytes copied in
+        each direction."""
+        names = self._output_names(outputs, smoother)
+        dev_batch = host_batch.to(device, non_blocking=True)
+        dev_res = self.run(dev_batch, smoother=smoother, res=dev_res)
+        d2h = copy_out(self._extract(dev_batch, dev_res, names, smoother, {}), host_out)
+        return {"h2d_bytes": host_batch.input_bytes(), "d2h_bytes": d2h}
+
+    def run_host_pipelined(self, host_batches: Sequence[TrackBatchN], host_outs: Sequence, smoother: bool = True,
+                           device="cuda", outputs="all") -> Dict[str, int]:
+        """:meth:`BatchedUKF.run_host_pipelined` for five-state tiles: while tile i is filtered and smoothed, tile
+        i+1's inputs travel host->device and tile i-1's selected ``outputs`` device->host, on three streams with two
+        resident buffer sets.  ``host_batches`` / ``host_outs`` live in pinned memory and all tiles share one shape
+        (``ValueError`` otherwise).  Returns the bytes copied over all tiles in each direction; synchronise before
+        reading ``host_outs``."""
+        return run_host_pipelined(self, host_batches, host_outs, self._output_names(outputs, smoother), smoother, device)

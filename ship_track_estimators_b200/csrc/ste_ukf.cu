@@ -284,9 +284,24 @@ __global__ void __launch_bounds__(kThreads) geodetic_kernel(int T, int64_t ld, c
 // observations it assimilated, one thread per track walking the forward pass's update cadence.
 // Streaming reads of [step][row][track] planes; HBM-bound (two to four doubles per update).
 // ------------------------------------------------------------------------------------------ //
+// NS = 4 reads the n = 4 tile (SteProblem / SteInputs, cadence from upd_mask or substeps), NS = 5 the five-state fleet
+// tile (SteProblemN / SteInputsN, upd_mask required).  The arithmetic is the same for both.
+template <int NS> struct MetricsTile;
+template <> struct MetricsTile<4> {
+    using Problem = SteProblem;
+    using Inputs = SteInputs;
+    __device__ static int substeps(const SteProblem &p) { return p.substeps > 0 ? p.substeps : 1; }
+};
+template <> struct MetricsTile<5> {
+    using Problem = SteProblemN;
+    using Inputs = SteInputsN;
+    __device__ static int substeps(const SteProblemN &) { return 1; }
+};
+
+template <int NS>
 struct MetricsArgs {
-    SteProblem prob;
-    SteInputs in;
+    typename MetricsTile<NS>::Problem prob;
+    typename MetricsTile<NS>::Inputs in;
     const double *mean;
     double *rmse, *cum_abs, *max_abs, *abs_diff;
     int32_t *n_pairs;
@@ -295,26 +310,27 @@ struct MetricsArgs {
 // One thread per (track, observation row): the rows of a track are independent sums, and twice (position-only) to four
 // times the threads of a one-thread-per-track launch keep twice to four times the loads in flight.  blockIdx.y
 // counts the rows that exist (z[r] != NULL), in order.
-__global__ void __launch_bounds__(kThreads) track_metrics_kernel(const __grid_constant__ MetricsArgs a) {
+template <int NS>
+__global__ void __launch_bounds__(kThreads) track_metrics_kernel(const __grid_constant__ MetricsArgs<NS> a) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= a.prob.n_tracks) return;
     int r = 0;
-    for (int seen = -1; r < 4; ++r) {
+    for (int seen = -1; r < NS; ++r) {
         if (a.in.z[r] && ++seen == (int)blockIdx.y) break;
     }
     const int64_t ld = a.prob.ld;
     const int nt = a.in.n_steps ? min(a.in.n_steps[t], a.prob.max_steps) : a.prob.max_steps;
-    const int k_sub = a.prob.substeps > 0 ? a.prob.substeps : 1;
+    const int k_sub = MetricsTile<NS>::substeps(a.prob);
     const double *zr = a.in.z[r] + t;
     const double *mr = a.mean + (int64_t)r * ld + t;
     double sq = 0.0, sa = 0.0, mx = 0.0;
     int pairs = 0, ui = 0;
     auto pair = [&](int state, int obs) {
-        const double d = fabs(STE_LOAD_STREAM(mr + ((int64_t)state * 4) * ld) - zr[(int64_t)obs * ld]);
+        const double d = fabs(STE_LOAD_STREAM(mr + ((int64_t)state * NS) * ld) - zr[(int64_t)obs * ld]);
         sq = fma(d, d, sq);
         sa += d;
         mx = fmax(mx, d);   // NaN residuals propagate through sq / sa
-        if (a.abs_diff) STE_STORE_STREAM(a.abs_diff + ((int64_t)obs * 4 + r) * ld + t, d);
+        if (a.abs_diff) STE_STORE_STREAM(a.abs_diff + ((int64_t)obs * NS + r) * ld + t, d);
         ++pairs;
     };
     pair(0, 0);
@@ -904,8 +920,8 @@ static bool is_symmetric_n(int n, const double *M) {
     return true;
 }
 
-static int validate_fleet_n(const SteProblemN *p, const SteInputsN *in, const SteOutputsN *out, bool backward) {
-    if (!p || !in || !out) return fail(STE_ERR_INVALID_ARG, "null SteProblemN / SteInputsN / SteOutputsN");
+// the problem checks shared by the fleet passes and the five-state metrics
+static int validate_problem_n(const SteProblemN *p) {
     if (p->model == STE_MODEL_GEODETIC && p->n == 4)
         return fail(STE_ERR_UNSUPPORTED, "n = 4 geodetic_dynamics runs on the batched n = 4 path: ste_ukf_forward_f64 / ste_urtss_backward_f64");
     if (int rc = model_dim_ok(p->n, p->model)) return rc;
@@ -914,6 +930,12 @@ static int validate_fleet_n(const SteProblemN *p, const SteInputsN *in, const St
     if (p->ld < p->n_tracks) return fail(STE_ERR_INVALID_ARG, "ld < n_tracks");
     if (!is_symmetric_n(p->n, p->Q) || !is_symmetric_n(p->n, p->R) || !is_symmetric_n(p->n, p->P0))
         return fail(STE_ERR_UNSUPPORTED, "Q, R and P0 must be symmetric");
+    return STE_OK;
+}
+
+static int validate_fleet_n(const SteProblemN *p, const SteInputsN *in, const SteOutputsN *out, bool backward) {
+    if (!p || !in || !out) return fail(STE_ERR_INVALID_ARG, "null SteProblemN / SteInputsN / SteOutputsN");
+    if (int rc = validate_problem_n(p)) return rc;
     if (!in->dt || !in->sog_rate || (!backward && (!in->x0 || !in->upd_mask)) || (backward && !in->rate_repeat))
         return fail(STE_ERR_INVALID_ARG, "missing input array");
     if (!out->mean_f || !out->cov_f || !out->status || (backward && (!out->mean_s || !out->cov_s)))
@@ -1032,21 +1054,42 @@ int ste_derive_inputs_f64(int32_t n_tracks, int32_t max_obs, int64_t ld, int32_t
     return check_launch("derive_inputs_kernel");
 }
 
+extern "C++" {
+template <int NS>
+static int launch_track_metrics(const MetricsArgs<NS> &a, cudaStream_t s) {
+    int rows = 0;
+    for (int r = 0; r < NS; ++r) rows += a.in.z[r] != nullptr;
+    if (rows == 0) return fail(STE_ERR_INVALID_ARG, "no observation row to compare with");
+    const dim3 grid((a.prob.n_tracks + kThreads - 1) / kThreads, rows), block(kThreads);
+    track_metrics_kernel<NS><<<grid, block, 0, s>>>(a);
+    return check_launch("track_metrics_kernel");
+}
+}
+
 int ste_track_metrics_f64(const SteProblem *prob, const SteInputs *in, const double *mean, double *rmse, double *cum_abs,
                           double *max_abs, double *abs_diff, int32_t *n_pairs, void *stream) {
     if (int rc = validate_problem(prob)) return rc;
     if (!in || !mean) return fail(STE_ERR_INVALID_ARG, "null SteInputs / state array");
     if (prob->n_tracks == 0) return STE_OK;
-    MetricsArgs a{};
+    MetricsArgs<4> a{};
     a.prob = *prob;
     a.in = *in;
     a.mean = mean; a.rmse = rmse; a.cum_abs = cum_abs; a.max_abs = max_abs; a.abs_diff = abs_diff; a.n_pairs = n_pairs;
-    int rows = 0;
-    for (int r = 0; r < 4; ++r) rows += in->z[r] != nullptr;
-    if (rows == 0) return fail(STE_ERR_INVALID_ARG, "no observation row to compare with");
-    const dim3 grid((prob->n_tracks + kThreads - 1) / kThreads, rows), block(kThreads);
-    track_metrics_kernel<<<grid, block, 0, (cudaStream_t)stream>>>(a);
-    return check_launch("track_metrics_kernel");
+    return launch_track_metrics(a, (cudaStream_t)stream);
+}
+
+int ste_track_metrics_n_f64(const SteProblemN *prob, const SteInputsN *in, const double *mean, double *rmse, double *cum_abs,
+                            double *max_abs, double *abs_diff, int32_t *n_pairs, void *stream) {
+    if (!prob || !in) return fail(STE_ERR_INVALID_ARG, "null SteProblemN / SteInputsN");
+    if (int rc = validate_problem_n(prob)) return rc;
+    if (!in->upd_mask) return fail(STE_ERR_INVALID_ARG, "missing input array");
+    if (!mean) return fail(STE_ERR_INVALID_ARG, "null state array");
+    if (prob->n_tracks == 0) return STE_OK;
+    MetricsArgs<5> a{};
+    a.prob = *prob;
+    a.in = *in;
+    a.mean = mean; a.rmse = rmse; a.cum_abs = cum_abs; a.max_abs = max_abs; a.abs_diff = abs_diff; a.n_pairs = n_pairs;
+    return launch_track_metrics(a, (cudaStream_t)stream);
 }
 
 int ste_probe_fastmath(int32_t kind, int32_t n, const double *a, const double *b, double *out0, double *out1, void *stream) {

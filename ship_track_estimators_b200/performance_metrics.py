@@ -4,7 +4,7 @@
 (``performance_metrics.py:4-58``); they are array utilities on whatever the caller holds (numpy
 arrays, or torch tensors on any device - the arithmetic then runs where the tensors live).
 ``track_metrics`` is what a 16 M-track run needs instead of copying every state to the host: one
-kernel launch (``ste_track_metrics_f64``) that reduces, per track, the residuals between a state
+kernel launch (``ste_track_metrics_f64``, ``ste_track_metrics_n_f64`` at n = 5) that reduces, per track, the residuals between a state
 estimate and the observations it assimilated.
 """
 from __future__ import annotations
@@ -48,21 +48,30 @@ def track_metrics(ukf, batch, res, which: str = "smoothed", keep_abs_diff: bool 
     when the measurement model uses them) and every track: ``rmse``, the last element of
     ``cum_abs_diff`` and the maximum of ``abs_diff`` over the pairs (state after the update,
     observation), the prior being paired with the first fix.  Returns device tensors
-    ``rmse``/``cum_abs``/``max_abs`` of shape ``[4, T]`` (NaN in rows the batch does not carry),
-    ``n_pairs`` ``[T]`` and, on request, ``abs_diff`` ``[max_obs, 4, T]``.
+    ``rmse``/``cum_abs``/``max_abs`` of shape ``[n, T]`` (NaN in rows the batch does not carry),
+    ``n_pairs`` ``[T]`` and, on request, ``abs_diff`` ``[max_obs, n, T]``.
+
+    ``n`` is 4 for a ``batch.BatchedUKF`` / ``TrackBatch`` / ``TrackResults`` triple
+    (``ste_track_metrics_f64``) and 5 for a ``batch_n.BatchedUKFN`` / ``TrackBatchN`` / ``TrackResultsN``
+    one (``ste_track_metrics_n_f64``); there the observations are the rows the forward pass
+    assimilated, after the filter's measurement model.
     """
+    from .batch_n import BatchedUKFN
+
     mean = {"smoothed": res.mean_s, "filtered": res.mean_f}[which]
     if mean is None:
         raise ValueError("results hold no smoothed states")
     ukf._check_shapes(batch, res, smoother=(which == "smoothed"))
+    five = isinstance(ukf, BatchedUKFN)
+    n, fn = (5, ukf._lib.ste_track_metrics_n_f64) if five else (4, ukf._lib.ste_track_metrics_f64)
     dev, T, ld = batch.device, batch.n_tracks, int(mean.shape[-1])
-    out = {k: torch.full((4, ld), float("nan"), dtype=torch.float64, device=dev) for k in ("rmse", "cum_abs", "max_abs")}
+    out = {k: torch.full((n, ld), float("nan"), dtype=torch.float64, device=dev) for k in ("rmse", "cum_abs", "max_abs")}
     n_pairs = torch.zeros(ld, dtype=torch.int32, device=dev)
-    ad = torch.full((batch.max_obs, 4, ld), float("nan"), dtype=torch.float64, device=dev) if keep_abs_diff else None
+    ad = torch.full((batch.max_obs, n, ld), float("nan"), dtype=torch.float64, device=dev) if keep_abs_diff else None
     p, i = ukf._problem(batch), ukf._inputs(batch)
     with torch.cuda.device(dev):
-        nat.check(ukf._lib.ste_track_metrics_f64(C.byref(p), C.byref(i), nat.ptr(mean), nat.ptr(out["rmse"]), nat.ptr(out["cum_abs"]),
-                                                  nat.ptr(out["max_abs"]), nat.ptr(ad), nat.ptr(n_pairs), nat.current_stream()))
+        nat.check(fn(C.byref(p), C.byref(i), nat.ptr(mean), nat.ptr(out["rmse"]), nat.ptr(out["cum_abs"]), nat.ptr(out["max_abs"]),
+                     nat.ptr(ad), nat.ptr(n_pairs), nat.current_stream()))
     out = {k: v[:, :T] for k, v in out.items()}
     out["n_pairs"] = n_pairs[:T]
     if ad is not None:
