@@ -330,6 +330,44 @@ int ste_track_metrics_f64(const SteProblem *prob, const SteInputs *in, const dou
 int ste_track_metrics_n_f64(const SteProblemN *prob, const SteInputsN *in, const double *mean, double *rmse,
                             double *cum_abs, double *max_abs, double *abs_diff, int32_t *n_pairs, void *stream);
 
+/* The CLI's text files for many ships at once: np.savetxt(path, X) with its defaults (fmt "%.18e", delimiter " ", newline
+ * "\n"), as the reference CLI writes predictions, variances, dts and tracks (main_cli.py:146-167).  Every value is
+ * formatted as CPython's "%.18e" % x (PyOS_double_to_string(x, 'e', 18): 19 significant digits, correctly rounded, ties
+ * to even; "inf", "-inf", every NaN "nan"), followed by " " or, after a row's last column, "\n".
+ *
+ * A table is one file kind (say, the filtered means); an item is one ship.  Values are numbered item-major, then table,
+ * row and column: segment g = item * n_tables + table holds values [value_start[g], value_start[g + 1]) (device,
+ * n_items * n_tables + 1 entries, value_start[0] = 0, non-decreasing), rows of n_cols values.  Value (row r, column c)
+ * of item i in table t is read from t.base[((r / t.row_div) * t.row_stride + t.plane[c]) * t.ld + t.track[i]], the usual
+ * SoA layout (plane, track): the diagonal of a row-major n x n covariance is planes 0, n + 1, 2 (n + 1), ...; of the
+ * packed 4 x 4 layout (STE_FLAG_PACKED_COV) planes 0, 4, 7, 9; row_div repeats source rows (the _dts file: dts /
+ * substeps, each repeated substeps times).  value_start and track must only address rows and tracks the sources hold
+ * (track[i] < n_tracks).
+ *
+ * ste_text_convert_f64: converts every value; digits [n_values] (the 19 significant digits as an integer), meta
+ *   [n_values] (kind, sign, decimal exponent, separator) and length [n_values] (bytes of the field and its separator).
+ * The caller forms end = inclusive scan of length (int64); the text of value v is out[end[v] - length[v], end[v]) and the
+ *   file of segment g starts at the end of value value_start[g] - 1.
+ * ste_text_write: writes the text of every value into out (device), which must hold STE_TEXT_MAX_VALUE_BYTES per value
+ *   (the longest field, "-1.234567890123456789e-308", and its separator) whatever the total turns out to be. */
+#define STE_TEXT_MAX_COLS 8
+#define STE_TEXT_MAX_TABLES 8
+#define STE_TEXT_MAX_VALUE_BYTES 27
+typedef struct SteTextTable {
+    const double *base;      /* source planes (device)                                          */
+    const int32_t *track;    /* [n_items] column of item i in base (device)                     */
+    int64_t ld;              /* leading dimension of base (>= n_tracks)                         */
+    int32_t n_tracks;        /* columns of base                                                 */
+    int32_t row_stride;      /* planes per source row (>= 1)                                    */
+    int32_t row_div;         /* output row r reads source row r / row_div (>= 1)                */
+    int32_t n_cols;          /* values per output row, 1 .. STE_TEXT_MAX_COLS                   */
+    int32_t plane[STE_TEXT_MAX_COLS]; /* plane of column c within a source row, [0, row_stride) */
+} SteTextTable;
+int ste_text_convert_f64(const SteTextTable *tables, int32_t n_tables, int32_t n_items, const int64_t *value_start,
+                         int64_t n_values, uint64_t *digits, int32_t *meta, int32_t *length, void *stream);
+int ste_text_write(int64_t n_values, const uint64_t *digits, const int32_t *meta, const int64_t *end, uint8_t *out,
+                   int64_t out_bytes, void *stream);
+
 /* Test hook: evaluates the library's own fp64 elementary functions (csrc/ste_fastmath.cuh) on n
  * arguments.  kind 0 sincos(a), |a| <= 105615 -> (out0, out1); 1 atan2(a, b); 2 sqrt(a); 3 rsqrt(a); 4 1/a; 5 a/b;
  * 6 atan2(a, b) for b >= 0. */

@@ -125,6 +125,22 @@ class SteOutputsN(C.Structure):
     ]
 
 
+STE_TEXT_MAX_COLS, STE_TEXT_MAX_TABLES, STE_TEXT_MAX_VALUE_BYTES = 8, 8, 27
+
+
+class SteTextTable(C.Structure):
+    _fields_ = [
+        ("base", _dptr),
+        ("track", _dptr),
+        ("ld", C.c_int64),
+        ("n_tracks", C.c_int32),
+        ("row_stride", C.c_int32),
+        ("row_div", C.c_int32),
+        ("n_cols", C.c_int32),
+        ("plane", C.c_int32 * STE_TEXT_MAX_COLS),
+    ]
+
+
 class NativeError(RuntimeError):
     """A non-zero return code of the C ABI."""
 
@@ -155,6 +171,8 @@ _PROTOTYPES = {
     "ste_derive_inputs_f64": (C.c_int, [C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_int32] + [_dptr] * 8 + [C.c_void_p]),
     "ste_track_metrics_f64": (C.c_int, [C.POINTER(SteProblem), C.POINTER(SteInputs)] + [_dptr] * 6 + [C.c_void_p]),
     "ste_track_metrics_n_f64": (C.c_int, [C.POINTER(SteProblemN), C.POINTER(SteInputsN)] + [_dptr] * 6 + [C.c_void_p]),
+    "ste_text_convert_f64": (C.c_int, [C.POINTER(SteTextTable), C.c_int32, C.c_int32, _dptr, C.c_int64] + [_dptr] * 3 + [C.c_void_p]),
+    "ste_text_write": (C.c_int, [C.c_int64] + [_dptr] * 4 + [C.c_int64, C.c_void_p]),
     "ste_probe_fastmath": (C.c_int, [C.c_int32, C.c_int32, _dptr, _dptr, _dptr, _dptr, C.c_void_p]),
     "ste_probe_fp64_latency": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, _dptr, _dptr, C.c_void_p]),
     "ste_probe_fp64_fma": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, _dptr, C.c_void_p]),

@@ -13,8 +13,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB_PATH = os.environ.get("STE_UKF_LIB") or os.path.join(CSRC, "libste_ukf.so")  # env override: developer A/B builds
-SOURCES = ["ste_ukf.cu"]
-HEADERS = ["ste_fastmath.cuh", "ste_math.cuh", "ste_filter.cuh", "ste_tracks.cuh", "ste_generic.cuh", "ste_ingest.cuh",
+SOURCES = ["ste_ukf.cu", "ste_text.cu"]
+HEADERS = ["ste_fastmath.cuh", "ste_math.cuh", "ste_filter.cuh", "ste_tracks.cuh", "ste_generic.cuh", "ste_ingest.cuh", "ste_text.cuh",
            os.path.join("..", "..", "include", "ste_ukf.h")]
 
 NVCC_FLAGS = [

@@ -675,6 +675,10 @@ static int check_launch(const char *what) {
     return STE_OK;
 }
 
+// the same two for the library's other translation units (ste_text.cu)
+int report_error(int code, const char *what) { return fail(code, "%s", what); }
+int report_launch(const char *what) { return check_launch(what); }
+
 static bool is_symmetric(const double *M) {
     for (int i = 0; i < 4; ++i)
         for (int j = 0; j < i; ++j)
