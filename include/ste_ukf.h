@@ -39,6 +39,8 @@ extern "C" {
                             /* 6: fleet path of the five-state model: SteProblemN / SteInputsN / SteOutputsN, ste_ukf_forward_n_f64,      */
                             /*    ste_urtss_backward_tracks_n_f64                                                                          */
                             /* 7: ste_track_metrics_n_f64 (fit metrics of the five-state fleet path)                                      */
+                            /*    additive, no struct changed: SteNoiseN, ste_ukf_forward_noise_n_f64,                                    */
+                            /*    ste_urtss_backward_tracks_noise_n_f64 (per-track Q / R of the five-state fleet path)                    */
 #define STE_STATS_PLANES 15
 #define STE_DIM 4
 #define STE_NSIGMA 9
@@ -210,7 +212,9 @@ int ste_process_f64(int32_t model, int32_t n, int32_t n_tracks, int64_t ld, cons
  * everywhere else (element (plane, t) at base[plane * ld + t]); matrices are row-major n x n planes.  The arithmetic is
  * that of ste_ukf_predict_n_f64 / ste_ukf_update_n_f64 / ste_urtss_backward_n_f64: every track is bit-identical to those
  * single-step kernels driven step by step.  No gating, full (not packed) covariances.  H, Q, R, P0: reference
- * UnscentedKalmanFilter.__init__ (unscented.py:20-74), row-major n x n in the first n*n entries; Q, R, P0 symmetric. */
+ * UnscentedKalmanFilter.__init__ (unscented.py:20-74), row-major n x n in the first n*n entries; Q, R, P0 symmetric.
+ * Q and R are shared by the tracks of a launch unless the _noise_ entry points below give each track its own
+ * (SteNoiseN): such a track is bit-identical to the single-step kernels run with its matrices. */
 typedef struct SteProblemN {
     int32_t n;             /* state dimension: 5                                            */
     int32_t model;         /* STE_MODEL_GEODETIC_TURN                                       */
@@ -260,6 +264,22 @@ int ste_ukf_forward_n_f64(const SteProblemN *prob, const SteInputsN *in, SteOutp
 /* UnscentedKalmanFilter.rts_step (unscented.py:267-351) for T ragged tracks: track t has n_steps[t] + 1 states and
  * reads rate[step / rate_repeat[t]]; reads mean_f / cov_f, writes mean_s / cov_s. */
 int ste_urtss_backward_tracks_n_f64(const SteProblemN *prob, const SteInputsN *in, SteOutputsN *out, void *stream);
+
+/* Per-track process and measurement noise for fleets that mix ship classes: the two passes above with each track's own
+ * Q and R.  The planes are row-major n x n in the layout of SteInputsN.P0, element (i, j) of track t at
+ * base[(i * n + j) * ld + t]; each replaces SteProblemN.Q / R for its track, noise tapes included (scaled by that
+ * track's sqrt(diag Q) / sqrt(diag R)).  A NULL pointer, or noise == NULL, keeps the launch's shared matrix, and then the
+ * call is the entry point above.  The backward pass reads Q_tracks only.  The planes must be symmetric: the library
+ * cannot read device memory before the launch, so the caller checks it (the Python layer, batch_n.TrackBatchN, does).
+ * These are separate entry points so that SteInputsN, and every binary built against it, stays as it was. */
+typedef struct SteNoiseN {
+    const double *Q_tracks;   /* [n*n][ld] per-track process noise, or NULL -> SteProblemN.Q     */
+    const double *R_tracks;   /* [n*n][ld] per-track measurement noise, or NULL -> SteProblemN.R */
+} SteNoiseN;
+int ste_ukf_forward_noise_n_f64(const SteProblemN *prob, const SteInputsN *in, const SteNoiseN *noise, SteOutputsN *out,
+                                void *stream);
+int ste_urtss_backward_tracks_noise_n_f64(const SteProblemN *prob, const SteInputsN *in, const SteNoiseN *noise,
+                                          SteOutputsN *out, void *stream);
 
 /* UnscentedKalmanFilter.criterion_index and the denominator of update_lambda_factor
  * (unscented.py:389-483) for T filters: with y = z - x (not z - Hx, no angle wrap) and

@@ -3,8 +3,9 @@
 The state is ``[lon, lat, SOG, COG, COG rate]``, the turn rate a state that persists (the model behind
 ``UnscentedKalmanFilter(..., non_linear_process=geodetic_dynamics_turn)``).  :class:`TrackBatchN` is the
 structure-of-arrays tile (track index fastest), :class:`BatchedUKFN` launches one whole-track forward
-kernel and one ragged backward kernel per tile (``ste_ukf_forward_n_f64`` /
-``ste_urtss_backward_tracks_n_f64``) and :class:`TrackResultsN` carries the per-step states back.
+kernel and one ragged backward kernel per tile (``ste_ukf_forward_noise_n_f64`` /
+``ste_urtss_backward_tracks_noise_n_f64``, with per-track ``Q`` / ``R`` when the tile has them) and
+:class:`TrackResultsN` carries the per-step states back.
 
 Every track is bit-identical to the dimension-generic single-step kernels driven step by step (the
 class API's ``predict`` / ``update``) and to ``ste_urtss_backward_n_f64`` on that track alone: the
@@ -31,7 +32,8 @@ NS = 5   # state dimension of geodetic_dynamics_turn
 #: step, five observation rows and two rates per fix; 120 B more with noise tapes).  The pipelined host path keeps two
 #: input and two result sets resident, plus 80 B of diagonal scratch per state and set for ``outputs="cli"``:
 #: 1e8 states take 2 x 48 GB + 2 x 6.5 GB (+ 24 GB with tapes) + 16 GB = 125 GB (149 GB) of a B200's 180 GB.
-#: The n = 4 budget, 4e8 states, would need 384 GB for the two result sets alone.
+#: The n = 4 budget, 4e8 states, would need 384 GB for the two result sets alone.  Per-track ``Q`` / ``R`` add 400 B per
+#: TRACK, not per state (25 doubles each, per input set): a tile of 1e8 states in 1e6 tracks carries 0.8 GB more.
 STATE_BUDGET = 100_000_000
 
 
@@ -40,6 +42,21 @@ def _as55(name: str, M) -> np.ndarray:
     if M.shape != (NS, NS):
         raise ValueError(f"{name} has shape {M.shape}: the five-state path takes 5 x 5 matrices")
     return np.ascontiguousarray(M)
+
+
+def noise_planes(name: str, mats: Sequence, T: int) -> np.ndarray:
+    """``[25][T]`` row-major planes of one symmetric 5 x 5 matrix per track (the layout of ``SteNoiseN.Q_tracks`` /
+    ``R_tracks``); ``ValueError`` for a wrong count, shape or a non-symmetric matrix.  The kernels cannot check
+    symmetry, so every per-track noise matrix passes through here."""
+    if len(mats) != T:
+        raise ValueError(f"{name}: {len(mats)} matrices for {T} tracks (one 5 x 5 matrix per track)")
+    out = np.empty((NS * NS, T))
+    for i, M in enumerate(mats):
+        M = _as55(f"{name}[{i}]", M)
+        if not np.array_equal(M, M.T):
+            raise ValueError(f"{name}[{i}] must be symmetric")
+        out[:, i] = M.reshape(-1)
+    return out
 
 
 @dataclass
@@ -58,11 +75,16 @@ class TrackBatchN:
     noise_pred: Optional[torch.Tensor] = None  # [max_steps][5][T] unit normals
     noise_upd: Optional[torch.Tensor] = None  # [max_obs][5][T], row = update index
     noise_bwd: Optional[torch.Tensor] = None  # [max_steps][5][T], row = backward step
+    # per-track noise, row-major 5 x 5 planes replacing the filter's shared matrix for each track (symmetric: from_tracks
+    # and from_batch check it; check() cannot without a device synchronisation)
+    Q: Optional[torch.Tensor] = None  # [25][T] process noise
+    R: Optional[torch.Tensor] = None  # [25][T] measurement noise
     n_steps_host: Optional[np.ndarray] = None
     # column j holds the caller's track order[j] (ragged tiles are packed by decreasing length); None = caller's order
     order: Optional[np.ndarray] = None
 
-    _TENSORS = ("x0", "dt", "upd_mask", "n_steps", "sog_rate", "cog_rate", "rate_repeat", "P0", "noise_pred", "noise_upd", "noise_bwd")
+    _TENSORS = ("x0", "dt", "upd_mask", "n_steps", "sog_rate", "cog_rate", "rate_repeat", "P0", "noise_pred", "noise_upd", "noise_bwd",
+                "Q", "R")
 
     @property
     def n_tracks(self) -> int:
@@ -94,7 +116,8 @@ class TrackBatchN:
                   ("n_steps", self.n_steps, (T,), torch.int32), ("sog_rate", self.sog_rate, (M, T), f64),
                   ("cog_rate", self.cog_rate, (M, T), f64), ("rate_repeat", self.rate_repeat, (T,), torch.int32),
                   ("P0", self.P0, (NS * NS, T), f64), ("noise_pred", self.noise_pred, (N, NS, T), f64),
-                  ("noise_upd", self.noise_upd, (M, NS, T), f64), ("noise_bwd", self.noise_bwd, (N, NS, T), f64)]
+                  ("noise_upd", self.noise_upd, (M, NS, T), f64), ("noise_bwd", self.noise_bwd, (N, NS, T), f64),
+                  ("Q", self.Q, (NS * NS, T), f64), ("R", self.R, (NS * NS, T), f64)]
         if len(self.z) != NS:
             raise ValueError("TrackBatchN.z must list the five observation rows (None for an absent row)")
         expect += [(f"z[{r}]", zr, (M, T), f64) for r, zr in enumerate(self.z)]
@@ -148,7 +171,7 @@ class TrackBatchN:
     def fleet_tiles(cls, tracks: Sequence, dt_arrays: Sequence[np.ndarray], x0: Optional[Sequence[np.ndarray]] = None,
                     time0: float = 0.0, noise: Optional[Sequence[Optional[Dict[str, np.ndarray]]]] = None, smoother: bool = True,
                     device="cuda", P0: Optional[Sequence[np.ndarray]] = None, state_budget: Optional[int] = None,
-                    **plan) -> List["TrackBatchN"]:
+                    Q: Optional[Sequence[np.ndarray]] = None, R: Optional[Sequence[np.ndarray]] = None, **plan) -> List["TrackBatchN"]:
         """A fleet too large for one tile, as tiles of :meth:`from_tracks` (same arguments): the tracks are sorted once
         by decreasing length and cut by ``sharding.plan_ragged_tiles`` (``state_budget`` stored states per tile,
         default :data:`STATE_BUDGET`; ``plan``: its ``granule`` / ``max_tracks``).  Column j of a tile holds the
@@ -157,6 +180,9 @@ class TrackBatchN:
 
         if len(tracks) == 0:
             raise ValueError("empty batch")
+        for name, mats in (("Q", Q), ("R", R)):
+            if mats is not None:
+                noise_planes(name, mats, len(tracks))   # errors name the caller's index, before any tile is built
         dt_arrays = [np.asarray(d, dtype=np.float64).reshape(-1) for d in dt_arrays]
         order = length_order([len(d) for d in dt_arrays])
         order = np.arange(len(tracks)) if order is None else order
@@ -166,7 +192,7 @@ class TrackBatchN:
             idx = order[lo:hi]
             pick = lambda seq: None if seq is None else [seq[j] for j in idx]   # noqa: E731
             tile = cls.from_tracks(pick(tracks), pick(dt_arrays), x0=pick(x0), time0=time0, noise=pick(noise), smoother=smoother,
-                                   sort_by_length=False, device=device, P0=pick(P0))
+                                   sort_by_length=False, device=device, P0=pick(P0), Q=pick(Q), R=pick(R))
             tile.order = np.array(idx)
             tiles.append(tile)
         return tiles
@@ -175,16 +201,21 @@ class TrackBatchN:
     @classmethod
     def from_tracks(cls, tracks: Sequence, dt_arrays: Sequence[np.ndarray], x0: Optional[Sequence[np.ndarray]] = None,
                     time0: float = 0.0, noise: Optional[Sequence[Optional[Dict[str, np.ndarray]]]] = None, smoother: bool = True,
-                    sort_by_length: bool = True, device="cuda", P0: Optional[Sequence[np.ndarray]] = None) -> "TrackBatchN":
+                    sort_by_length: bool = True, device="cuda", P0: Optional[Sequence[np.ndarray]] = None,
+                    Q: Optional[Sequence[np.ndarray]] = None, R: Optional[Sequence[np.ndarray]] = None) -> "TrackBatchN":
         """Pack ``ShipTrack``-like objects (``dts, z, sog_rate, cog_rate``) with their step grids, as
         :meth:`TrackBatch.from_tracks` does.  ``z`` has 4 or 5 rows and is zero-padded to 5; the default
         ``x0`` is its padded first column.  ``noise``: per track ``None`` or a dict of unit normals
         ``pred (n_steps, 5)``, ``upd (n_updates, 5)``, ``bwd (n_steps, 5)`` (backward tape indexed by step).
         ``P0``: one 5 x 5 prior covariance per track instead of the filter's shared one (used as given, e.g. the
-        not exactly symmetric covariance a previous run ended with).  Raises ``IndexError`` where the reference would."""
+        not exactly symmetric covariance a previous run ended with).  ``Q`` / ``R``: one symmetric 5 x 5 process /
+        measurement noise matrix per track, in the caller's order, instead of the filter's shared one (each track then
+        equals a filter built with its own matrices; ``ValueError`` for a wrong count, shape or an asymmetric matrix).
+        Raises ``IndexError`` where the reference would."""
         T = len(tracks)
         if T == 0:
             raise ValueError("empty batch")
+        planes = {name: noise_planes(name, mats, T) for name, mats in (("Q", Q), ("R", R)) if mats is not None}
         dt_arrays = [np.asarray(d, dtype=np.float64).reshape(-1) for d in dt_arrays]
         order = length_order([len(d) for d in dt_arrays]) if sort_by_length else None
         if order is not None:
@@ -193,6 +224,7 @@ class TrackBatchN:
             x0 = None if x0 is None else [x0[j] for j in order]
             noise = None if noise is None else [noise[j] for j in order]
             P0 = None if P0 is None else [P0[j] for j in order]
+            planes = {name: pl[:, order] for name, pl in planes.items()}
         nsteps = np.array([len(d) for d in dt_arrays], dtype=np.int32)
         nobs = np.array([np.asarray(tr.z).shape[1] for tr in tracks], dtype=np.int32)
         N, M = max(int(nsteps.max()), 1), int(nobs.max())
@@ -216,7 +248,7 @@ class TrackBatchN:
         def up(a):
             return torch.from_numpy(np.ascontiguousarray(a)).to(dev)
 
-        kw = {}
+        kw = {name: up(pl) for name, pl in planes.items()}
         if P0 is not None:
             kw["P0"] = up(np.stack([_as55("P0", Pi) for Pi in P0], axis=-1).reshape(NS * NS, T))
         if noise is not None:
@@ -235,16 +267,24 @@ class TrackBatchN:
                    order=order, **kw)
 
     @classmethod
-    def from_batch(cls, b: TrackBatch, turn_rate0: float = 0.0) -> "TrackBatchN":
+    def from_batch(cls, b: TrackBatch, turn_rate0: float = 0.0, Q: Optional[Sequence[np.ndarray]] = None,
+                   R: Optional[Sequence[np.ndarray]] = None) -> "TrackBatchN":
         """The five-state tile of an n = 4 tile already on the device (e.g. ``read_csv_fleet_device(...).to_batch()``):
         step grid, rates, observation rows, lengths and order are shared; the turn rate starts at ``turn_rate0``.  A
         tile in the cadence form (``upd_mask`` / ``n_steps`` / ``rate_repeat`` None) has them materialised on the
-        device from ``substeps`` / ``rate_repeat_all``.  No host round trip."""
+        device from ``substeps`` / ``rate_repeat_all``.  No host round trip.  ``Q`` / ``R``: one symmetric 5 x 5
+        matrix per ship, in the caller's (ship) order, checked as by :meth:`from_tracks`; column j gets the matrix of
+        ship ``b.order[j]``."""
         b.check()
         for name in ("P0", "R", "noise_pred", "noise_upd", "noise_bwd"):
             if getattr(b, name) is not None:
                 raise ValueError(f"TrackBatch.{name} is 4-state data; build the five-state tile with TrackBatchN.from_tracks")
         dev, T, N = b.device, b.n_tracks, b.max_steps
+        kw = {}
+        for name, mats in (("Q", Q), ("R", R)):
+            if mats is not None:
+                pl = noise_planes(name, mats, T)
+                kw[name] = torch.from_numpy(np.ascontiguousarray(pl if b.order is None else pl[:, b.order])).to(dev)
         x0 = torch.cat([b.x0, torch.full((1, T), float(turn_rate0), dtype=torch.float64, device=dev)]).contiguous()
         mask = b.upd_mask
         if mask is None:
@@ -254,7 +294,7 @@ class TrackBatchN:
         n_steps = b.n_steps if b.n_steps is not None else torch.full((T,), N, dtype=torch.int32, device=dev)
         rep = b.rate_repeat if b.rate_repeat is not None else torch.full((T,), max(int(b.rate_repeat_all), 1), dtype=torch.int32, device=dev)
         return cls(x0=x0, dt=b.dt, upd_mask=mask, n_steps=n_steps, sog_rate=b.sog_rate, cog_rate=b.cog_rate, z=list(b.z) + [None],
-                   rate_repeat=rep, n_steps_host=b.n_steps_host, order=b.order)
+                   rate_repeat=rep, n_steps_host=b.n_steps_host, order=b.order, **kw)
 
 
 @dataclass
@@ -400,6 +440,10 @@ class BatchedUKFN:
         return i
 
     @staticmethod
+    def _noise(b: TrackBatchN) -> nat.SteNoiseN:
+        return nat.SteNoiseN(nat.ptr(b.Q), nat.ptr(b.R))
+
+    @staticmethod
     def _outputs(r: TrackResultsN) -> nat.SteOutputsN:
         o = nat.SteOutputsN()
         o.mean_f, o.cov_f, o.mean_s, o.cov_s = nat.ptr(r.mean_f), nat.ptr(r.cov_f), nat.ptr(r.mean_s), nat.ptr(r.cov_s)
@@ -436,7 +480,8 @@ class BatchedUKFN:
         p, i, o = self._problem(b), self._inputs(b), self._outputs(res)
         res.filtered_by = id(b)
         with torch.cuda.device(b.device):
-            nat.check(self._lib.ste_ukf_forward_n_f64(C.byref(p), C.byref(i), C.byref(o), nat.current_stream()))
+            nat.check(self._lib.ste_ukf_forward_noise_n_f64(C.byref(p), C.byref(i), C.byref(self._noise(b)), C.byref(o),
+                                                            nat.current_stream()))
 
     def backward(self, b: TrackBatchN, res: TrackResultsN) -> None:
         """Launch the URTSS backward pass over the filtered states in ``res`` (written by ``forward(b, res)``)."""
@@ -447,7 +492,8 @@ class BatchedUKFN:
             raise ValueError("the smoother needs TrackBatchN.rate_repeat (from_tracks(..., smoother=True))")
         p, i, o = self._problem(b), self._inputs(b), self._outputs(res)
         with torch.cuda.device(b.device):
-            nat.check(self._lib.ste_urtss_backward_tracks_n_f64(C.byref(p), C.byref(i), C.byref(o), nat.current_stream()))
+            nat.check(self._lib.ste_urtss_backward_tracks_noise_n_f64(C.byref(p), C.byref(i), C.byref(self._noise(b)), C.byref(o),
+                                                                      nat.current_stream()))
 
     def run(self, b: TrackBatchN, smoother: bool = True, res: Optional[TrackResultsN] = None) -> TrackResultsN:
         res = res if res is not None else self.allocate(b, smoother=smoother)

@@ -5,7 +5,7 @@ from __future__ import annotations
 import os
 import time
 from concurrent.futures import ThreadPoolExecutor
-from typing import Optional, Sequence
+from typing import Mapping, Optional, Sequence
 
 import numpy as np
 
@@ -167,7 +167,7 @@ def _write_fleet_outputs_device(prefix, fleet, results, substeps, directory, shi
 def estimate_fleet(track_file: str, settings: dict, id_col: str = "id", lat_col: str = "lat", lon_col: str = "lon",
                    ship_ids: Optional[Sequence] = None, reverse: bool = False, apply_rts_smoother: bool = False,
                    output_prefix: str = "output", directory: str = ".", device="cuda", geodesy: str = "wgs84", min_fixes: int = 3,
-                   tile_plan: Optional[dict] = None, formatter: str = "host"):
+                   tile_plan: Optional[dict] = None, formatter: str = "host", ship_settings: Optional[Mapping[str, Mapping]] = None):
     """``track_estimator`` for every ship of a CSV at once: one parse (``ingest.read_csv_fleet``), SOG /
     COG / rates on the device (the CLI's default WGS84 pair, its box smoothing), one filter launch and
     one smoother launch for the whole fleet, then the CLI's files per ship.  ``settings`` is the
@@ -181,23 +181,33 @@ def estimate_fleet(track_file: str, settings: dict, id_col: str = "id", lat_col:
     (``batch_n.STATE_BUDGET`` stored states; ``tile_plan``: other keyword arguments of
     ``sharding.plan_ragged_tiles``) runs tile by tile, each tile's files written before the next tile runs;
     ``results`` is then None.  ``ValueError`` when no ship has ``min_fixes`` fixes.  ``formatter``: that of
-    :func:`write_fleet_outputs` (``"device"`` formats the files on the GPU)."""
+    :func:`write_fleet_outputs` (``"device"`` formats the files on the GPU).
+
+    ``ship_settings`` (``dim: 5``) maps a ship id to its own noise, ``{"Q": ..., "R": ...}`` (either or both) in the
+    ``input.json`` matrix format: those ships get what the class API gives with that ``Q`` / ``R``, the others the
+    file's.  It is checked before any device work: an id the file does not hold or another key raises ``ValueError``,
+    a matrix of the wrong dimension what ``input.json`` would raise, an asymmetric one ``ValueError``, and ``dim: 4``
+    ``NotImplementedError``."""
     from .main_cli import get_input_settings
 
     _check_formatter(formatter)
     dim, dt, nsteps, H, Q, R, P, smooth_control = get_input_settings(settings)
     if dim not in (4, 5):
         raise NotImplementedError("the CUDA path implements the 4-state geodetic model and the 5-state turn-rate model")
+    overrides = _ship_noise(ship_settings, dim)
     from ..ingest import read_csv_fleet
 
     fleet = read_csv_fleet(track_file, id_col=id_col, lat_col=lat_col, lon_col=lon_col, ship_ids=ship_ids, reverse=reverse,
                            on_bad_rows="skip")
+    unknown = sorted(set(overrides) - set(fleet.ids))
+    if unknown:
+        raise ValueError(f"ship_settings names ships that are not in {track_file!r}: {unknown}")
     fleet = fleet.select([i for i in range(fleet.n_tracks) if fleet.n_obs[i] >= min_fixes])
     substeps = nsteps if dt in [-1, 0, None] else 1                       # main_cli.py:114-117
     width = smooth_control if smooth_control not in [-1, 0, 1, None] else 0   # main_cli.py:99-104
     if dim == 5:
         return fleet, _estimate_fleet_n5(fleet, H, Q, R, P, substeps, width, apply_rts_smoother, output_prefix, directory, device,
-                                         geodesy, tile_plan or {}, formatter)
+                                         geodesy, tile_plan or {}, formatter, overrides)
     from ..batch import BatchedUKF
 
     ukf = BatchedUKF(H, Q, R, P)
@@ -208,7 +218,30 @@ def estimate_fleet(track_file: str, settings: dict, id_col: str = "id", lat_col:
     return fleet, results
 
 
-def _estimate_fleet_n5(fleet, H, Q, R, P, substeps, width, smoother, prefix, directory, device, geodesy, tile_plan, formatter):
+def _ship_noise(ship_settings: Optional[Mapping[str, Mapping]], dim: int) -> dict:
+    """``{str(ship id): {"Q": 5 x 5, "R": 5 x 5}}`` (either key) from ``estimate_fleet``'s ``ship_settings``."""
+    if not ship_settings:
+        return {}
+    if dim != 5:
+        raise NotImplementedError("ship_settings needs dim: 5; the n = 4 path takes a per-track R through "
+                                  "TrackBatch.from_tracks(R=...) but has no per-track Q")
+    from ..batch_n import noise_planes
+    from .main_cli import _get_input_matrix
+
+    out = {}
+    for sid, entry in ship_settings.items():
+        extra = sorted(set(entry) - {"Q", "R"})
+        if extra:
+            raise ValueError(f"ship_settings[{sid!r}]: unknown keys {extra} (per-ship settings take Q and R)")
+        mats = {name: _get_input_matrix(entry, name, dim).astype(np.float64) for name in ("Q", "R") if name in entry}
+        for name, M in mats.items():
+            noise_planes(f"ship_settings[{sid!r}].{name}", [M], 1)   # ValueError unless symmetric
+        out[str(sid)] = mats
+    return out
+
+
+def _estimate_fleet_n5(fleet, H, Q, R, P, substeps, width, smoother, prefix, directory, device, geodesy, tile_plan, formatter,
+                       overrides):
     import numpy as np
 
     from ..batch_n import STATE_BUDGET, BatchedUKFN, TrackBatchN
@@ -224,11 +257,15 @@ def _estimate_fleet_n5(fleet, H, Q, R, P, substeps, width, smoother, prefix, dir
     steps = (fleet.n_obs[order].astype(np.int64) - 1) * substeps
     plan = dict(tile_plan)
     tiles = plan_ragged_tiles(steps, plan.pop("state_budget", STATE_BUDGET), **plan)
+    # per-ship matrices in the fleet's ship order, for the kinds some ship overrides (the others stay shared)
+    own = {name: [overrides.get(sid, {}).get(name, M) for sid in fleet.ids] for name, M in (("Q", Q), ("R", R))
+           if any(name in o for o in overrides.values())}
     results = None
     for lo, hi in tiles:
         ships = order[lo:hi] if len(tiles) > 1 else None
         part = fleet if ships is None else fleet.select(ships)
-        res = ukf.run(TrackBatchN.from_batch(part.to_batch(**kw)), smoother=smoother)
+        noise = {name: (mats if ships is None else [mats[i] for i in ships]) for name, mats in own.items()}
+        res = ukf.run(TrackBatchN.from_batch(part.to_batch(**kw), **noise), smoother=smoother)
         res.check_status()   # IndexError / FloatingPointError where the per-ship reference run would fail
         write_fleet_outputs(prefix, part, res, substeps, directory, formatter=formatter)
         results = res if ships is None else None

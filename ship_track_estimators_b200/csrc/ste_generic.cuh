@@ -114,11 +114,11 @@ struct ProblemN {
     double H[kMaxN * kMaxN], Q[kMaxN * kMaxN], R[kMaxN * kMaxN];
 };
 
-// UnscentedKalmanFilter.predict (unscented.py:144-207) on a thread-local state: x [n], P [n][D] in place.
-// noise: unit normals noise[r * ns] or NULL; sigma_prior / sigma_post: planes [n*(2n+1)] at stride ss, or NULL.
-// Returns STE_STATUS_* bits.
+// UnscentedKalmanFilter.predict (unscented.py:144-207) on a thread-local state: x [n], P [n][D] in place; Q row-major
+// n x n (p.Q, or a track's own).  noise: unit normals noise[r * ns] or NULL, scaled by sqrt(diag Q); sigma_prior /
+// sigma_post: planes [n*(2n+1)] at stride ss, or NULL.  Returns STE_STATUS_* bits.
 template <int NC>
-STE_DEV int predict_core(const ProblemN &p, double *x, double *P, double d, double sr, double cr, const double *noise, int64_t ns,
+STE_DEV int predict_core(const ProblemN &p, const double *Q, double *x, double *P, double d, double sr, double cr, const double *noise, int64_t ns,
                          double *sigma_prior, double *sigma_post, int64_t ss) {
     constexpr int D = DimN<NC>::LD, DL = DimN<NC>::LL;
     const int n = NC > 0 ? NC : p.n, L = 2 * n + 1;
@@ -144,14 +144,14 @@ STE_DEV int predict_core(const ProblemN &p, double *x, double *P, double d, doub
     for (int r = 0; r < n; ++r) {
         double acc = w0 * Y[r * DL];
         for (int j = 1; j < L; ++j) acc = fma(wi, Y[r * DL + j], acc);
-        mean[r] = acc + (noise ? noise[r * ns] * sqrt(p.Q[r * n + r]) : 0.0);   // :195-202
+        mean[r] = acc + (noise ? noise[r * ns] * sqrt(Q[r * n + r]) : 0.0);   // :195-202
     }
     bool bad = false;
     for (int r = 0; r < n; ++r) {
         for (int q = 0; q < n; ++q) {
             double acc = w0 * (Y[r * DL] - mean[r]) * (Y[q * DL] - mean[q]);
             for (int j = 1; j < L; ++j) acc = fma(wi * (Y[r * DL + j] - mean[r]), Y[q * DL + j] - mean[q], acc);
-            const double v = acc + p.Q[r * n + q];   // :205-207, about the noisy mean
+            const double v = acc + Q[r * n + q];   // :205-207, about the noisy mean
             P[r * D + q] = v;
             bad |= !(v * 0.0 == 0.0);
         }
@@ -162,13 +162,14 @@ STE_DEV int predict_core(const ProblemN &p, double *x, double *P, double d, doub
 }
 
 // UnscentedKalmanFilter.update (unscented.py:209-265) on a thread-local state, dense H and R: x [n], P [n][D] in place;
-// zin [n] the observation, noise unit normals noise[r * ns] or NULL.  Returns STE_STATUS_* bits.
+// R row-major n x n (p.R, or a track's own); zin [n] the observation, noise unit normals noise[r * ns] or NULL, scaled
+// by sqrt(diag R).  Returns STE_STATUS_* bits.
 template <int NC>
-STE_DEV int update_core(const ProblemN &p, double *x, double *P, const double *zin, const double *noise, int64_t ns) {
+STE_DEV int update_core(const ProblemN &p, const double *R, double *x, double *P, const double *zin, const double *noise, int64_t ns) {
     constexpr int D = DimN<NC>::LD;
     const int n = NC > 0 ? NC : p.n;
     double z[D], y[D], PHt[D * D], S[D * D], Si[D * D], K[D * D], A[D * D], AP[D * D];
-    for (int r = 0; r < n; ++r) z[r] = zin[r] + (noise ? noise[r * ns] * sqrt(p.R[r * n + r]) : 0.0);   // :232-236
+    for (int r = 0; r < n; ++r) z[r] = zin[r] + (noise ? noise[r * ns] * sqrt(R[r * n + r]) : 0.0);   // :232-236
     for (int i = 0; i < n; ++i)
         for (int j = 0; j < n; ++j) {
             double acc = 0.0;
@@ -177,7 +178,7 @@ STE_DEV int update_core(const ProblemN &p, double *x, double *P, const double *z
         }
     for (int i = 0; i < n; ++i)
         for (int j = 0; j < n; ++j) {
-            double acc = p.R[i * n + j];
+            double acc = R[i * n + j];
             for (int k = 0; k < n; ++k) acc = fma(p.H[i * n + k], PHt[k * D + j], acc);
             S[i * D + j] = acc;
         }
@@ -216,7 +217,7 @@ STE_DEV int update_core(const ProblemN &p, double *x, double *P, const double *z
     for (int i = 0; i < n; ++i)
         for (int j = 0; j < n; ++j) {
             double acc = 0.0;
-            for (int k = 0; k < n; ++k) acc = fma(K[i * D + k], p.R[k * n + j], acc);
+            for (int k = 0; k < n; ++k) acc = fma(K[i * D + k], R[k * n + j], acc);
             PHt[i * D + j] = acc;
         }
     bool bad = false;
@@ -243,7 +244,7 @@ STE_DEV void predict_n(const ProblemN &p, int t, double *x_io, double *P_io, con
     for (int i = 0; i < n; ++i)
         for (int j = 0; j < n; ++j) P[i * kMaxN + j] = P_io[(i * n + j) * ld + t];
     const double d = dt[t], sr = sog_rate ? sog_rate[t] : 0.0, cr = cog_rate ? cog_rate[t] : 0.0;
-    const int st = predict_core<0>(p, x, P, d, sr, cr, noise ? noise + t : nullptr, ld, sigma_prior ? sigma_prior + t : nullptr,
+    const int st = predict_core<0>(p, p.Q, x, P, d, sr, cr, noise ? noise + t : nullptr, ld, sigma_prior ? sigma_prior + t : nullptr,
                                    sigma_post ? sigma_post + t : nullptr, ld);
     for (int r = 0; r < n; ++r) {
         for (int q = 0; q < n; ++q) P_io[(r * n + q) * ld + t] = P[r * kMaxN + q];
@@ -262,7 +263,7 @@ STE_DEV void update_n(const ProblemN &p, int t, double *x_io, double *P_io, cons
         z[r] = z_in[r * ld + t];
         for (int q = 0; q < n; ++q) P[r * kMaxN + q] = P_io[(r * n + q) * ld + t];
     }
-    const int st = update_core<0>(p, x, P, z, noise ? noise + t : nullptr, ld);
+    const int st = update_core<0>(p, p.R, x, P, z, noise ? noise + t : nullptr, ld);
     for (int i = 0; i < n; ++i) {
         for (int j = 0; j < n; ++j) P_io[(i * n + j) * ld + t] = P[i * kMaxN + j];
         x_io[i * ld + t] = x[i];
@@ -275,9 +276,10 @@ STE_DEV void update_n(const ProblemN &p, int t, double *x_io, double *P_io, cons
 // [n_rates][ld], indexed by step / rate_repeat as the reference's np.repeat expansion does (:287-292); noise [S-1][n][ld]
 // unit normals in step order or NULL.  The last state is copied (the loop starts at S - 2, :297).  Arithmetic written
 // literally after the reference: P_b about the FILTERED mean (:324-325), the cross covariance about the noisy x_b
-// (:328-330), pinv(P_b), state index 3 wrapped as the heading (:340, 346).  Returns STE_STATUS_* bits.
+// (:328-330), pinv(P_b), state index 3 wrapped as the heading (:340, 346).  Q row-major n x n (p.Q, or the track's own),
+// the noise scaled by sqrt(diag Q).  Returns STE_STATUS_* bits.
 template <int NC>
-STE_DEV int rts_n(const ProblemN &p, int t, int n_states, int rate_repeat, int n_rates, const double *mean_f, const double *cov_f,
+STE_DEV int rts_n(const ProblemN &p, const double *Q, int t, int n_states, int rate_repeat, int n_rates, const double *mean_f, const double *cov_f,
                   const double *dt, const double *sog_rate, const double *cog_rate, const double *noise, double *mean_s,
                   double *cov_s) {
     constexpr int D = DimN<NC>::LD, DL = DimN<NC>::LL;
@@ -324,7 +326,7 @@ STE_DEV int rts_n(const ProblemN &p, int t, int n_states, int rate_repeat, int n
         for (int r = 0; r < n; ++r) {
             double acc = w0 * Y[r * DL];
             for (int j = 1; j < L; ++j) acc = fma(wi, Y[r * DL + j], acc);
-            xb[r] = acc + (noise ? noise[((int64_t)step * n + r) * ld + t] * sqrt(p.Q[r * n + r]) : 0.0);   // :313-322
+            xb[r] = acc + (noise ? noise[((int64_t)step * n + r) * ld + t] * sqrt(Q[r * n + r]) : 0.0);   // :313-322
         }
         for (int r = 0; r < n; ++r)
             for (int q = 0; q < n; ++q) {
@@ -334,7 +336,7 @@ STE_DEV int rts_n(const ProblemN &p, int t, int n_states, int rate_repeat, int n
                     pb = fma(wi * (Y[r * DL + j] - xf[r]), Y[q * DL + j] - xf[q], pb);
                     dd = fma(wi * (X[r * DL + j] - xf[r]), Y[q * DL + j] - xb[q], dd);
                 }
-                Pb[r * D + q] = pb + p.Q[r * n + q];
+                Pb[r * D + q] = pb + Q[r * n + q];
                 Dc[r * D + q] = dd;
             }
         fun_sym_n<NC>(n, Pb, true, Pbi);

@@ -498,7 +498,7 @@ __global__ void __launch_bounds__(64) urtss_backward_n_kernel(const __grid_const
                                                              double *mean_s, double *cov_s, int32_t *status) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= p.n_tracks) return;
-    const int st = rts_n<0>(p, t, n_states, rate_repeat, n_rates, mean_f, cov_f, dt, sog_rate, cog_rate, noise, mean_s, cov_s);
+    const int st = rts_n<0>(p, p.Q, t, n_states, rate_repeat, n_rates, mean_f, cov_f, dt, sog_rate, cog_rate, noise, mean_s, cov_s);
     if (status) status[t] = st;
 }
 
@@ -519,11 +519,25 @@ struct FleetArgsN {
     int32_t max_steps, max_obs;
     SteInputsN in;
     SteOutputsN out;
+    SteNoiseN noise;   // per-track Q / R planes, or NULL (last, so the shared path's parameter offsets stay as they were)
 };
+
+// Q and R of track t: with PerTrack, its own planes (noise.Q_tracks / R_tracks, the launch's matrix where one is NULL)
+// loaded once, before the time loop; otherwise the launch's matrices, read from the kernel parameters.  The host picks
+// PerTrack only when a plane set is present, so a launch without one keeps the shared path's code and registers.
+template <int NC, bool PerTrack>
+STE_DEV const double *track_matrix(const double *shared, const double *planes, int64_t ld, int t, double *own) {
+    if constexpr (PerTrack) {
+        for (int k = 0; k < NC * NC; ++k) own[k] = planes ? planes[k * ld + t] : shared[k];
+        return own;
+    } else {
+        return shared;
+    }
+}
 
 // KalmanFilterBase.run (kalman_filter.py:36-117): row 0 the prior, the initial update with observation 0, then per step
 // a predict with the rates of the current update index and, where upd_mask is set, an update with the next observation.
-template <int NC>
+template <int NC, bool PerTrack>
 __global__ void __launch_bounds__(kThreadsN) ukf_forward_n_kernel(const __grid_constant__ FleetArgsN a) {
     constexpr int D = DimN<NC>::LD, n = NC;
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
@@ -531,7 +545,9 @@ __global__ void __launch_bounds__(kThreadsN) ukf_forward_n_kernel(const __grid_c
     const SteInputsN &in = a.in;
     const int64_t ld = a.p.ld;
     const int nt = in.n_steps ? min(in.n_steps[t], a.max_steps) : a.max_steps;
-    double x[D], P[D * D], z[D];
+    double x[D], P[D * D], z[D], Qt[PerTrack ? n * n : 1], Rt[PerTrack ? n * n : 1];
+    const double *Q = track_matrix<NC, PerTrack>(a.p.Q, a.noise.Q_tracks, ld, t, Qt);
+    const double *R = track_matrix<NC, PerTrack>(a.p.R, a.noise.R_tracks, ld, t, Rt);
     for (int r = 0; r < n; ++r) x[r] = in.x0[r * ld + t];
     for (int i = 0; i < n; ++i)
         for (int j = 0; j < n; ++j) P[i * D + j] = in.P0 ? in.P0[(i * n + j) * ld + t] : a.P0[i * n + j];
@@ -543,14 +559,14 @@ __global__ void __launch_bounds__(kThreadsN) ukf_forward_n_kernel(const __grid_c
     };
     auto update = [&](int u) {   // observation row u; rows the caller left NULL read as 0
         for (int r = 0; r < n; ++r) z[r] = in.z[r] ? in.z[r][(int64_t)u * ld + t] : 0.0;
-        return update_core<NC>(a.p, x, P, z, in.noise_upd ? in.noise_upd + (int64_t)u * n * ld + t : nullptr, ld);
+        return update_core<NC>(a.p, R, x, P, z, in.noise_upd ? in.noise_upd + (int64_t)u * n * ld + t : nullptr, ld);
     };
     store(0);                      // :76-81
     int status = update(0), ui = 0;
     for (int s = 0; s < nt; ++s) {
         const double d = in.dt[(int64_t)s * ld + t], sr = in.sog_rate[(int64_t)ui * ld + t],
                      cr = in.cog_rate ? in.cog_rate[(int64_t)ui * ld + t] : 0.0;
-        status |= predict_core<NC>(a.p, x, P, d, sr, cr, in.noise_pred ? in.noise_pred + (int64_t)s * n * ld + t : nullptr, ld,
+        status |= predict_core<NC>(a.p, Q, x, P, d, sr, cr, in.noise_pred ? in.noise_pred + (int64_t)s * n * ld + t : nullptr, ld,
                                    nullptr, nullptr, 0);
         if (in.upd_mask[(int64_t)s * ld + t]) {   // :101-108
             if (ui + 1 < a.max_obs) status |= update(++ui);
@@ -563,15 +579,17 @@ __global__ void __launch_bounds__(kThreadsN) ukf_forward_n_kernel(const __grid_c
 }
 
 // UnscentedKalmanFilter.rts_step (unscented.py:267-351) over ragged tracks: n_states = n_steps[t] + 1 and rate_repeat[t]
-// per track; the status bits are OR-ed into the forward pass's.
-template <int NC>
+// per track; the status bits are OR-ed into the forward pass's.  Q as in the forward pass (PerTrack: noise.Q_tracks set).
+template <int NC, bool PerTrack>
 __global__ void __launch_bounds__(kThreadsN) urtss_backward_n_tracks_kernel(const __grid_constant__ FleetArgsN a) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= a.p.n_tracks) return;
     const SteInputsN &in = a.in;
     const int nt = in.n_steps ? min(in.n_steps[t], a.max_steps) : a.max_steps;
     const int rep = max(in.rate_repeat[t], 1);
-    a.out.status[t] |= rts_n<NC>(a.p, t, nt + 1, rep, a.max_obs, a.out.mean_f, a.out.cov_f, in.dt, in.sog_rate, in.cog_rate,
+    double Qt[PerTrack ? NC * NC : 1];
+    const double *Q = track_matrix<NC, PerTrack>(a.p.Q, a.noise.Q_tracks, a.p.ld, t, Qt);
+    a.out.status[t] |= rts_n<NC>(a.p, Q, t, nt + 1, rep, a.max_obs, a.out.mean_f, a.out.cov_f, in.dt, in.sog_rate, in.cog_rate,
                                  in.noise_bwd, a.out.mean_s, a.out.cov_s);
 }
 
@@ -950,7 +968,7 @@ static int validate_fleet_n(const SteProblemN *p, const SteInputsN *in, const St
     return STE_OK;
 }
 
-static FleetArgsN fleet_args(const SteProblemN *prob, const SteInputsN *in, const SteOutputsN *out) {
+static FleetArgsN fleet_args(const SteProblemN *prob, const SteInputsN *in, const SteOutputsN *out, const SteNoiseN *noise) {
     FleetArgsN a{};
     const int n = prob->n;
     a.p.n = n; a.p.model = prob->model; a.p.n_tracks = prob->n_tracks; a.p.ld = prob->ld;
@@ -961,22 +979,41 @@ static FleetArgsN fleet_args(const SteProblemN *prob, const SteInputsN *in, cons
     a.max_steps = prob->max_steps; a.max_obs = prob->max_obs;
     a.in = *in;
     a.out = *out;
+    if (noise) a.noise = *noise;
     return a;
 }
 
 int ste_ukf_forward_n_f64(const SteProblemN *prob, const SteInputsN *in, SteOutputsN *out, void *stream) {
+    return ste_ukf_forward_noise_n_f64(prob, in, nullptr, out, stream);
+}
+
+int ste_ukf_forward_noise_n_f64(const SteProblemN *prob, const SteInputsN *in, const SteNoiseN *noise, SteOutputsN *out,
+                                void *stream) {
     if (int rc = validate_fleet_n(prob, in, out, false)) return rc;
     if (prob->n_tracks == 0) return STE_OK;
-    const FleetArgsN a = fleet_args(prob, in, out);
-    ukf_forward_n_kernel<5><<<(prob->n_tracks + kThreadsN - 1) / kThreadsN, kThreadsN, 0, (cudaStream_t)stream>>>(a);
+    const FleetArgsN a = fleet_args(prob, in, out, noise);
+    const int blocks = (prob->n_tracks + kThreadsN - 1) / kThreadsN;
+    if (a.noise.Q_tracks || a.noise.R_tracks)
+        ukf_forward_n_kernel<5, true><<<blocks, kThreadsN, 0, (cudaStream_t)stream>>>(a);
+    else
+        ukf_forward_n_kernel<5, false><<<blocks, kThreadsN, 0, (cudaStream_t)stream>>>(a);
     return check_launch("ukf_forward_n_kernel");
 }
 
 int ste_urtss_backward_tracks_n_f64(const SteProblemN *prob, const SteInputsN *in, SteOutputsN *out, void *stream) {
+    return ste_urtss_backward_tracks_noise_n_f64(prob, in, nullptr, out, stream);
+}
+
+int ste_urtss_backward_tracks_noise_n_f64(const SteProblemN *prob, const SteInputsN *in, const SteNoiseN *noise,
+                                          SteOutputsN *out, void *stream) {
     if (int rc = validate_fleet_n(prob, in, out, true)) return rc;
     if (prob->n_tracks == 0) return STE_OK;
-    const FleetArgsN a = fleet_args(prob, in, out);
-    urtss_backward_n_tracks_kernel<5><<<(prob->n_tracks + kThreadsN - 1) / kThreadsN, kThreadsN, 0, (cudaStream_t)stream>>>(a);
+    const FleetArgsN a = fleet_args(prob, in, out, noise);
+    const int blocks = (prob->n_tracks + kThreadsN - 1) / kThreadsN;
+    if (a.noise.Q_tracks)
+        urtss_backward_n_tracks_kernel<5, true><<<blocks, kThreadsN, 0, (cudaStream_t)stream>>>(a);
+    else
+        urtss_backward_n_tracks_kernel<5, false><<<blocks, kThreadsN, 0, (cudaStream_t)stream>>>(a);
     return check_launch("urtss_backward_n_tracks_kernel");
 }
 

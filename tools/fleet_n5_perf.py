@@ -2,11 +2,15 @@
 operations and HBM bytes per track-step counted from the shapes, the n = 4 BatchedUKF on the same tile for context, and
 the class API's per-step cost.  Prints one JSON line.
 
-    python tools/fleet_n5_perf.py [--tracks 151552] [--steps 256] [--reps 5] [--out profiles/fleet_n5_perf.json]
+    python tools/fleet_n5_perf.py [--tracks 151552] [--steps 256] [--reps 5] [--per-track-noise] [--out profiles/fleet_n5_perf.json]
 
 The tile is ragged (make_tracks, lengths uniform in [steps/2, steps] fixes per track at k = 1, the same step count at
 k = 2); its inputs and outputs (about 70 GB at the default size) are far above the 126 MB L2.  Needs a CUDA device: there
-is no CPU measurement."""
+is no CPU measurement.
+
+``--per-track-noise`` also runs the tile with its own Q and R per track (``TrackBatchN.Q`` / ``R``: two ship classes,
+alternate tracks, differing in the position R and the turn-rate Q) and times it against the shared-matrix tile, the two
+launches alternating in every repetition so that both see the same machine state."""
 import argparse
 import json
 import os
@@ -57,6 +61,34 @@ def time_launches(fn, reps):
         b.synchronize()
         times.append(a.elapsed_time(b) * 1e-3)
     return float(np.median(times)), float(min(times)), float(max(times))
+
+
+def time_alternating(fns, reps):
+    """Median / min / max seconds of each launch in ``fns`` (name -> callable), the launches interleaved per repetition."""
+    for fn in fns.values():
+        fn()
+    torch.cuda.synchronize()
+    times = {name: [] for name in fns}
+    for _ in range(reps):
+        for name, fn in fns.items():
+            a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            a.record()
+            fn()
+            b.record()
+            b.synchronize()
+            times[name].append(a.elapsed_time(b) * 1e-3)
+    return {name: (float(np.median(t)), float(min(t)), float(max(t))) for name, t in times.items()}
+
+
+def class_planes(T, Q, R):
+    """[25][T] planes of two ship classes on alternate tracks: the given (Q, R), and a logbook class with R = 0.25 deg^2
+    on the position and a 100x larger turn-rate Q."""
+    Q2, R2 = Q.copy(), R.copy()
+    Q2[4, 4] *= 100.0
+    R2[0, 0] = R2[1, 1] = 0.25
+    odd = (np.arange(T) % 2).astype(bool)
+    planes = lambda A, B: torch.from_numpy(np.where(odd[None, :], B.reshape(25, 1), A.reshape(25, 1))).to("cuda")   # noqa: E731
+    return planes(Q, Q2), planes(R, R2)
 
 
 def fp64_peak():
@@ -121,6 +153,7 @@ def main():
     ap.add_argument("--tracks", type=int, default=151552)
     ap.add_argument("--steps", type=int, default=256)
     ap.add_argument("--reps", type=int, default=5)
+    ap.add_argument("--per-track-noise", action="store_true", help="also time the tile with per-track Q and R")
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     if not torch.cuda.is_available():
@@ -144,8 +177,18 @@ def main():
         b = TrackBatchN.from_batch(b4, turn_rate0=0.0)
         steps = b.track_steps()
         res = engine.allocate(b)
-        fwd = time_launches(lambda: engine.forward(b, res), args.reps)
-        bwd = time_launches(lambda: engine.backward(b, res), args.reps)
+        if args.per_track_noise:
+            Qp, Rp = class_planes(b.n_tracks, engine.Q, engine.R)
+            bq = TrackBatchN(**{**b.__dict__, "Q": Qp, "R": Rp})
+            resq = engine.allocate(bq)   # a result set of its own: the smoother reads the states its tile filtered
+            fwd_all = time_alternating({"shared": lambda: engine.forward(b, res), "per_track": lambda: engine.forward(bq, resq)}, args.reps)
+            bwd_all = time_alternating({"shared": lambda: engine.backward(b, res), "per_track": lambda: engine.backward(bq, resq)}, args.reps)
+            st_q = resq.check_status(raise_on=0)
+            del resq
+            fwd, bwd = fwd_all["shared"], bwd_all["shared"]
+        else:
+            fwd = time_launches(lambda: engine.forward(b, res), args.reps)
+            bwd = time_launches(lambda: engine.backward(b, res), args.reps)
         st = res.check_status(raise_on=0)
         del res
         torch.cuda.empty_cache()
@@ -164,6 +207,13 @@ def main():
             t = row[f"{p}_s"]
             row[f"{p}_fp64_share_of_probe_peak"] = fl[p] * steps / t / peak
             row[f"{p}_hbm_share_of_datasheet"] = by[p] * steps / t / 7.7e12
+        if args.per_track_noise:
+            fq, bq_ = fwd_all["per_track"], bwd_all["per_track"]
+            row["per_track_noise"] = {"status": st_q, "forward_s": fq[0], "forward_min_max_s": fq[1:], "backward_s": bq_[0],
+                                      "backward_min_max_s": bq_[1:], "both_track_steps_per_s": steps / (fq[0] + bq_[0]),
+                                      "forward_vs_shared": fq[0] / fwd[0], "backward_vs_shared": bq_[0] / bwd[0],
+                                      "both_vs_shared": (fq[0] + bq_[0]) / (fwd[0] + bwd[0])}
+            del bq, Qp, Rp
         row["n4_batched_ukf_run_s"] = n4[0]
         row["n4_batched_ukf_track_steps_per_s"] = steps / n4[0]
         out[f"k{k}"] = row
