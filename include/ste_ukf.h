@@ -41,6 +41,8 @@ extern "C" {
                             /* 7: ste_track_metrics_n_f64 (fit metrics of the five-state fleet path)                                      */
                             /*    additive, no struct changed: SteNoiseN, ste_ukf_forward_noise_n_f64,                                    */
                             /*    ste_urtss_backward_tracks_noise_n_f64 (per-track Q / R of the five-state fleet path)                    */
+                            /*    additive, no struct changed: SteInnovations, ste_ukf_forward_innov_f64, ste_ukf_forward_innov_n_f64     */
+                            /*    (per-update innovation statistics of the forward passes)                                               */
 #define STE_STATS_PLANES 15
 #define STE_DIM 4
 #define STE_NSIGMA 9
@@ -280,6 +282,30 @@ int ste_ukf_forward_noise_n_f64(const SteProblemN *prob, const SteInputsN *in, c
                                 void *stream);
 int ste_urtss_backward_tracks_noise_n_f64(const SteProblemN *prob, const SteInputsN *in, const SteNoiseN *noise,
                                           SteOutputsN *out, void *stream);
+
+/* Innovation statistics of the forward passes, for choosing Q and R by maximum likelihood, testing a filter's
+ * consistency and flagging suspect fixes.  For update u of track t (u = 0 is the initial update with observation 0),
+ * with x-, P- the state the update receives:
+ *   y = z - H x-           z as the update uses it (after the noise-tape draw); the heading row wrapped as the update
+ *                          wraps it.  On the position-only path (H = diag(1,1,0,0)) only rows 0 and 1 take part.
+ *   S = H P- H^T + rs R    the matrix whose pseudo-inverse the update applies (rs: the robustification's scale of R,
+ *                          1 without gating; R: the track's own where one is given)
+ *   nis    = y^T S^+ y
+ *   rank   = the eigenvalues of S the pseudo-inverse keeps (|lambda| > 1e-15 max |lambda|, numpy's rule)
+ *   loglik = -1/2 (nis + sum log lambda_k + rank log 2 pi) over the kept eigenvalues; NaN when one of them is
+ *            negative (S indefinite).  No status bit changes.
+ * Element (u, t) of each plane is at base[u * ld + t]; rows at or beyond n_updates[t] are not written.  Every other
+ * output is bit-identical to the call without statistics.  innov == NULL: exactly ste_ukf_forward_f64 /
+ * ste_ukf_forward_noise_n_f64.  A non-NULL innov with a NULL plane returns STE_ERR_INVALID_ARG. */
+typedef struct SteInnovations {
+    double  *nis;     /* [max_obs][ld] y^T S^+ y per update, row = update index           */
+    double  *loglik;  /* [max_obs][ld] Gaussian log-likelihood of the update's observation */
+    uint8_t *rank;    /* [max_obs][ld] eigenvalues of S kept by the pseudo-inverse         */
+} SteInnovations;
+int ste_ukf_forward_innov_f64(const SteProblem *prob, const SteInputs *in, const SteInnovations *innov,
+                              SteOutputs *out, void *stream);
+int ste_ukf_forward_innov_n_f64(const SteProblemN *prob, const SteInputsN *in, const SteNoiseN *noise,
+                                const SteInnovations *innov, SteOutputsN *out, void *stream);
 
 /* UnscentedKalmanFilter.criterion_index and the denominator of update_lambda_factor
  * (unscented.py:389-483) for T filters: with y = z - x (not z - Hx, no angle wrap) and

@@ -121,6 +121,14 @@ class SteNoiseN(C.Structure):
     ]
 
 
+class SteInnovations(C.Structure):
+    _fields_ = [
+        ("nis", _dptr),
+        ("loglik", _dptr),
+        ("rank", _dptr),
+    ]
+
+
 class SteOutputsN(C.Structure):
     _fields_ = [
         ("mean_f", _dptr),
@@ -174,6 +182,10 @@ _PROTOTYPES = {
                                               C.c_void_p]),
     "ste_urtss_backward_tracks_noise_n_f64": (C.c_int, [C.POINTER(SteProblemN), C.POINTER(SteInputsN), C.POINTER(SteNoiseN),
                                                         C.POINTER(SteOutputsN), C.c_void_p]),
+    "ste_ukf_forward_innov_f64": (C.c_int, [C.POINTER(SteProblem), C.POINTER(SteInputs), C.POINTER(SteInnovations), C.POINTER(SteOutputs),
+                                            C.c_void_p]),
+    "ste_ukf_forward_innov_n_f64": (C.c_int, [C.POINTER(SteProblemN), C.POINTER(SteInputsN), C.POINTER(SteNoiseN), C.POINTER(SteInnovations),
+                                              C.POINTER(SteOutputsN), C.c_void_p]),
     "ste_process_f64": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int64] + [_dptr] * 5 + [C.c_void_p]),
     "ste_csv_parse_rows": (C.c_int, [_dptr, _dptr, C.c_int64, C.POINTER(C.c_int32)] + [_dptr] * 9 + [C.c_void_p]),
     "ste_gate_terms_f64": (C.c_int, [C.POINTER(SteProblem)] + [_dptr] * 5 + [C.c_void_p]),

@@ -421,6 +421,11 @@ class TrackResults:
     order: Optional[np.ndarray] = None  # TrackBatch.order of the tile these results belong to
     filtered_by: Optional[int] = field(default=None, repr=False, compare=False)  # id() of the tile last filtered into these buffers
     _column_of: Optional[np.ndarray] = field(default=None, repr=False, compare=False)
+    # innovation statistics per update (allocate(..., innovations=True)), [max_obs][T], row = update index: y^T S^+ y, the
+    # Gaussian log-likelihood of the update's observation and the rank of S^+ (include/ste_ukf.h, SteInnovations)
+    nis: Optional[torch.Tensor] = None
+    loglik: Optional[torch.Tensor] = None
+    innov_rank: Optional[torch.Tensor] = None
 
     @property
     def packed_cov(self) -> bool:
@@ -434,7 +439,8 @@ class TrackResults:
         idx = np.array([[0, 1, 2, 3], [1, 4, 5, 6], [2, 5, 7, 8], [3, 6, 8, 9]])
         return c[..., idx]
 
-    _TENSORS = ("mean_f", "cov_f", "mean_s", "cov_s", "status", "n_updates", "gate_iters", "gate_lambda", "gate_scale")
+    _TENSORS = ("mean_f", "cov_f", "mean_s", "cov_s", "status", "n_updates", "gate_iters", "gate_lambda", "gate_scale", "nis", "loglik",
+                "innov_rank")
 
     def host_like(self, pinned: bool = True) -> "TrackResults":
         """Empty host buffers of the same shapes (page-locked by default) for device->host copies."""
@@ -520,6 +526,8 @@ class TrackResults:
             out["gate_iters"] = self.gate_iters[:m, i].cpu().numpy().astype(np.int32)
             out["gate_lambda"] = self.gate_lambda[:m, i].cpu().numpy()
             out["gate_scale"] = self.gate_scale[:m, i].cpu().numpy()
+        if self.nis is not None:
+            innovation_columns(self, out, i)
         return out
 
 
@@ -601,12 +609,15 @@ class BatchedUKF:
         i.noise_pred, i.noise_upd, i.noise_bwd = nat.ptr(b.noise_pred), nat.ptr(b.noise_upd), nat.ptr(b.noise_bwd)
         return i
 
-    def allocate(self, b: TrackBatch, smoother: bool = True, in_place: bool = False, reuse_stats: bool = True) -> TrackResults:
+    def allocate(self, b: TrackBatch, smoother: bool = True, in_place: bool = False, reuse_stats: bool = True,
+                 innovations: bool = False) -> TrackResults:
         """Output buffers for a tile (caller-owned, reusable across tiles of the same shape).
 
         ``reuse_stats``: also allocate the 240 B/step tape on which the forward pass leaves the
         smoother's sigma-point statistics, so the backward pass does not recompute them (the
-        reference does).  ``False`` trades that memory for ~2x the smoother's arithmetic."""
+        reference does).  ``False`` trades that memory for ~2x the smoother's arithmetic.
+        ``innovations``: also allocate the ``nis`` / ``loglik`` / ``innov_rank`` planes ``[max_obs][T]``
+        that the forward pass then fills per update (17 B per update; see :func:`allocate_innovations`)."""
         dev, T, S = b.device, b.n_tracks, b.max_steps + 1
         f64 = dict(dtype=torch.float64, device=dev)
         C = 10 if self.packed_cov else 16
@@ -626,6 +637,8 @@ class BatchedUKF:
             res.gate_iters = torch.zeros(b.max_obs, T, dtype=torch.uint8, device=dev)
             res.gate_lambda = torch.ones(b.max_obs, T, **f64)
             res.gate_scale = torch.ones(b.max_obs, T, **f64)
+        if innovations:
+            allocate_innovations(res, b.max_obs, T, dev)
         return res
 
     def _outputs(self, r: TrackResults) -> nat.SteOutputs:
@@ -670,6 +683,7 @@ class BatchedUKF:
             if t is None or tuple(t.shape) != shape or t.device != dev or not t.is_contiguous():
                 got = "None" if t is None else f"{tuple(t.shape)} on {t.device}"
                 raise ValueError(f"TrackResults.{name}: expected a contiguous tensor of shape {shape} on {dev} for this tile, got {got}")
+        check_innovations(res, "TrackResults", b.max_obs, T, dev)
         if self.model.gating and res.gate_iters is None:
             raise ValueError("results were allocated without gating buffers (allocate() with a gating model)")
 
@@ -682,7 +696,11 @@ class BatchedUKF:
         p, i, o = self._problem(b), self._inputs(b), self._outputs(res)
         res.filtered_by = id(b)
         with torch.cuda.device(b.device):
-            nat.check(self._lib.ste_ukf_forward_f64(C.byref(p), C.byref(i), C.byref(o), nat.current_stream()))
+            if res.nis is None:
+                nat.check(self._lib.ste_ukf_forward_f64(C.byref(p), C.byref(i), C.byref(o), nat.current_stream()))
+            else:
+                nat.check(self._lib.ste_ukf_forward_innov_f64(C.byref(p), C.byref(i), C.byref(innovation_planes(res)), C.byref(o),
+                                                              nat.current_stream()))
 
     def backward(self, b: TrackBatch, res: TrackResults) -> None:
         """Launch the URTSS backward pass over the filtered states in ``res``."""
@@ -705,7 +723,10 @@ class BatchedUKF:
         (filtered by an earlier ``forward``/``fused`` call into ``bwd_res``), as blocks of two roles
         resident on every SM together.  Bit-identical to ``forward(fwd_batch, fwd_res);
         backward(bwd_batch, bwd_res)``, and on B200 ~13 % slower than those two launches (two
-        instruction streams per SM overflow the instruction cache).  The two result sets must be distinct."""
+        instruction streams per SM overflow the instruction cache).  The two result sets must be distinct.
+        The fused launch writes no innovation statistics: ``fwd_res`` with innovation planes raises ``ValueError``."""
+        if fwd_res.nis is not None:
+            raise ValueError("the fused pass writes no innovation statistics: filter tiles with innovation planes with forward()")
         self._check_rows(fwd_batch)
         self._check_shapes(fwd_batch, fwd_res)
         self._check_shapes(bwd_batch, bwd_res, smoother=True)
@@ -879,12 +900,52 @@ class BatchedUKF:
         return run_host_pipelined(self, host_batches, host_outs, self._output_names(outputs, smoother), smoother, device,
                                   layout=self.packed_cov)
 
-    def run(self, b: TrackBatch, smoother: bool = True, res: Optional[TrackResults] = None, in_place: bool = False) -> TrackResults:
-        res = res if res is not None else self.allocate(b, smoother=smoother, in_place=in_place)
+    def run(self, b: TrackBatch, smoother: bool = True, res: Optional[TrackResults] = None, in_place: bool = False,
+            innovations: bool = False) -> TrackResults:
+        """Filter (and smooth) a tile into ``res`` or new buffers; ``innovations=True`` allocates the innovation
+        statistics planes with them (``allocate``)."""
+        res = res if res is not None else self.allocate(b, smoother=smoother, in_place=in_place, innovations=innovations)
         self.forward(b, res)
         if smoother:
             self.backward(b, res)
         return res
+
+
+# ---------------------------------------------------------------------- #
+# innovation statistics planes, shared by TrackResults and TrackResultsN  #
+# ---------------------------------------------------------------------- #
+def allocate_innovations(res, max_obs: int, T: int, dev) -> None:
+    """Give ``res`` the ``nis`` / ``loglik`` (float64, NaN until written) and ``innov_rank`` (uint8) planes ``[max_obs][T]``."""
+    res.nis = torch.full((max_obs, T), float("nan"), dtype=torch.float64, device=dev)
+    res.loglik = torch.full((max_obs, T), float("nan"), dtype=torch.float64, device=dev)
+    res.innov_rank = torch.zeros(max_obs, T, dtype=torch.uint8, device=dev)
+
+
+def check_innovations(res, what: str, max_obs: int, T: int, dev) -> None:
+    """All three innovation planes or none, each a contiguous ``[max_obs][T]`` tensor of its dtype on ``dev``."""
+    planes = (("nis", torch.float64), ("loglik", torch.float64), ("innov_rank", torch.uint8))
+    present = [getattr(res, n) is not None for n, _ in planes]
+    if any(present) and not all(present):
+        raise ValueError(f"{what}: nis, loglik and innov_rank are allocated together (allocate(..., innovations=True))")
+    if not any(present):
+        return
+    for name, dtype in planes:
+        t = getattr(res, name)
+        if tuple(t.shape) != (max_obs, T) or t.dtype != dtype or t.device != dev or not t.is_contiguous():
+            raise ValueError(f"{what}.{name}: expected a contiguous {dtype} tensor of shape {(max_obs, T)} on {dev} for this tile, "
+                             f"got {t.dtype} {tuple(t.shape)} on {t.device}")
+
+
+def innovation_planes(res) -> nat.SteInnovations:
+    return nat.SteInnovations(nat.ptr(res.nis), nat.ptr(res.loglik), nat.ptr(res.innov_rank))
+
+
+def innovation_columns(res, out: Dict[str, np.ndarray], j: int) -> None:
+    """The innovation statistics of column ``j``'s ``out["n_updates"]`` updates into ``out``."""
+    m = out["n_updates"]
+    out["nis"] = res.nis[:m, j].cpu().numpy()
+    out["loglik"] = res.loglik[:m, j].cpu().numpy()
+    out["innov_rank"] = res.innov_rank[:m, j].cpu().numpy().astype(np.int32)
 
 
 # ---------------------------------------------------------------------- #

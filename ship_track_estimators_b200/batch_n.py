@@ -22,7 +22,8 @@ import numpy as np
 import torch
 
 from . import _native as nat
-from .batch import (BatchedUKF, TrackBatch, TrackResults, copy_out, length_order, output_names, run_host_pipelined,
+from .batch import (BatchedUKF, TrackBatch, TrackResults, allocate_innovations, check_innovations, copy_out, innovation_columns,
+                    innovation_planes, length_order, output_names, run_host_pipelined,
                     track_rate_repeat, track_rates, track_update_mask)
 
 NS = 5   # state dimension of geodetic_dynamics_turn
@@ -311,8 +312,12 @@ class TrackResultsN:
     order: Optional[np.ndarray] = None
     filtered_by: Optional[int] = field(default=None, repr=False, compare=False)   # id() of the tile last filtered here
     _column_of: Optional[np.ndarray] = field(default=None, repr=False, compare=False)
+    # innovation statistics per update (allocate(..., innovations=True)), [max_obs][T], as TrackResults'
+    nis: Optional[torch.Tensor] = None
+    loglik: Optional[torch.Tensor] = None
+    innov_rank: Optional[torch.Tensor] = None
 
-    _TENSORS = ("mean_f", "cov_f", "mean_s", "cov_s", "status", "n_updates")
+    _TENSORS = ("mean_f", "cov_f", "mean_s", "cov_s", "status", "n_updates", "nis", "loglik", "innov_rank")
 
     def host_like(self, pinned: bool = True) -> "TrackResultsN":
         """Empty host buffers of the same shapes (page-locked by default) for device->host copies."""
@@ -373,6 +378,8 @@ class TrackResultsN:
         if self.mean_s is not None:
             out["means_s"] = self.mean_s[: n + 1, :, j].cpu().numpy()
             out["covs_s"] = self.cov_s[: n + 1, :, j].cpu().numpy().reshape(n + 1, NS, NS)
+        if self.nis is not None:
+            innovation_columns(self, out, j)
         return out
 
 
@@ -450,15 +457,19 @@ class BatchedUKFN:
         o.status, o.n_updates = nat.ptr(r.status), nat.ptr(r.n_updates)
         return o
 
-    def allocate(self, b: TrackBatchN, smoother: bool = True) -> TrackResultsN:
-        """Output buffers for a tile (reusable across tiles of the same shape)."""
+    def allocate(self, b: TrackBatchN, smoother: bool = True, innovations: bool = False) -> TrackResultsN:
+        """Output buffers for a tile (reusable across tiles of the same shape).  ``innovations``: also the ``nis`` /
+        ``loglik`` / ``innov_rank`` planes ``[max_obs][T]`` that the forward pass then fills per update."""
         dev, T, S = b.device, b.n_tracks, b.max_steps + 1
         f64 = dict(dtype=torch.float64, device=dev)
-        return TrackResultsN(
+        res = TrackResultsN(
             mean_f=torch.empty(S, NS, T, **f64), cov_f=torch.empty(S, NS * NS, T, **f64),
             mean_s=torch.empty(S, NS, T, **f64) if smoother else None, cov_s=torch.empty(S, NS * NS, T, **f64) if smoother else None,
             status=torch.zeros(T, dtype=torch.int32, device=dev), n_updates=torch.zeros(T, dtype=torch.int32, device=dev),
             n_steps_host=b.n_steps_host, order=b.order)
+        if innovations:
+            allocate_innovations(res, b.max_obs, T, dev)
+        return res
 
     def _check_shapes(self, b: TrackBatchN, res: TrackResultsN, smoother: bool = False) -> None:
         b.check()
@@ -473,6 +484,7 @@ class BatchedUKFN:
             if t is None or tuple(t.shape) != shape or t.device != dev or not t.is_contiguous():
                 got = "None" if t is None else f"{tuple(t.shape)} on {t.device}"
                 raise ValueError(f"TrackResultsN.{name}: expected a contiguous tensor of shape {shape} on {dev} for this tile, got {got}")
+        check_innovations(res, "TrackResultsN", b.max_obs, T, dev)
 
     def forward(self, b: TrackBatchN, res: TrackResultsN) -> None:
         """Launch the forward filter (asynchronous on the current stream)."""
@@ -480,8 +492,12 @@ class BatchedUKFN:
         p, i, o = self._problem(b), self._inputs(b), self._outputs(res)
         res.filtered_by = id(b)
         with torch.cuda.device(b.device):
-            nat.check(self._lib.ste_ukf_forward_noise_n_f64(C.byref(p), C.byref(i), C.byref(self._noise(b)), C.byref(o),
-                                                            nat.current_stream()))
+            if res.nis is None:
+                nat.check(self._lib.ste_ukf_forward_noise_n_f64(C.byref(p), C.byref(i), C.byref(self._noise(b)), C.byref(o),
+                                                                nat.current_stream()))
+            else:
+                nat.check(self._lib.ste_ukf_forward_innov_n_f64(C.byref(p), C.byref(i), C.byref(self._noise(b)),
+                                                                C.byref(innovation_planes(res)), C.byref(o), nat.current_stream()))
 
     def backward(self, b: TrackBatchN, res: TrackResultsN) -> None:
         """Launch the URTSS backward pass over the filtered states in ``res`` (written by ``forward(b, res)``)."""
@@ -495,8 +511,10 @@ class BatchedUKFN:
             nat.check(self._lib.ste_urtss_backward_tracks_noise_n_f64(C.byref(p), C.byref(i), C.byref(self._noise(b)), C.byref(o),
                                                                       nat.current_stream()))
 
-    def run(self, b: TrackBatchN, smoother: bool = True, res: Optional[TrackResultsN] = None) -> TrackResultsN:
-        res = res if res is not None else self.allocate(b, smoother=smoother)
+    def run(self, b: TrackBatchN, smoother: bool = True, res: Optional[TrackResultsN] = None, innovations: bool = False) -> TrackResultsN:
+        """Filter (and smooth) a tile into ``res`` or new buffers; ``innovations=True`` allocates the innovation
+        statistics planes with them (``allocate``)."""
+        res = res if res is not None else self.allocate(b, smoother=smoother, innovations=innovations)
         self.forward(b, res)
         if smoother:
             self.backward(b, res)

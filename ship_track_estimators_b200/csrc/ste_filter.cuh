@@ -410,16 +410,16 @@ STE_DEV double quad_form(const double (&A)[10], const double (&y)[4]) {
 }
 
 // update (:209-265), generic H / R.  z is consumed (noise added in place as the reference does).
-template <bool GATING>
+template <bool GATING, bool INNOV = false>
 STE_DEV void ukf_update_generic(double (&x)[4], double (&P)[10], const Model &m,
                                                    double (&z)[4], const double *unit_noise /*[4] or null*/,
                                                    double chi, int max_iter, int &status, int &gate_it,
-                                                   double &gate_lam, double &rs) {
+                                                   double &gate_lam, double &rs, Innov *iv = nullptr) {
     const double *H = m.H, *R = m.R;
-    double HP[16], S[10], Sinv[10];
+    double HP[16], S[10], Sinv[10], lpd;
     rs = 1.0;
     innovation_cov(P, H, R, rs, HP, S);
-    pinv_sym4(S, Sinv);
+    int dropped = pinv_sym4<INNOV>(S, Sinv, &lpd);
     gate_it = 0;
     gate_lam = 1.0;
     if (GATING) {
@@ -453,7 +453,7 @@ STE_DEV void ukf_update_generic(double (&x)[4], double (&P)[10], const Model &m,
             gate_lam = gate_lam + (gamma - chi) / den;
             rs *= gate_lam;
             innovation_cov(P, H, R, rs, HP, S);
-            pinv_sym4(S, Sinv);
+            dropped = pinv_sym4<INNOV>(S, Sinv, &lpd);
             gamma = fabs(quad_form(Sinv, yg));
             ++gate_it;
         }
@@ -482,6 +482,7 @@ STE_DEV void ukf_update_generic(double (&x)[4], double (&P)[10], const Model &m,
         y[i] = acc;
     }
     y[3] = wrap180(y[3]);  // :250
+    if constexpr (INNOV) *iv = Innov{quad_form(Sinv, y), lpd, 4 - dropped};
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
         double acc = x[i];
@@ -529,14 +530,16 @@ STE_DEV void ukf_update_generic(double (&x)[4], double (&P)[10], const Model &m,
 // 2x2 block (every example and the CLI input.json of the reference).  S = H P H^T + R is then
 // block-diagonal with an exactly-zero trailing block, pinv(S) = [pinv(S22) 0; 0 0], and K has two
 // non-zero columns; the arithmetic below is the generic path with the zeros removed.
-template <bool GATING>
+// INNOV: the statistics of rows 0 and 1, the only ones S^+ does not zero.
+template <bool GATING, bool INNOV = false>
 STE_DEV void ukf_update_position(double (&x)[4], double (&P)[10], const Model &m,
                                                     double (&z)[4], const double *unit_noise, double chi,
                                                     int max_iter, int &status, int &gate_it,
-                                                    double &gate_lam, double &rs) {
+                                                    double &gate_lam, double &rs, Innov *iv = nullptr) {
     const double r00 = m.R[0], r01 = m.R[1], r11 = m.R[5];
     rs = 1.0;
-    double Si[3];
+    double Si[3], lpd;
+    int dropped;
     gate_it = 0;
     gate_lam = 1.0;
     if (GATING) {
@@ -545,7 +548,7 @@ STE_DEV void ukf_update_position(double (&x)[4], double (&P)[10], const Model &m
         const double y0 = z[0] - x[0], y1 = z[1] - x[1];
 #pragma unroll 1
         for (;;) {
-            pinv_sym2(fma(rs, r00, P[SYM(0, 0)]), fma(rs, r01, P[SYM(0, 1)]), fma(rs, r11, P[SYM(1, 1)]), Si);
+            dropped = pinv_sym2<INNOV>(fma(rs, r00, P[SYM(0, 0)]), fma(rs, r01, P[SYM(0, 1)]), fma(rs, r11, P[SYM(1, 1)]), Si, &lpd);
             const double v0 = fma(Si[0], y0, Si[1] * y1), v1 = fma(Si[1], y0, Si[2] * y1);
             const double gamma = fabs(fma(y0, v0, y1 * v1));
             if (!(gamma > chi)) break;
@@ -559,7 +562,7 @@ STE_DEV void ukf_update_position(double (&x)[4], double (&P)[10], const Model &m
             ++gate_it;
         }
     } else {
-        pinv_sym2(fma(rs, r00, P[SYM(0, 0)]), fma(rs, r01, P[SYM(0, 1)]), fma(rs, r11, P[SYM(1, 1)]), Si);
+        dropped = pinv_sym2<INNOV>(fma(rs, r00, P[SYM(0, 0)]), fma(rs, r01, P[SYM(0, 1)]), fma(rs, r11, P[SYM(1, 1)]), Si, &lpd);
     }
     if (unit_noise) {
         z[0] = fma(unit_noise[0], sqrt(rs * r00), z[0]);
@@ -572,6 +575,7 @@ STE_DEV void ukf_update_position(double (&x)[4], double (&P)[10], const Model &m
         K1[r] = fma(P[SYM(r, 0)], Si[1], P[SYM(r, 1)] * Si[2]);
     }
     const double y0 = z[0] - x[0], y1 = z[1] - x[1];
+    if constexpr (INNOV) *iv = Innov{fma(y0, fma(Si[0], y0, Si[1] * y1), y1 * fma(Si[1], y0, Si[2] * y1)), lpd, 2 - dropped};
 #pragma unroll
     for (int r = 0; r < 4; ++r) x[r] = fma(K0[r], y0, fma(K1[r], y1, x[r]));
     x[3] = py_mod360(x[3]);

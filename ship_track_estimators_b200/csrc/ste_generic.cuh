@@ -79,8 +79,9 @@ STE_DEV void eig_sym_n(int n, double *A, double *V) {
 
 // F = V f(diag) V^T of the symmetric part of A.  inverse: Moore-Penrose with numpy's rcond 1e-15;
 // otherwise Re sqrtm (negative eigenvalues contribute 0; returns true when one was clamped).
-template <int NC>
-STE_DEV bool fun_sym_n(int n, const double *Ain, bool inverse, double *F) {
+// INNOV (inverse only): also the log pseudo-determinant and the rank of the kept spectrum (struct Innov).
+template <int NC, bool INNOV = false>
+STE_DEV bool fun_sym_n(int n, const double *Ain, bool inverse, double *F, Innov *iv = nullptr) {
     constexpr int D = DimN<NC>::LD;
     double A[D * D], V[D * D], f[D];
     for (int i = 0; i < n; ++i)
@@ -89,10 +90,20 @@ STE_DEV bool fun_sym_n(int n, const double *Ain, bool inverse, double *F) {
     double wmax = 0.0;
     for (int k = 0; k < n; ++k) wmax = fmax(wmax, fabs(A[k * D + k]));
     bool flagged = false;
+    if constexpr (INNOV) {
+        iv->log_pdet = 0.0;
+        iv->rank = 0;
+    }
     for (int k = 0; k < n; ++k) {
         const double w = A[k * D + k];
         if (inverse) {
             f[k] = fabs(w) > kPinvRcond * wmax ? 1.0 / w : 0.0;
+            if constexpr (INNOV) {
+                if (fabs(w) > kPinvRcond * wmax) {
+                    iv->log_pdet += log(w);
+                    ++iv->rank;
+                }
+            }
         } else {
             flagged |= w < -1e-13 * wmax;
             f[k] = sqrt(fmax(w, 0.0));
@@ -163,9 +174,10 @@ STE_DEV int predict_core(const ProblemN &p, const double *Q, double *x, double *
 
 // UnscentedKalmanFilter.update (unscented.py:209-265) on a thread-local state, dense H and R: x [n], P [n][D] in place;
 // R row-major n x n (p.R, or a track's own); zin [n] the observation, noise unit normals noise[r * ns] or NULL, scaled
-// by sqrt(diag R).  Returns STE_STATUS_* bits.
-template <int NC>
-STE_DEV int update_core(const ProblemN &p, const double *R, double *x, double *P, const double *zin, const double *noise, int64_t ns) {
+// by sqrt(diag R).  Returns STE_STATUS_* bits.  INNOV: also the update's innovation statistics into *iv (struct Innov).
+template <int NC, bool INNOV = false>
+STE_DEV int update_core(const ProblemN &p, const double *R, double *x, double *P, const double *zin, const double *noise, int64_t ns,
+                        Innov *iv = nullptr) {
     constexpr int D = DimN<NC>::LD;
     const int n = NC > 0 ? NC : p.n;
     double z[D], y[D], PHt[D * D], S[D * D], Si[D * D], K[D * D], A[D * D], AP[D * D];
@@ -182,7 +194,7 @@ STE_DEV int update_core(const ProblemN &p, const double *R, double *x, double *P
             for (int k = 0; k < n; ++k) acc = fma(p.H[i * n + k], PHt[k * D + j], acc);
             S[i * D + j] = acc;
         }
-    fun_sym_n<NC>(n, S, true, Si);
+    fun_sym_n<NC, INNOV>(n, S, true, Si, iv);
     for (int i = 0; i < n; ++i)
         for (int j = 0; j < n; ++j) {
             double acc = 0.0;
@@ -195,6 +207,15 @@ STE_DEV int update_core(const ProblemN &p, const double *R, double *x, double *P
         y[i] = acc;
     }
     if (n > 3) y[3] = wrap180(y[3]);   // :250 (the reference indexes state 3 unconditionally)
+    if constexpr (INNOV) {
+        double nis = 0.0;
+        for (int i = 0; i < n; ++i) {
+            double row = 0.0;
+            for (int j = 0; j < n; ++j) row = fma(Si[i * D + j], y[j], row);
+            nis = fma(y[i], row, nis);
+        }
+        iv->nis = nis;
+    }
     for (int i = 0; i < n; ++i) {
         double acc = x[i];
         for (int k = 0; k < n; ++k) acc = fma(K[i * D + k], y[k], acc);

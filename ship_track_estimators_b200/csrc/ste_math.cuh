@@ -24,6 +24,7 @@ constexpr double kW0 = 1.0 - 4.0 / 3.0;               // unscented.py:125  (n = 
 constexpr double kWi = (1.0 - kW0) / 8.0;             // unscented.py:132
 constexpr double kSigmaScale = 4.0 / (1.0 - kW0);     // unscented.py:95   (= 3)
 constexpr double kPinvRcond = 1e-15;                  // numpy.linalg.pinv default rcond
+constexpr double kLog2Pi = 1.8378770664093454835606594728112;   // log(2 pi): Gaussian log-likelihood of an innovation
 
 STE_HD constexpr int SYM(int i, int j) {
     return i <= j ? (i * 4 - (i * (i - 1)) / 2 + (j - i)) : (j * 4 - (j * (j - 1)) / 2 + (i - j));
@@ -414,9 +415,20 @@ STE_DEV bool sqrt_psd4(const double (&A)[10], double scale, double (&M)[10], con
     return false;
 }
 
+// Innovation statistics of one update, formed by the INNOV instantiations from what the update already holds: the
+// innovation y = z - H x (after the noise draw and the heading wrap), the S = H P H^T + rs R whose pseudo-inverse it
+// applied, and that pseudo-inverse's factorisation.  nis = y^T S^+ y; log_pdet = sum of log(lambda) over the rank
+// eigenvalues S^+ kept (NaN when one of them is negative).
+struct Innov {
+    double nis, log_pdet;
+    int rank;
+};
+
 // Moore-Penrose inverse of a symmetric 4x4 with numpy's cutoff: singular values (|eigenvalues|)
-// <= rcond * max are treated as zero.  Returns the number of dropped eigenvalues.
-STE_DEV int pinv_sym4(const double (&A)[10], double (&Ainv)[10]) {
+// <= rcond * max are treated as zero.  Returns the number of dropped eigenvalues.  INNOV: also the
+// log pseudo-determinant, the sum of log(w) over the kept eigenvalues (NaN when one is negative).
+template <bool INNOV = false>
+STE_DEV int pinv_sym4(const double (&A)[10], double (&Ainv)[10], double *log_pdet = nullptr) {
     double a[10], V[16], f[4];
 #pragma unroll
     for (int i = 0; i < 10; ++i) a[i] = A[i];
@@ -430,6 +442,12 @@ STE_DEV int pinv_sym4(const double (&A)[10], double (&Ainv)[10]) {
         const bool keep = fabs(w[k]) > cut;
         f[k] = keep ? fast_rcp(w[k]) : 0.0;
         dropped += keep ? 0 : 1;
+    }
+    if constexpr (INNOV) {
+        double lp = 0.0;
+#pragma unroll
+        for (int k = 0; k < 4; ++k) lp += fabs(w[k]) > cut ? log(w[k]) : 0.0;
+        *log_pdet = lp;
     }
     sym_from_eig(V, f, Ainv);
     return dropped;
@@ -495,7 +513,8 @@ STE_DEV int pinv_spd4(const double (&A)[10], double (&Ainv)[10]) {
 // Pseudo-inverse of a symmetric 2x2 [a b; b c] with the same cutoff rule (one Jacobi rotation
 // diagonalises a 2x2 exactly).  `floor_sv` is an extra singular value taking part in the
 // max (0 when the 2x2 is the only non-zero block of the full matrix).
-STE_COLD int pinv_sym2_eig(double a, double b, double c, double *inv) {
+template <bool INNOV>
+STE_DEV int pinv_sym2_eig_impl(double a, double b, double c, double *inv, double *log_pdet) {
     const double d = c - a;
     const double bb = b + b;
     const double h = fast_sqrt(fma(d, d, bb * bb));
@@ -511,7 +530,12 @@ STE_COLD int pinv_sym2_eig(double a, double b, double c, double *inv) {
     inv[0] = fma(cs * f0, cs, sn * f1 * sn);
     inv[1] = fma(-cs * f0, sn, sn * f1 * cs);
     inv[2] = fma(sn * f0, sn, cs * f1 * cs);
+    if constexpr (INNOV) *log_pdet = (k0 ? log(w0) : 0.0) + (k1 ? log(w1) : 0.0);
     return (k0 ? 0 : 1) + (k1 ? 0 : 1);
+}
+STE_COLD int pinv_sym2_eig(double a, double b, double c, double *inv) { return pinv_sym2_eig_impl<false>(a, b, c, inv, nullptr); }
+STE_COLD int pinv_sym2_eig_innov(double a, double b, double c, double *inv, double *log_pdet) {
+    return pinv_sym2_eig_impl<true>(a, b, c, inv, log_pdet);
 }
 
 // Hot path: S22 = P22 + R22 of a running filter is positive definite and well conditioned (R adds
@@ -519,18 +543,23 @@ STE_COLD int pinv_sym2_eig(double a, double b, double c, double *inv) {
 // critical path instead of two dependent square roots.  det = a c - b^2 is formed with an exact
 // product error term; anything that is not clearly positive definite (det <= 1e-8 a c, i.e. the
 // two rows closer than ~1e-4 rad to parallel, or a non-positive diagonal) takes the
-// eigen-decomposition with numpy's cutoff semantics.
-STE_DEV int pinv_sym2(double a, double b, double c, double (&inv)[3]) {
+// eigen-decomposition with numpy's cutoff semantics.  INNOV: also the log pseudo-determinant of the
+// factorisation taken (log det here, the kept eigenvalues' logs on the eigen branch).
+template <bool INNOV = false>
+STE_DEV int pinv_sym2(double a, double b, double c, double (&inv)[3], double *log_pdet = nullptr) {
     const double ac = a * c;
     const double det = fma(-b, b, ac) + fma(a, c, -ac);
     if (!(a > 0.0 && c > 0.0 && det > 1e-8 * ac)) {
         double t[3];
-        const int dropped = pinv_sym2_eig(a, b, c, t);
+        int dropped;
+        if constexpr (INNOV) dropped = pinv_sym2_eig_innov(a, b, c, t, log_pdet);
+        else dropped = pinv_sym2_eig(a, b, c, t);
         inv[0] = t[0];
         inv[1] = t[1];
         inv[2] = t[2];
         return dropped;
     }
+    if constexpr (INNOV) *log_pdet = log(det);
     const double r = fast_rcp(det);
     inv[0] = c * r;
     inv[1] = -b * r;

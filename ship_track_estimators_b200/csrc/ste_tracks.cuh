@@ -87,10 +87,12 @@ STE_DEV bool any_nonfinite(const double (&x)[4], const double (&P)[10]) {
 // Forward filter: KalmanFilterBase.run (kalman_filter.py:36-117).
 //
 // The time loop is written as begin() / step(s) / end() on a small state object.
+// INNOV: every update also stores its innovation statistics (struct Innov) into row u of the planes of `iv`.
 // ------------------------------------------------------------------------------------------ //
-template <bool POS_ONLY, bool GATING>
+template <bool POS_ONLY, bool GATING, bool INNOV = false>
 struct ForwardTrack {
     const KernelArgs &a;
+    const SteInnovations *iv;
     const int t;
     const Scratch sc;
     const int64_t ld;
@@ -106,8 +108,8 @@ struct ForwardTrack {
     int sub_left = 1;   // predicts left until the next update when the cadence is "every k-th step"
     bool consistent = true, upd_next = false;
 
-    STE_DEV ForwardTrack(const KernelArgs &args, int track, const Scratch &scratch)
-        : a(args), t(track), sc(scratch), ld(args.prob.ld), packed((args.prob.flags & STE_FLAG_PACKED_COV) != 0) {}
+    STE_DEV ForwardTrack(const KernelArgs &args, int track, const Scratch &scratch, const SteInnovations *innov = nullptr)
+        : a(args), iv(innov), t(track), sc(scratch), ld(args.prob.ld), packed((args.prob.flags & STE_FLAG_PACKED_COV) != 0) {}
 
     // observation rows are staged into scratch a whole predict ahead of their use
     // row u of a [row][track] input array for this track: base + t, then one 32 x 32 + 64-bit multiply-add (plane_ptr)
@@ -159,14 +161,21 @@ struct ForwardTrack {
         }
         int it;
         double lam, rs;
+        Innov st;
         if (POS_ONLY)
-            ukf_update_position<GATING>(x, P, model, z, noise, a.prob.gate_chi, a.prob.gate_max_iter, status, it, lam, rs);
+            ukf_update_position<GATING, INNOV>(x, P, model, z, noise, a.prob.gate_chi, a.prob.gate_max_iter, status, it, lam, rs, &st);
         else
-            ukf_update_generic<GATING>(x, P, model, z, noise, a.prob.gate_chi, a.prob.gate_max_iter, status, it, lam, rs);
+            ukf_update_generic<GATING, INNOV>(x, P, model, z, noise, a.prob.gate_chi, a.prob.gate_max_iter, status, it, lam, rs, &st);
         if (GATING) {
             if (a.out.gate_iters) a.out.gate_iters[(int64_t)u * ld + t] = (uint8_t)min_(it, 255);
             if (a.out.gate_lambda) a.out.gate_lambda[(int64_t)u * ld + t] = lam;
             if (a.out.gate_scale) a.out.gate_scale[(int64_t)u * ld + t] = rs;
+        }
+        if constexpr (INNOV) {
+            const int64_t row = (int64_t)u * ld + t;
+            iv->nis[row] = st.nis;
+            iv->loglik[row] = -0.5 * fma((double)st.rank, kLog2Pi, st.nis + st.log_pdet);
+            iv->rank[row] = (uint8_t)st.rank;
         }
     }
 
@@ -234,9 +243,9 @@ struct ForwardTrack {
     }
 };
 
-template <bool POS_ONLY, bool GATING>
-STE_DEV void forward_track(const KernelArgs &a, const int t, const Scratch &sc) {
-    ForwardTrack<POS_ONLY, GATING> f(a, t, sc);
+template <bool POS_ONLY, bool GATING, bool INNOV = false>
+STE_DEV void forward_track(const KernelArgs &a, const int t, const Scratch &sc, const SteInnovations *iv = nullptr) {
+    ForwardTrack<POS_ONLY, GATING, INNOV> f(a, t, sc, iv);
     f.begin();
 #if defined(STE_STEP_SYNC) && defined(__CUDA_ARCH__)
     // experiment: the warps of a block start every step together (instruction-cache locality); ragged lengths are safe,

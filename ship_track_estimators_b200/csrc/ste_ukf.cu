@@ -35,11 +35,23 @@ constexpr int kThreads = STE_THREADS;
 #define STE_BWD_RECOMPUTE_MIN_BLOCKS 3   // 62 scratch slots per thread: three 62 KB blocks per SM
 #endif
 
-template <bool POS_ONLY, bool GATING>
-__global__ void __launch_bounds__(kThreads, STE_FWD_MIN_BLOCKS) ukf_forward_kernel(const __grid_constant__ KernelArgs a) {
+// INNOV: the launch also writes the innovation statistics of every update.  Their planes travel in a parameter block of
+// their own (KernelArgsInnov), so that KernelArgs - and with it every other kernel's parameters - stays as it was.
+struct KernelArgsInnov : KernelArgs {
+    SteInnovations innov;
+};
+template <bool INNOV> struct ForwardArgs { using type = KernelArgs; };
+template <> struct ForwardArgs<true> { using type = KernelArgsInnov; };
+
+template <bool POS_ONLY, bool GATING, bool INNOV = false>
+__global__ void __launch_bounds__(kThreads, STE_FWD_MIN_BLOCKS) ukf_forward_kernel(const __grid_constant__ typename ForwardArgs<INNOV>::type a) {
     extern __shared__ double scratch[];   // kScratchSlotsFwd * kThreads doubles (62 KB: opt-in size)
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t < a.prob.n_tracks) forward_track<POS_ONLY, GATING>(a, t, Scratch{scratch + threadIdx.x, kThreads});
+    if constexpr (INNOV) {
+        if (t < a.prob.n_tracks) forward_track<POS_ONLY, GATING, true>(a, t, Scratch{scratch + threadIdx.x, kThreads}, &a.innov);
+    } else {
+        if (t < a.prob.n_tracks) forward_track<POS_ONLY, GATING>(a, t, Scratch{scratch + threadIdx.x, kThreads});
+    }
 }
 
 // TAPE: the launch has a statistics tape (same code either way; only the register budget differs)
@@ -520,6 +532,7 @@ struct FleetArgsN {
     SteInputsN in;
     SteOutputsN out;
     SteNoiseN noise;   // per-track Q / R planes, or NULL (last, so the shared path's parameter offsets stay as they were)
+    SteInnovations innov;   // innovation statistics planes (read by the Innov instantiation only)
 };
 
 // Q and R of track t: with PerTrack, its own planes (noise.Q_tracks / R_tracks, the launch's matrix where one is NULL)
@@ -537,7 +550,8 @@ STE_DEV const double *track_matrix(const double *shared, const double *planes, i
 
 // KalmanFilterBase.run (kalman_filter.py:36-117): row 0 the prior, the initial update with observation 0, then per step
 // a predict with the rates of the current update index and, where upd_mask is set, an update with the next observation.
-template <int NC, bool PerTrack>
+// Innov: every update also stores its innovation statistics into row u of a.innov's planes.
+template <int NC, bool PerTrack, bool Innov = false>
 __global__ void __launch_bounds__(kThreadsN) ukf_forward_n_kernel(const __grid_constant__ FleetArgsN a) {
     constexpr int D = DimN<NC>::LD, n = NC;
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
@@ -559,7 +573,17 @@ __global__ void __launch_bounds__(kThreadsN) ukf_forward_n_kernel(const __grid_c
     };
     auto update = [&](int u) {   // observation row u; rows the caller left NULL read as 0
         for (int r = 0; r < n; ++r) z[r] = in.z[r] ? in.z[r][(int64_t)u * ld + t] : 0.0;
-        return update_core<NC>(a.p, R, x, P, z, in.noise_upd ? in.noise_upd + (int64_t)u * n * ld + t : nullptr, ld);
+        if constexpr (Innov) {
+            ste::Innov st;
+            const int bits = update_core<NC, true>(a.p, R, x, P, z, in.noise_upd ? in.noise_upd + (int64_t)u * n * ld + t : nullptr, ld, &st);
+            const int64_t row = (int64_t)u * ld + t;
+            a.innov.nis[row] = st.nis;
+            a.innov.loglik[row] = -0.5 * fma((double)st.rank, kLog2Pi, st.nis + st.log_pdet);
+            a.innov.rank[row] = (uint8_t)st.rank;
+            return bits;
+        } else {
+            return update_core<NC>(a.p, R, x, P, z, in.noise_upd ? in.noise_upd + (int64_t)u * n * ld + t : nullptr, ld);
+        }
     };
     store(0);                      // :76-81
     int status = update(0), ui = 0;
@@ -776,26 +800,46 @@ static KernelArgs kernel_args(const SteProblem *prob, const SteInputs *in, const
     return a;
 }
 
+static int validate_innovations(const SteInnovations *innov) {
+    if (innov && (!innov->nis || !innov->loglik || !innov->rank))
+        return fail(STE_ERR_INVALID_ARG, "SteInnovations needs all three planes (nis, loglik, rank)");
+    return STE_OK;
+}
+
 extern "C++" {
-template <bool POS_ONLY, bool GATING>
-static int launch_forward(const KernelArgs &a, cudaStream_t s) {
+template <bool POS_ONLY, bool GATING, bool INNOV>
+static int launch_forward(const typename ForwardArgs<INNOV>::type &a, cudaStream_t s) {
     const dim3 grid((a.prob.n_tracks + kThreads - 1) / kThreads), block(kThreads);
     const size_t smem = sizeof(double) * kScratchSlotsFwd * kThreads;
-    if (cudaFuncSetAttribute(ukf_forward_kernel<POS_ONLY, GATING>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+    if (cudaFuncSetAttribute(ukf_forward_kernel<POS_ONLY, GATING, INNOV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
         return check_launch("cudaFuncSetAttribute(ukf_forward_kernel)");
-    ukf_forward_kernel<POS_ONLY, GATING><<<grid, block, smem, s>>>(a);
+    ukf_forward_kernel<POS_ONLY, GATING, INNOV><<<grid, block, smem, s>>>(a);
     return check_launch("ukf_forward_kernel");
+}
+
+template <bool INNOV>
+static int launch_forward(bool pos, bool gating, const typename ForwardArgs<INNOV>::type &a, cudaStream_t s) {
+    if (pos) return gating ? launch_forward<true, true, INNOV>(a, s) : launch_forward<true, false, INNOV>(a, s);
+    return gating ? launch_forward<false, true, INNOV>(a, s) : launch_forward<false, false, INNOV>(a, s);
 }
 }  // extern "C++"
 
 int ste_ukf_forward_f64(const SteProblem *prob, const SteInputs *in, SteOutputs *out, void *stream) {
+    return ste_ukf_forward_innov_f64(prob, in, nullptr, out, stream);
+}
+
+int ste_ukf_forward_innov_f64(const SteProblem *prob, const SteInputs *in, const SteInnovations *innov, SteOutputs *out,
+                              void *stream) {
     if (int rc = validate_forward(prob, in, out)) return rc;
+    if (int rc = validate_innovations(innov)) return rc;
     if (prob->n_tracks == 0) return STE_OK;
     const bool gating = (prob->flags & STE_FLAG_GATING) != 0, pos = position_only(*prob);
-    const KernelArgs a = kernel_args(prob, in, out);
     cudaStream_t s = (cudaStream_t)stream;
-    if (pos) return gating ? launch_forward<true, true>(a, s) : launch_forward<true, false>(a, s);
-    return gating ? launch_forward<false, true>(a, s) : launch_forward<false, false>(a, s);
+    if (!innov) return launch_forward<false>(pos, gating, kernel_args(prob, in, out), s);
+    KernelArgsInnov a;
+    static_cast<KernelArgs &>(a) = kernel_args(prob, in, out);
+    a.innov = *innov;
+    return launch_forward<true>(pos, gating, a, s);
 }
 
 int ste_urtss_backward_f64(const SteProblem *prob, const SteInputs *in, SteOutputs *out, void *stream) {
@@ -989,14 +1033,27 @@ int ste_ukf_forward_n_f64(const SteProblemN *prob, const SteInputsN *in, SteOutp
 
 int ste_ukf_forward_noise_n_f64(const SteProblemN *prob, const SteInputsN *in, const SteNoiseN *noise, SteOutputsN *out,
                                 void *stream) {
+    return ste_ukf_forward_innov_n_f64(prob, in, noise, nullptr, out, stream);
+}
+
+int ste_ukf_forward_innov_n_f64(const SteProblemN *prob, const SteInputsN *in, const SteNoiseN *noise,
+                                const SteInnovations *innov, SteOutputsN *out, void *stream) {
     if (int rc = validate_fleet_n(prob, in, out, false)) return rc;
+    if (int rc = validate_innovations(innov)) return rc;
     if (prob->n_tracks == 0) return STE_OK;
-    const FleetArgsN a = fleet_args(prob, in, out, noise);
+    FleetArgsN a = fleet_args(prob, in, out, noise);
     const int blocks = (prob->n_tracks + kThreadsN - 1) / kThreadsN;
-    if (a.noise.Q_tracks || a.noise.R_tracks)
-        ukf_forward_n_kernel<5, true><<<blocks, kThreadsN, 0, (cudaStream_t)stream>>>(a);
-    else
-        ukf_forward_n_kernel<5, false><<<blocks, kThreadsN, 0, (cudaStream_t)stream>>>(a);
+    cudaStream_t s = (cudaStream_t)stream;
+    const bool per_track = a.noise.Q_tracks || a.noise.R_tracks;
+    if (innov) {
+        a.innov = *innov;
+        if (per_track) ukf_forward_n_kernel<5, true, true><<<blocks, kThreadsN, 0, s>>>(a);
+        else ukf_forward_n_kernel<5, false, true><<<blocks, kThreadsN, 0, s>>>(a);
+    } else if (per_track) {
+        ukf_forward_n_kernel<5, true><<<blocks, kThreadsN, 0, s>>>(a);
+    } else {
+        ukf_forward_n_kernel<5, false><<<blocks, kThreadsN, 0, s>>>(a);
+    }
     return check_launch("ukf_forward_n_kernel");
 }
 

@@ -5,7 +5,8 @@
 arrays, or torch tensors on any device - the arithmetic then runs where the tensors live).
 ``track_metrics`` is what a 16 M-track run needs instead of copying every state to the host: one
 kernel launch (``ste_track_metrics_f64``, ``ste_track_metrics_n_f64`` at n = 5) that reduces, per track, the residuals between a state
-estimate and the observations it assimilated.
+estimate and the observations it assimilated.  ``innovation_metrics`` sums the per-update innovation
+statistics the forward pass can write (``allocate(..., innovations=True)``) into per-track scores.
 """
 from __future__ import annotations
 
@@ -17,7 +18,7 @@ import torch
 
 from . import _native as nat
 
-__all__ = ["rmse", "cum_abs_diff", "abs_diff", "track_metrics"]
+__all__ = ["rmse", "cum_abs_diff", "abs_diff", "track_metrics", "innovation_metrics"]
 
 
 def _is_tensor(*xs) -> bool:
@@ -77,3 +78,29 @@ def track_metrics(ukf, batch, res, which: str = "smoothed", keep_abs_diff: bool 
     if ad is not None:
         out["abs_diff"] = ad[:, :, :T]
     return out
+
+
+def innovation_metrics(res) -> Dict[str, torch.Tensor]:
+    """Per-track sums of the forward pass's innovation statistics, for choosing noise and testing consistency.
+
+    ``res`` is a ``TrackResults`` or ``TrackResultsN`` filtered with innovation planes (``allocate(...,
+    innovations=True)`` / ``run(..., innovations=True)``).  Returns tensors ``[T]`` on ``res``'s device, in the tile's
+    column order (as ``track_metrics``): ``loglik`` the Gaussian log-likelihood of the track's observations, each under
+    its one-step prediction (the sum over its updates), ``nis`` the summed normalised innovation squared ``y^T S^+ y``,
+    ``dof`` the summed rank of ``S`` and ``n_updates``.  Rows at or beyond a track's ``n_updates`` do not count.
+
+    ``track_metrics`` cannot choose ``R``: it compares the *updated* state with the fix just assimilated, and that
+    residual shrinks as ``R`` goes to zero because the filter snaps to its fixes.  The likelihood scores each fix before
+    it is assimilated, against the spread ``S = H P H^T + R`` the filter predicted for it, so an ``R`` (or ``Q``) too small
+    is penalised by large innovations and one too large by a large ``log det S``.  Packing the same ships once per
+    candidate ``(Q, R)`` (per-track planes) scores every candidate in one launch: the largest summed ``loglik`` is the
+    maximum-likelihood choice.  For a consistent filter ``nis`` follows a chi-squared law with ``dof`` degrees of freedom.
+    """
+    if res.nis is None or res.loglik is None or res.innov_rank is None:
+        raise ValueError("results hold no innovation statistics: allocate(..., innovations=True) before the forward pass")
+    n_upd = res.n_updates.to(torch.int64)
+    rows = torch.arange(res.nis.shape[0], device=res.nis.device)[:, None]
+    valid = rows < n_upd[None, :]
+    zero = torch.zeros((), dtype=torch.float64, device=res.nis.device)
+    return {"loglik": torch.where(valid, res.loglik, zero).sum(0), "nis": torch.where(valid, res.nis, zero).sum(0),
+            "dof": torch.where(valid, res.innov_rank.to(torch.int64), 0).sum(0), "n_updates": res.n_updates}
