@@ -43,6 +43,8 @@ extern "C" {
                             /*    ste_urtss_backward_tracks_noise_n_f64 (per-track Q / R of the five-state fleet path)                    */
                             /*    additive, no struct changed: SteInnovations, ste_ukf_forward_innov_f64, ste_ukf_forward_innov_n_f64     */
                             /*    (per-update innovation statistics of the forward passes)                                               */
+                            /*    additive, no struct changed: SteCandidates, SteScores, ste_ukf_score_f64, ste_ukf_score_n_f64           */
+                            /*    (log-likelihood scores of many noise candidates per track in one launch)                               */
 #define STE_STATS_PLANES 15
 #define STE_DIM 4
 #define STE_NSIGMA 9
@@ -306,6 +308,45 @@ int ste_ukf_forward_innov_f64(const SteProblem *prob, const SteInputs *in, const
                               SteOutputs *out, void *stream);
 int ste_ukf_forward_innov_n_f64(const SteProblemN *prob, const SteInputsN *in, const SteNoiseN *noise,
                                 const SteInnovations *innov, SteOutputsN *out, void *stream);
+
+/* Scores of many noise candidates, for choosing Q and R by maximum likelihood (a grid search): one store-free forward
+ * pass per (candidate, track) pair.  Candidate c's Q and R replace SteProblem(N).Q / R; everything else - H, P0, gating,
+ * flags, the inputs, the noise tapes (scaled by the candidate's sqrt(diag Q) / sqrt(diag R)) - is the tile's.  Nothing is
+ * stored per step.  For candidate c and track t, summed in update order over the track's updates u (u = 0 the initial
+ * update), with the statistics of SteInnovations:
+ *   loglik[c][t]    = sum_u -1/2 (nis_u + log pdet_u + rank_u log 2 pi)   (the per-update loglik plane, summed from 0.0)
+ *   nis[c][t]       = sum_u nis_u
+ *   dof[c][t]       = sum_u rank_u
+ *   n_updates[c][t] = updates assimilated incl. the initial one
+ *   status[c][t]    = the forward pass's STE_STATUS_* bits
+ * Each value equals what ste_ukf_forward_innov_f64 / ste_ukf_forward_innov_n_f64 run with that candidate's Q and R writes,
+ * summed in that order: bit for bit.  One launch covers every candidate (grid.y = candidate).  The table travels in the
+ * kernel parameters: at most STE_MAX_CANDIDATES per call, nothing allocated.  Returns before any launch:
+ *   STE_ERR_INVALID_ARG  n_cand outside [1, STE_MAX_CANDIDATES], a NULL table, matrix or output plane, ld_out < n_tracks,
+ *                        SteInputs.R_tracks set (a tile that carries its own noise), or what the forward pass refuses;
+ *   STE_ERR_UNSUPPORTED  an asymmetric or non-finite candidate; at n = 4, candidates whose R selects different updates
+ *                        (position-only for some, the generic update for others: split them into separate calls);
+ *                        gating with noise_upd, as the forward pass.
+ * The n = 5 entry point takes no SteNoiseN: a tile with per-track Q / R planes has nothing to score against. */
+#define STE_MAX_CANDIDATES 32
+typedef struct SteCandidates {
+    int32_t n_cand;           /* 1 .. STE_MAX_CANDIDATES                                          */
+    int32_t reserved;         /* must be 0                                                        */
+    const double *Q;          /* HOST [n_cand][n*n] row-major process noise, one matrix per candidate */
+    const double *R;          /* HOST [n_cand][n*n] row-major measurement noise                    */
+} SteCandidates;
+typedef struct SteScores {    /* DEVICE planes, element (c, t) at base[c * ld_out + t]                 */
+    double  *loglik;          /* [n_cand][ld_out] summed Gaussian log-likelihood                      */
+    double  *nis;             /* [n_cand][ld_out] summed y^T S^+ y                                     */
+    int32_t *dof;             /* [n_cand][ld_out] summed rank of S                                     */
+    int32_t *n_updates;       /* [n_cand][ld_out] updates assimilated                                  */
+    int32_t *status;          /* [n_cand][ld_out] STE_STATUS_* of the forward pass                     */
+    int64_t ld_out;           /* >= n_tracks                                                           */
+} SteScores;
+int ste_ukf_score_f64(const SteProblem *prob, const SteInputs *in, const SteCandidates *cand, SteScores *scores,
+                      void *stream);
+int ste_ukf_score_n_f64(const SteProblemN *prob, const SteInputsN *in, const SteCandidates *cand, SteScores *scores,
+                        void *stream);
 
 /* UnscentedKalmanFilter.criterion_index and the denominator of update_lambda_factor
  * (unscented.py:389-483) for T filters: with y = z - x (not z - Hx, no angle wrap) and

@@ -140,6 +140,29 @@ class SteOutputsN(C.Structure):
     ]
 
 
+STE_MAX_CANDIDATES = 32
+
+
+class SteCandidates(C.Structure):
+    _fields_ = [
+        ("n_cand", C.c_int32),
+        ("reserved", C.c_int32),
+        ("Q", C.POINTER(C.c_double)),   # host [n_cand][n*n]
+        ("R", C.POINTER(C.c_double)),
+    ]
+
+
+class SteScores(C.Structure):
+    _fields_ = [
+        ("loglik", _dptr),
+        ("nis", _dptr),
+        ("dof", _dptr),
+        ("n_updates", _dptr),
+        ("status", _dptr),
+        ("ld_out", C.c_int64),
+    ]
+
+
 STE_TEXT_MAX_COLS, STE_TEXT_MAX_TABLES, STE_TEXT_MAX_VALUE_BYTES = 8, 8, 27
 
 
@@ -186,6 +209,9 @@ _PROTOTYPES = {
                                             C.c_void_p]),
     "ste_ukf_forward_innov_n_f64": (C.c_int, [C.POINTER(SteProblemN), C.POINTER(SteInputsN), C.POINTER(SteNoiseN), C.POINTER(SteInnovations),
                                               C.POINTER(SteOutputsN), C.c_void_p]),
+    "ste_ukf_score_f64": (C.c_int, [C.POINTER(SteProblem), C.POINTER(SteInputs), C.POINTER(SteCandidates), C.POINTER(SteScores), C.c_void_p]),
+    "ste_ukf_score_n_f64": (C.c_int, [C.POINTER(SteProblemN), C.POINTER(SteInputsN), C.POINTER(SteCandidates), C.POINTER(SteScores),
+                                      C.c_void_p]),
     "ste_process_f64": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int64] + [_dptr] * 5 + [C.c_void_p]),
     "ste_csv_parse_rows": (C.c_int, [_dptr, _dptr, C.c_int64, C.POINTER(C.c_int32)] + [_dptr] * 9 + [C.c_void_p]),
     "ste_gate_terms_f64": (C.c_int, [C.POINTER(SteProblem)] + [_dptr] * 5 + [C.c_void_p]),

@@ -60,13 +60,17 @@ class FilterModel:
             if not np.array_equal(M, M.T):
                 raise NotImplementedError(f"{name} must be symmetric for the CUDA path")
 
+    def position_only(self) -> bool:
+        """Whether the kernels take the position-only update: H = diag(1,1,0,0) exactly, R zero outside its
+        leading 2x2 block and no ``force_generic``."""
+        return (not self.force_generic) and np.array_equal(self.H, np.diag([1.0, 1.0, 0.0, 0.0])) and not (
+            np.any(self.R[2:, :]) or np.any(self.R[:, 2:])
+        )
+
     def rows_needed(self) -> List[bool]:
         """Observation rows the update can actually read (a row multiplying only exact zeros of
         pinv(H P H^T + R) may be absent)."""
-        pos = (not self.force_generic) and np.array_equal(self.H, np.diag([1.0, 1.0, 0.0, 0.0])) and not (
-            np.any(self.R[2:, :]) or np.any(self.R[:, 2:])
-        )
-        if pos:
+        if self.position_only():
             return [True, True, False, False]
         return [bool(self.gating or np.any(self.H[r]) or np.any(self.R[r])) for r in range(4)]
 
@@ -900,6 +904,42 @@ class BatchedUKF:
         return run_host_pipelined(self, host_batches, host_outs, self._output_names(outputs, smoother), smoother, device,
                                   layout=self.packed_cov)
 
+    def score(self, b: TrackBatch, candidates: Sequence) -> Dict[str, torch.Tensor]:
+        """Log-likelihood scores of noise candidates for every track of ``b``, without storing any state.
+
+        ``candidates`` is a sequence of ``(Q, R)`` pairs, each checked as the constructor checks its own (4 x 4,
+        symmetric) and finite.  Candidate ``c`` is scored as this filter with ``Q, R = candidates[c]`` would run
+        ``run(b, smoother=False, innovations=True)``: its ``loglik`` / ``nis`` / ``dof`` / ``n_updates`` equal
+        ``performance_metrics.innovation_metrics`` of that run, bit for bit, and ``status`` its status.  Returns those
+        five device tensors ``[C][T]`` in the tile's column order (column j is the caller's track ``b.order[j]``).
+
+        Candidates whose ``R`` selects the position-only update and those that need the generic one are launched
+        apart; each launch covers up to ``STE_MAX_CANDIDATES`` candidates (asynchronous on the current stream).  A tile
+        with its own per-track ``R`` raises ``ValueError``: the candidates replace it."""
+        b.check()
+        if b.R is not None:
+            raise ValueError("TrackBatch.R: a tile with per-track measurement noise cannot be scored (the candidates replace R)")
+        if self.model.gating and b.noise_upd is not None:
+            raise NotImplementedError("gating with measurement noise tapes (data-dependent draw count)")
+        m = self.model
+        models = []
+        for c, (Qc, Rc) in enumerate(candidate_pairs(candidates)):
+            mc = FilterModel(H=m.H, Q=Qc, R=Rc, P0=m.P0, gating=m.gating, gate_chi=m.gate_chi, gate_max_iter=m.gate_max_iter,
+                             force_generic=m.force_generic)
+            if not (np.all(np.isfinite(mc.Q)) and np.all(np.isfinite(mc.R))):
+                raise ValueError(f"candidate {c}: Q and R must be finite")
+            for r, need in enumerate(mc.rows_needed()):
+                if need and b.z[r] is None:
+                    raise ValueError(f"candidate {c}: observation row {r} is referenced by H/R but absent from the batch")
+            models.append(mc)
+        pos = [mc.position_only() for mc in models]
+        groups = [[c for c in range(len(models)) if pos[c] == v] for v in (True, False)]
+        Q = np.stack([mc.Q.reshape(-1) for mc in models])
+        R = np.stack([mc.R.reshape(-1) for mc in models])
+        p, i = self._problem(b), self._inputs(b)
+        with torch.cuda.device(b.device):
+            return launch_scores(self._lib.ste_ukf_score_f64, p, i, [g for g in groups if g], Q, R, b.device)
+
     def run(self, b: TrackBatch, smoother: bool = True, res: Optional[TrackResults] = None, in_place: bool = False,
             innovations: bool = False) -> TrackResults:
         """Filter (and smooth) a tile into ``res`` or new buffers; ``innovations=True`` allocates the innovation
@@ -946,6 +986,51 @@ def innovation_columns(res, out: Dict[str, np.ndarray], j: int) -> None:
     out["nis"] = res.nis[:m, j].cpu().numpy()
     out["loglik"] = res.loglik[:m, j].cpu().numpy()
     out["innov_rank"] = res.innov_rank[:m, j].cpu().numpy().astype(np.int32)
+
+
+# ---------------------------------------------------------------------- #
+# noise-candidate scores, shared by BatchedUKF.score and BatchedUKFN.score #
+# ---------------------------------------------------------------------- #
+SCORE_KEYS = ("loglik", "nis", "dof", "n_updates", "status")
+
+
+def candidate_pairs(candidates: Sequence) -> List[tuple]:
+    """``candidates`` as a list of ``(Q, R)`` pairs; ``ValueError`` for an empty sequence or an entry that is not a pair."""
+    pairs = list(candidates)
+    if not pairs:
+        raise ValueError("no noise candidates to score")
+    for c, pair in enumerate(pairs):
+        if len(pair) != 2:
+            raise ValueError(f"candidate {c}: expected a (Q, R) pair")
+    return pairs
+
+
+def launch_scores(fn, p, i, groups: Sequence[Sequence[int]], Q: np.ndarray, R: np.ndarray, dev) -> Dict[str, torch.Tensor]:
+    """Score candidates ``Q[c]`` / ``R[c]`` (rows of row-major n x n entries) with the C entry point ``fn``
+    (``ste_ukf_score_f64`` / ``ste_ukf_score_n_f64``) on problem ``p`` and inputs ``i``: one launch per chunk of at
+    most ``STE_MAX_CANDIDATES`` candidates of each group (a list of candidate indices).  Returns the ``SCORE_KEYS`` tensors ``[C][T]``."""
+    n_cand, T = len(Q), int(p.n_tracks)
+    f64, i32 = dict(dtype=torch.float64, device=dev), dict(dtype=torch.int32, device=dev)
+    out = {"loglik": torch.empty(n_cand, T, **f64), "nis": torch.empty(n_cand, T, **f64), "dof": torch.empty(n_cand, T, **i32),
+           "n_updates": torch.empty(n_cand, T, **i32), "status": torch.empty(n_cand, T, **i32)}
+    if T == 0:
+        return out
+    for group in groups:
+        for lo in range(0, len(group), nat.STE_MAX_CANDIDATES):
+            sel = list(group[lo: lo + nat.STE_MAX_CANDIDATES])
+            rows = slice(sel[0], sel[0] + len(sel))
+            direct = sel == list(range(rows.start, rows.stop))   # consecutive candidates are written in place
+            dst = {k: v[rows] if direct else torch.empty(len(sel), T, dtype=v.dtype, device=dev) for k, v in out.items()}
+            Qh, Rh = np.ascontiguousarray(Q[sel], dtype=np.float64), np.ascontiguousarray(R[sel], dtype=np.float64)
+            dp = C.POINTER(C.c_double)
+            cand = nat.SteCandidates(len(sel), 0, Qh.ctypes.data_as(dp), Rh.ctypes.data_as(dp))
+            sc = nat.SteScores(*(nat.ptr(dst[k]) for k in SCORE_KEYS), T)
+            nat.check(fn(C.byref(p), C.byref(i), C.byref(cand), C.byref(sc), nat.current_stream()))
+            if not direct:
+                idx = torch.tensor(sel, dtype=torch.int64, device=dev)
+                for k, v in out.items():
+                    v.index_copy_(0, idx, dst[k])
+    return out
 
 
 # ---------------------------------------------------------------------- #

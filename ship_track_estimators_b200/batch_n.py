@@ -22,8 +22,8 @@ import numpy as np
 import torch
 
 from . import _native as nat
-from .batch import (BatchedUKF, TrackBatch, TrackResults, allocate_innovations, check_innovations, copy_out, innovation_columns,
-                    innovation_planes, length_order, output_names, run_host_pipelined,
+from .batch import (BatchedUKF, TrackBatch, TrackResults, allocate_innovations, candidate_pairs, check_innovations, copy_out,
+                    innovation_columns, innovation_planes, launch_scores, length_order, output_names, run_host_pipelined,
                     track_rate_repeat, track_rates, track_update_mask)
 
 NS = 5   # state dimension of geodetic_dynamics_turn
@@ -519,6 +519,31 @@ class BatchedUKFN:
         if smoother:
             self.backward(b, res)
         return res
+
+    def score(self, b: TrackBatchN, candidates: Sequence) -> Dict[str, torch.Tensor]:
+        """Log-likelihood scores of noise candidates for every track of ``b``, without storing any state: what
+        :meth:`BatchedUKF.score` does for the five-state tile.  ``candidates`` is a sequence of ``(Q, R)`` pairs of
+        symmetric, finite 5 x 5 matrices (``ValueError`` otherwise).  Returns the device tensors ``loglik``, ``nis``,
+        ``dof``, ``n_updates`` and ``status`` ``[C][T]`` in the tile's column order, each equal bit for bit to
+        ``innovation_metrics`` (and the status) of ``run(b, smoother=False, innovations=True)`` on a filter built with
+        that candidate's matrices.  One launch per ``STE_MAX_CANDIDATES`` candidates, on the current stream.  A tile
+        with per-track ``Q`` / ``R`` planes raises ``ValueError``: the candidates replace them."""
+        b.check()
+        if b.Q is not None or b.R is not None:
+            raise ValueError("TrackBatchN.Q / R: a tile with per-track noise cannot be scored (the candidates replace Q and R)")
+        mats = {"Q": [], "R": []}
+        for c, pair in enumerate(candidate_pairs(candidates)):
+            for name, M in zip(("Q", "R"), pair):
+                M = _as55(f"candidate {c} {name}", M)
+                if not np.array_equal(M, M.T):
+                    raise ValueError(f"candidate {c}: {name} must be symmetric")
+                if not np.all(np.isfinite(M)):
+                    raise ValueError(f"candidate {c}: {name} must be finite")
+                mats[name].append(M.reshape(-1))
+        Q, R = np.stack(mats["Q"]), np.stack(mats["R"])
+        p, i = self._problem(b), self._inputs(b)
+        with torch.cuda.device(b.device):
+            return launch_scores(self._lib.ste_ukf_score_n_f64, p, i, [list(range(len(Q)))], Q, R, b.device)
 
     def run_many(self, batches: Sequence[TrackBatchN], results: Sequence[TrackResultsN]) -> None:
         """Filter and smooth a sequence of resident tiles (e.g. :meth:`TrackBatchN.fleet_tiles`): two launches per tile,

@@ -33,6 +33,14 @@ struct KernelArgs {
     SteOutputs out;
 };
 
+// The scoring launch (ste_ukf_score_f64): the tile's arguments, the per-(candidate, track) sums and the candidate table,
+// all in the kernel parameters.  Candidate blockIdx.y replaces prob.Q / prob.R; `out` is unused (zero).
+struct KernelArgsScore : KernelArgs {
+    SteScores scores;
+    double Q[STE_MAX_CANDIDATES][16];
+    double R[STE_MAX_CANDIDATES][16];
+};
+
 // Covariance storage: 16 planes per state (the full row-major 4x4 the reference returns) or, with
 // STE_FLAG_PACKED_COV, only the 10 unique entries in SYM() order.  Both passes keep covariances
 // exactly symmetric, so the packed form loses nothing; it cuts the state traffic by 30 %.
@@ -88,11 +96,16 @@ STE_DEV bool any_nonfinite(const double (&x)[4], const double (&P)[10]) {
 //
 // The time loop is written as begin() / step(s) / end() on a small state object.
 // INNOV: every update also stores its innovation statistics (struct Innov) into row u of the planes of `iv`.
+// SCORE: the scoring form - candidate `cand` of `sa` supplies Q and R, nothing is stored per step (no states, no
+// smoother tape, no gating planes: the robustification itself still runs) and the statistics of the updates are summed
+// in update order, then written once per track into the candidate's row of sa->scores.
 // ------------------------------------------------------------------------------------------ //
-template <bool POS_ONLY, bool GATING, bool INNOV = false>
+template <bool POS_ONLY, bool GATING, bool INNOV = false, bool SCORE = false>
 struct ForwardTrack {
     const KernelArgs &a;
     const SteInnovations *iv;
+    const KernelArgsScore *sa;
+    const int cand;
     const int t;
     const Scratch sc;
     const int64_t ld;
@@ -107,9 +120,23 @@ struct ForwardTrack {
     int rep = 1, ri = 0, rc = 0;
     int sub_left = 1;   // predicts left until the next update when the cadence is "every k-th step"
     bool consistent = true, upd_next = false;
+    double loglik_sum = 0.0, nis_sum = 0.0;   // SCORE: sums over the updates so far
+    int dof_sum = 0;
 
-    STE_DEV ForwardTrack(const KernelArgs &args, int track, const Scratch &scratch, const SteInnovations *innov = nullptr)
-        : a(args), iv(innov), t(track), sc(scratch), ld(args.prob.ld), packed((args.prob.flags & STE_FLAG_PACKED_COV) != 0) {}
+    STE_DEV ForwardTrack(const KernelArgs &args, int track, const Scratch &scratch, const SteInnovations *innov = nullptr,
+                         const KernelArgsScore *score = nullptr, int candidate = 0)
+        : a(args), iv(innov), sa(score), cand(candidate), t(track), sc(scratch), ld(args.prob.ld),
+          packed((args.prob.flags & STE_FLAG_PACKED_COV) != 0) {}
+
+    // the process and measurement noise of the run: the tile's, or (SCORE) the candidate's
+    STE_DEV const double *Qm() const {
+        if constexpr (SCORE) return sa->Q[cand];
+        else return a.prob.Q;
+    }
+    STE_DEV const double *Rm() const {
+        if constexpr (SCORE) return sa->R[cand];
+        else return a.prob.R;
+    }
 
     // observation rows are staged into scratch a whole predict ahead of their use
     // row u of a [row][track] input array for this track: base + t, then one 32 x 32 + 64-bit multiply-add (plane_ptr)
@@ -139,7 +166,7 @@ struct ForwardTrack {
     STE_DEV void assimilate(int u) {
         // a per-track measurement covariance (SteInputs.R_tracks: ships with different sensors) replaces the
         // shared R; only the generic update reads a full 4x4 R
-        const double *Rp = a.prob.R;
+        const double *Rp = Rm();
         double Rt[16];
         if constexpr (!POS_ONLY) {
             if (a.in.R_tracks) {
@@ -148,7 +175,7 @@ struct ForwardTrack {
                 Rp = Rt;
             }
         }
-        const Model model{a.prob.H, a.prob.Q, Rp};
+        const Model model{a.prob.H, Qm(), Rp};
         double z[4], un[4];
         stage_wait();
 #pragma unroll
@@ -163,10 +190,10 @@ struct ForwardTrack {
         double lam, rs;
         Innov st;
         if (POS_ONLY)
-            ukf_update_position<GATING, INNOV>(x, P, model, z, noise, a.prob.gate_chi, a.prob.gate_max_iter, status, it, lam, rs, &st);
+            ukf_update_position<GATING, INNOV || SCORE>(x, P, model, z, noise, a.prob.gate_chi, a.prob.gate_max_iter, status, it, lam, rs, &st);
         else
-            ukf_update_generic<GATING, INNOV>(x, P, model, z, noise, a.prob.gate_chi, a.prob.gate_max_iter, status, it, lam, rs, &st);
-        if (GATING) {
+            ukf_update_generic<GATING, INNOV || SCORE>(x, P, model, z, noise, a.prob.gate_chi, a.prob.gate_max_iter, status, it, lam, rs, &st);
+        if (GATING && !SCORE) {
             if (a.out.gate_iters) a.out.gate_iters[(int64_t)u * ld + t] = (uint8_t)min_(it, 255);
             if (a.out.gate_lambda) a.out.gate_lambda[(int64_t)u * ld + t] = lam;
             if (a.out.gate_scale) a.out.gate_scale[(int64_t)u * ld + t] = rs;
@@ -176,6 +203,11 @@ struct ForwardTrack {
             iv->nis[row] = st.nis;
             iv->loglik[row] = -0.5 * fma((double)st.rank, kLog2Pi, st.nis + st.log_pdet);
             iv->rank[row] = (uint8_t)st.rank;
+        }
+        if constexpr (SCORE) {   // the expression the innovation planes store, added in update order
+            loglik_sum += -0.5 * fma((double)st.rank, kLog2Pi, st.nis + st.log_pdet);
+            nis_sum += st.nis;
+            dof_sum += st.rank;
         }
     }
 
@@ -190,7 +222,7 @@ struct ForwardTrack {
 #pragma unroll
             for (int j = i; j < 4; ++j)
                 P[SYM(i, j)] = a.in.P0 ? a.in.P0[(i * 4 + j) * ld + t] : a.prob.P0[i * 4 + j];
-        store_state(a.out.mean_f, a.out.cov_f, ld, 0, t, packed, x, P);  // the prior (kalman_filter.py:76-77)
+        if constexpr (!SCORE) store_state(a.out.mean_f, a.out.cov_f, ld, 0, t, packed, x, P);  // the prior (kalman_filter.py:76-77)
 #pragma unroll
         for (int r = 0; r < 4; ++r) sc.at(kScratchObs + r) = 0.0;   // absent rows read as 0
         stage_obs(0);
@@ -219,33 +251,44 @@ struct ForwardTrack {
             stage_step(s + 1, ui + (advance ? 1 : 0));
             upd_next = step_updates(s + 1);
         }
-        double *stats = a.out.smooth_stats ? a.out.smooth_stats + ((int64_t)s * kStatsPlanes) * ld + t : nullptr;
+        double *stats = (!SCORE && a.out.smooth_stats) ? a.out.smooth_stats + ((int64_t)s * kStatsPlanes) * ld + t : nullptr;
         double e[4] = {0.0, 0.0, 0.0, 0.0};
         if (a.in.noise_pred) {
 #pragma unroll
             for (int r = 0; r < 4; ++r)
-                e[r] = a.in.noise_pred[((int64_t)s * 4 + r) * ld + t] * sqrt(a.prob.Q[r * 5]);
+                e[r] = a.in.noise_pred[((int64_t)s * 4 + r) * ld + t] * sqrt(Qm()[r * 5]);
         }
-        ukf_predict(x, P, a.prob.Q, dt, sr, cr, e, status, sc, nullptr, nullptr, stats, ld, !(a.prob.flags & STE_FLAG_LONG_STEPS),
+        ukf_predict(x, P, Qm(), dt, sr, cr, e, status, sc, nullptr, nullptr, stats, ld, !(a.prob.flags & STE_FLAG_LONG_STEPS),
                     a.in.noise_pred != nullptr);
         // more matched update times than observation rows: the reference raises IndexError here
         // (kalman_filter.py:101-108); the track is flagged and the update skipped, nothing is re-read
         if (advance) assimilate(++ui);
         else stage_wait();   // the next step's inputs must have landed before they are read
-        store_state(a.out.mean_f, a.out.cov_f, ld, s + 1, t, packed, x, P);
+        if constexpr (!SCORE) store_state(a.out.mean_f, a.out.cov_f, ld, s + 1, t, packed, x, P);
     }
 
     STE_DEV void end() {
         if (any_nonfinite(x, P)) status |= STE_STATUS_NONFINITE;
-        if (a.out.smooth_stats && !consistent) status |= STE_STATUS_SMOOTH_RECOMPUTE;
-        a.out.status[t] = status;
-        if (a.out.n_updates) a.out.n_updates[t] = ui + 1;
+        if constexpr (SCORE) {
+            const SteScores &o = sa->scores;
+            const int64_t row = (int64_t)cand * o.ld_out + t;
+            o.loglik[row] = loglik_sum;
+            o.nis[row] = nis_sum;
+            o.dof[row] = dof_sum;
+            o.n_updates[row] = ui + 1;
+            o.status[row] = status;
+        } else {
+            if (a.out.smooth_stats && !consistent) status |= STE_STATUS_SMOOTH_RECOMPUTE;
+            a.out.status[t] = status;
+            if (a.out.n_updates) a.out.n_updates[t] = ui + 1;
+        }
     }
 };
 
-template <bool POS_ONLY, bool GATING, bool INNOV = false>
-STE_DEV void forward_track(const KernelArgs &a, const int t, const Scratch &sc, const SteInnovations *iv = nullptr) {
-    ForwardTrack<POS_ONLY, GATING, INNOV> f(a, t, sc, iv);
+template <bool POS_ONLY, bool GATING, bool INNOV = false, bool SCORE = false>
+STE_DEV void forward_track(const KernelArgs &a, const int t, const Scratch &sc, const SteInnovations *iv = nullptr,
+                           const KernelArgsScore *sa = nullptr, int cand = 0) {
+    ForwardTrack<POS_ONLY, GATING, INNOV, SCORE> f(a, t, sc, iv, sa, cand);
     f.begin();
 #if defined(STE_STEP_SYNC) && defined(__CUDA_ARCH__)
     // experiment: the warps of a block start every step together (instruction-cache locality); ragged lengths are safe,

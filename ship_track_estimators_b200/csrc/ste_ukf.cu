@@ -6,6 +6,7 @@
 // contiguous 256-byte segment.  The kernels are bound by the FP64 pipe (about 26 flop per
 // algorithmic byte, DESIGN.md), so the time loop keeps every matrix in registers and
 // prefetches the next step's inputs while the current step computes.
+#include <cmath>
 #include <cstdio>
 #include <cstring>
 
@@ -52,6 +53,16 @@ __global__ void __launch_bounds__(kThreads, STE_FWD_MIN_BLOCKS) ukf_forward_kern
     } else {
         if (t < a.prob.n_tracks) forward_track<POS_ONLY, GATING>(a, t, Scratch{scratch + threadIdx.x, kThreads});
     }
+}
+
+// Scoring form of the forward pass (ste_ukf_score_f64): blockIdx.y is the candidate, so every warp reads one candidate's
+// Q and R from the parameter block.  Each (candidate, track) pair runs forward_track's arithmetic with the candidate's
+// matrices and writes only its sums.
+template <bool POS_ONLY, bool GATING>
+__global__ void __launch_bounds__(kThreads, STE_FWD_MIN_BLOCKS) ukf_score_kernel(const __grid_constant__ KernelArgsScore a) {
+    extern __shared__ double scratch[];   // kScratchSlotsFwd * kThreads doubles, as the forward pass
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t < a.prob.n_tracks) forward_track<POS_ONLY, GATING, false, true>(a, t, Scratch{scratch + threadIdx.x, kThreads}, nullptr, &a, blockIdx.y);
 }
 
 // TAPE: the launch has a statistics tape (same code either way; only the register budget differs)
@@ -602,6 +613,63 @@ __global__ void __launch_bounds__(kThreadsN) ukf_forward_n_kernel(const __grid_c
     if (a.out.n_updates) a.out.n_updates[t] = ui + 1;
 }
 
+// Scoring form of ukf_forward_n_kernel (ste_ukf_score_n_f64): the same time loop, predict_core / update_core calls and
+// statistics, with the Q and R of candidate blockIdx.y (so every warp reads one candidate's matrices) and no stored state;
+// the statistics of the updates are summed in update order and written once per (candidate, track).
+struct ScoreArgsN {
+    ProblemN p;
+    double P0[kMaxN * kMaxN];   // shared prior, row-major n x n
+    int32_t max_steps, max_obs;
+    SteInputsN in;
+    SteScores scores;
+    double Q[STE_MAX_CANDIDATES][25], R[STE_MAX_CANDIDATES][25];   // row-major n x n per candidate
+};
+
+template <int NC>
+__global__ void __launch_bounds__(kThreadsN) ukf_score_n_kernel(const __grid_constant__ ScoreArgsN a) {
+    static_assert(NC * NC <= 25, "the candidate table holds 5 x 5 matrices");
+    constexpr int D = DimN<NC>::LD, n = NC;
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= a.p.n_tracks) return;
+    const int c = blockIdx.y;
+    const SteInputsN &in = a.in;
+    const int64_t ld = a.p.ld;
+    const int nt = in.n_steps ? min(in.n_steps[t], a.max_steps) : a.max_steps;
+    const double *Q = a.Q[c], *R = a.R[c];
+    double x[D], P[D * D], z[D];
+    for (int r = 0; r < n; ++r) x[r] = in.x0[r * ld + t];
+    for (int i = 0; i < n; ++i)
+        for (int j = 0; j < n; ++j) P[i * D + j] = in.P0 ? in.P0[(i * n + j) * ld + t] : a.P0[i * n + j];
+    double loglik = 0.0, nis = 0.0;
+    int dof = 0;
+    auto update = [&](int u) {   // observation row u; rows the caller left NULL read as 0
+        for (int r = 0; r < n; ++r) z[r] = in.z[r] ? in.z[r][(int64_t)u * ld + t] : 0.0;
+        ste::Innov st;
+        const int bits = update_core<NC, true>(a.p, R, x, P, z, in.noise_upd ? in.noise_upd + (int64_t)u * n * ld + t : nullptr, ld, &st);
+        loglik += -0.5 * fma((double)st.rank, kLog2Pi, st.nis + st.log_pdet);   // the loglik plane's expression
+        nis += st.nis;
+        dof += st.rank;
+        return bits;
+    };
+    int status = update(0), ui = 0;
+    for (int s = 0; s < nt; ++s) {
+        const double d = in.dt[(int64_t)s * ld + t], sr = in.sog_rate[(int64_t)ui * ld + t],
+                     cr = in.cog_rate ? in.cog_rate[(int64_t)ui * ld + t] : 0.0;
+        status |= predict_core<NC>(a.p, Q, x, P, d, sr, cr, in.noise_pred ? in.noise_pred + (int64_t)s * n * ld + t : nullptr, ld,
+                                   nullptr, nullptr, 0);
+        if (in.upd_mask[(int64_t)s * ld + t]) {
+            if (ui + 1 < a.max_obs) status |= update(++ui);
+            else status |= STE_STATUS_OBS_OVERRUN;
+        }
+    }
+    const int64_t row = (int64_t)c * a.scores.ld_out + t;
+    a.scores.loglik[row] = loglik;
+    a.scores.nis[row] = nis;
+    a.scores.dof[row] = dof;
+    a.scores.n_updates[row] = ui + 1;
+    a.scores.status[row] = status;
+}
+
 // UnscentedKalmanFilter.rts_step (unscented.py:267-351) over ragged tracks: n_states = n_steps[t] + 1 and rate_repeat[t]
 // per track; the status bits are OR-ed into the forward pass's.  Q as in the forward pass (PerTrack: noise.Q_tracks set).
 template <int NC, bool PerTrack>
@@ -728,6 +796,13 @@ static bool is_symmetric(const double *M) {
     return true;
 }
 
+static bool is_symmetric_n(int n, const double *M) {
+    for (int i = 0; i < n; ++i)
+        for (int j = 0; j < i; ++j)
+            if (M[i * n + j] != M[j * n + i]) return false;
+    return true;
+}
+
 // H == diag(1,1,0,0) exactly and R zero outside its leading 2x2 block
 static bool position_only(const SteProblem &p) {
     if (p.flags & STE_FLAG_FORCE_GENERIC) return false;
@@ -760,11 +835,19 @@ int ste_version(void) { return STE_ABI_VERSION; }
 
 const char *ste_last_error(void) { return g_err; }
 
+static int forward_input_rules(const SteProblem *prob, const SteInputs *in);
+
 static int validate_forward(const SteProblem *prob, const SteInputs *in, const SteOutputs *out) {
     if (int rc = validate_problem(prob)) return rc;
     if (!in || !out) return fail(STE_ERR_INVALID_ARG, "null SteInputs/SteOutputs");
     if (!in->x0 || !in->dt || !in->sog_rate || !in->cog_rate) return fail(STE_ERR_INVALID_ARG, "missing input array");
     if (!out->mean_f || !out->cov_f || !out->status) return fail(STE_ERR_INVALID_ARG, "missing output array");
+    return forward_input_rules(prob, in);
+}
+
+// what the forward pass requires of a tile's inputs beyond their presence: gating without measurement noise, the update
+// variant a per-track R needs, and every observation row the update reads
+static int forward_input_rules(const SteProblem *prob, const SteInputs *in) {
     const bool gating = (prob->flags & STE_FLAG_GATING) != 0;
     if (gating && in->noise_upd)
         return fail(STE_ERR_UNSUPPORTED, "gating draws a data-dependent number of normals; only zero measurement noise is supported with it");
@@ -840,6 +923,73 @@ int ste_ukf_forward_innov_f64(const SteProblem *prob, const SteInputs *in, const
     static_cast<KernelArgs &>(a) = kernel_args(prob, in, out);
     a.innov = *innov;
     return launch_forward<true>(pos, gating, a, s);
+}
+
+// ------------------------------------------------------------------------------------------ //
+// Noise-candidate scores (ste_ukf_score_f64 / ste_ukf_score_n_f64)
+// ------------------------------------------------------------------------------------------ //
+static int validate_candidates(const SteCandidates *cand, int n) {
+    if (!cand || !cand->Q || !cand->R) return fail(STE_ERR_INVALID_ARG, "null SteCandidates table or matrix");
+    if (cand->n_cand < 1 || cand->n_cand > STE_MAX_CANDIDATES)
+        return fail(STE_ERR_INVALID_ARG, "SteCandidates.n_cand outside [1, STE_MAX_CANDIDATES]");
+    for (int c = 0; c < cand->n_cand; ++c) {
+        const double *Q = cand->Q + (size_t)c * n * n, *R = cand->R + (size_t)c * n * n;
+        for (int k = 0; k < n * n; ++k)
+            if (!std::isfinite(Q[k]) || !std::isfinite(R[k])) return fail(STE_ERR_UNSUPPORTED, "a candidate Q or R is not finite");
+        if (!is_symmetric_n(n, Q) || !is_symmetric_n(n, R)) return fail(STE_ERR_UNSUPPORTED, "candidate Q and R must be symmetric");
+    }
+    return STE_OK;
+}
+
+static int validate_scores(const SteScores *sc, int32_t n_tracks) {
+    if (!sc || !sc->loglik || !sc->nis || !sc->dof || !sc->n_updates || !sc->status)
+        return fail(STE_ERR_INVALID_ARG, "SteScores needs all five planes (loglik, nis, dof, n_updates, status)");
+    if (sc->ld_out < n_tracks) return fail(STE_ERR_INVALID_ARG, "SteScores.ld_out < n_tracks");
+    return STE_OK;
+}
+
+extern "C++" {
+template <bool POS_ONLY, bool GATING>
+static int launch_score(const KernelArgsScore &a, int n_cand, cudaStream_t s) {
+    const dim3 grid((a.prob.n_tracks + kThreads - 1) / kThreads, n_cand), block(kThreads);
+    const size_t smem = sizeof(double) * kScratchSlotsFwd * kThreads;
+    if (cudaFuncSetAttribute(ukf_score_kernel<POS_ONLY, GATING>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+        return check_launch("cudaFuncSetAttribute(ukf_score_kernel)");
+    ukf_score_kernel<POS_ONLY, GATING><<<grid, block, smem, s>>>(a);
+    return check_launch("ukf_score_kernel");
+}
+}  // extern "C++"
+
+int ste_ukf_score_f64(const SteProblem *prob, const SteInputs *in, const SteCandidates *cand, SteScores *scores, void *stream) {
+    if (!prob || !in) return fail(STE_ERR_INVALID_ARG, "null SteProblem / SteInputs");
+    if (int rc = validate_candidates(cand, 4)) return rc;
+    if (int rc = validate_scores(scores, prob->n_tracks)) return rc;
+    if (in->R_tracks)
+        return fail(STE_ERR_INVALID_ARG, "a tile with its own R (SteInputs.R_tracks) cannot be scored: the candidates replace R");
+    KernelArgsScore a{};
+    bool pos = false;
+    for (int c = 0; c < cand->n_cand; ++c) {
+        SteProblem pc = *prob;   // the tile as the forward pass would see it with candidate c
+        memcpy(pc.Q, cand->Q + c * 16, sizeof(pc.Q));
+        memcpy(pc.R, cand->R + c * 16, sizeof(pc.R));
+        if (int rc = validate_problem(&pc)) return rc;
+        if (!in->x0 || !in->dt || !in->sog_rate || !in->cog_rate) return fail(STE_ERR_INVALID_ARG, "missing input array");
+        if (int rc = forward_input_rules(&pc, in)) return rc;
+        const bool pc_pos = position_only(pc);
+        if (c > 0 && pc_pos != pos)
+            return fail(STE_ERR_UNSUPPORTED, "the candidates' R select different updates (position-only and generic): score them in separate calls");
+        pos = pc_pos;
+        memcpy(a.Q[c], pc.Q, sizeof(pc.Q));
+        memcpy(a.R[c], pc.R, sizeof(pc.R));
+    }
+    if (prob->n_tracks == 0) return STE_OK;
+    a.prob = *prob;
+    a.in = *in;
+    a.scores = *scores;
+    const bool gating = (prob->flags & STE_FLAG_GATING) != 0;
+    cudaStream_t s = (cudaStream_t)stream;
+    if (pos) return gating ? launch_score<true, true>(a, cand->n_cand, s) : launch_score<true, false>(a, cand->n_cand, s);
+    return gating ? launch_score<false, true>(a, cand->n_cand, s) : launch_score<false, false>(a, cand->n_cand, s);
 }
 
 int ste_urtss_backward_f64(const SteProblem *prob, const SteInputs *in, SteOutputs *out, void *stream) {
@@ -979,13 +1129,6 @@ int ste_urtss_backward_n_f64(int32_t n, int32_t model, int32_t n_tracks, int64_t
     return check_launch("urtss_backward_n_kernel");
 }
 
-static bool is_symmetric_n(int n, const double *M) {
-    for (int i = 0; i < n; ++i)
-        for (int j = 0; j < i; ++j)
-            if (M[i * n + j] != M[j * n + i]) return false;
-    return true;
-}
-
 // the problem checks shared by the fleet passes and the five-state metrics
 static int validate_problem_n(const SteProblemN *p) {
     if (p->model == STE_MODEL_GEODETIC && p->n == 4)
@@ -1055,6 +1198,35 @@ int ste_ukf_forward_innov_n_f64(const SteProblemN *prob, const SteInputsN *in, c
         ukf_forward_n_kernel<5, false><<<blocks, kThreadsN, 0, s>>>(a);
     }
     return check_launch("ukf_forward_n_kernel");
+}
+
+int ste_ukf_score_n_f64(const SteProblemN *prob, const SteInputsN *in, const SteCandidates *cand, SteScores *scores, void *stream) {
+    if (!prob || !in) return fail(STE_ERR_INVALID_ARG, "null SteProblemN / SteInputsN");
+    if (int rc = validate_candidates(cand, 5)) return rc;
+    if (int rc = validate_scores(scores, prob->n_tracks)) return rc;
+    ScoreArgsN a{};
+    for (int c = 0; c < cand->n_cand; ++c) {
+        SteProblemN pc = *prob;   // the tile as the forward pass would see it with candidate c
+        memcpy(pc.Q, cand->Q + c * 25, sizeof(double) * 25);
+        memcpy(pc.R, cand->R + c * 25, sizeof(double) * 25);
+        if (int rc = validate_problem_n(&pc)) return rc;
+        memcpy(a.Q[c], pc.Q, sizeof(a.Q[c]));
+        memcpy(a.R[c], pc.R, sizeof(a.R[c]));
+    }
+    if (!in->x0 || !in->dt || !in->sog_rate || !in->upd_mask) return fail(STE_ERR_INVALID_ARG, "missing input array");
+    if (prob->n_tracks == 0) return STE_OK;
+    const int n = prob->n;
+    a.p.n = n; a.p.model = prob->model; a.p.n_tracks = prob->n_tracks; a.p.ld = prob->ld;
+    memcpy(a.p.H, prob->H, sizeof(double) * n * n);
+    memcpy(a.p.Q, prob->Q, sizeof(double) * n * n);
+    memcpy(a.p.R, prob->R, sizeof(double) * n * n);
+    memcpy(a.P0, prob->P0, sizeof(double) * n * n);
+    a.max_steps = prob->max_steps; a.max_obs = prob->max_obs;
+    a.in = *in;
+    a.scores = *scores;
+    const dim3 grid((prob->n_tracks + kThreadsN - 1) / kThreadsN, cand->n_cand);
+    ukf_score_n_kernel<5><<<grid, kThreadsN, 0, (cudaStream_t)stream>>>(a);
+    return check_launch("ukf_score_n_kernel");
 }
 
 int ste_urtss_backward_tracks_n_f64(const SteProblemN *prob, const SteInputsN *in, SteOutputsN *out, void *stream) {

@@ -92,9 +92,9 @@ def innovation_metrics(res) -> Dict[str, torch.Tensor]:
     ``track_metrics`` cannot choose ``R``: it compares the *updated* state with the fix just assimilated, and that
     residual shrinks as ``R`` goes to zero because the filter snaps to its fixes.  The likelihood scores each fix before
     it is assimilated, against the spread ``S = H P H^T + R`` the filter predicted for it, so an ``R`` (or ``Q``) too small
-    is penalised by large innovations and one too large by a large ``log det S``.  Packing the same ships once per
-    candidate ``(Q, R)`` (per-track planes) scores every candidate in one launch: the largest summed ``loglik`` is the
-    maximum-likelihood choice.  For a consistent filter ``nis`` follows a chi-squared law with ``dof`` degrees of freedom.
+    is penalised by large innovations and one too large by a large ``log det S``: the largest summed ``loglik`` is the
+    maximum-likelihood choice.  ``BatchedUKF.score`` / ``BatchedUKFN.score`` compute these sums for many candidates
+    ``(Q, R)`` at once without storing any state, and ``tuning.fit_noise`` chooses among them.  For a consistent filter ``nis`` follows a chi-squared law with ``dof`` degrees of freedom.
     """
     if res.nis is None or res.loglik is None or res.innov_rank is None:
         raise ValueError("results hold no innovation statistics: allocate(..., innovations=True) before the forward pass")
