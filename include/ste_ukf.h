@@ -45,6 +45,8 @@ extern "C" {
                             /*    (per-update innovation statistics of the forward passes)                                               */
                             /*    additive, no struct changed: SteCandidates, SteScores, ste_ukf_score_f64, ste_ukf_score_n_f64           */
                             /*    (log-likelihood scores of many noise candidates per track in one launch)                               */
+                            /*    additive, no struct changed: ste_ukf_forward_noise_f64, ste_urtss_backward_noise_f64                    */
+                            /*    (per-track Q of the n = 4 passes, in SteNoiseN)                                                          */
 #define STE_STATS_PLANES 15
 #define STE_DIM 4
 #define STE_NSIGMA 9
@@ -308,6 +310,24 @@ int ste_ukf_forward_innov_f64(const SteProblem *prob, const SteInputs *in, const
                               SteOutputs *out, void *stream);
 int ste_ukf_forward_innov_n_f64(const SteProblemN *prob, const SteInputsN *in, const SteNoiseN *noise,
                                 const SteInnovations *innov, SteOutputsN *out, void *stream);
+
+/* Per-track process noise on the n = 4 passes, for fleets that mix ship classes: ste_ukf_forward_innov_f64 and
+ * ste_urtss_backward_f64 with each track's own Q.  noise->Q_tracks holds row-major 4 x 4 planes [16][ld] in the layout of
+ * SteInputs.P0, element (i, j) of track t at base[(i * 4 + j) * ld + t]; each replaces SteProblem.Q for its track
+ * wherever the passes read Q, noise tapes included (scaled by that track's sqrt(diag Q)).  Such a track is bit-identical
+ * to the same track run with its matrix as the launch's SteProblem.Q.
+ *  - noise == NULL or noise->Q_tracks == NULL: exactly ste_ukf_forward_innov_f64 / ste_urtss_backward_f64.
+ *  - noise->R_tracks must be NULL (STE_ERR_INVALID_ARG before any launch): at n = 4 a per-track R travels in
+ *    SteInputs.R_tracks.
+ *  - Everything else is checked as by those entry points.
+ * The backward pass must receive the same Q_tracks as the forward pass that wrote its statistics tape: the tape's
+ * predicted covariance includes the track's Q.  The planes must be symmetric: the library cannot read device memory
+ * before the launch, so the caller checks it (the Python layer, batch.TrackBatch, does).  The fused pass
+ * (ste_ukf_fused_f64) and the scores (ste_ukf_score_f64) take no per-track Q. */
+int ste_ukf_forward_noise_f64(const SteProblem *prob, const SteInputs *in, const SteNoiseN *noise, const SteInnovations *innov,
+                              SteOutputs *out, void *stream);
+int ste_urtss_backward_noise_f64(const SteProblem *prob, const SteInputs *in, const SteNoiseN *noise, SteOutputs *out,
+                                 void *stream);
 
 /* Scores of many noise candidates, for choosing Q and R by maximum likelihood (a grid search): one store-free forward
  * pass per (candidate, track) pair.  Candidate c's Q and R replace SteProblem(N).Q / R; everything else - H, P0, gating,

@@ -209,6 +209,10 @@ _PROTOTYPES = {
                                             C.c_void_p]),
     "ste_ukf_forward_innov_n_f64": (C.c_int, [C.POINTER(SteProblemN), C.POINTER(SteInputsN), C.POINTER(SteNoiseN), C.POINTER(SteInnovations),
                                               C.POINTER(SteOutputsN), C.c_void_p]),
+    "ste_ukf_forward_noise_f64": (C.c_int, [C.POINTER(SteProblem), C.POINTER(SteInputs), C.POINTER(SteNoiseN), C.POINTER(SteInnovations),
+                                            C.POINTER(SteOutputs), C.c_void_p]),
+    "ste_urtss_backward_noise_f64": (C.c_int, [C.POINTER(SteProblem), C.POINTER(SteInputs), C.POINTER(SteNoiseN), C.POINTER(SteOutputs),
+                                               C.c_void_p]),
     "ste_ukf_score_f64": (C.c_int, [C.POINTER(SteProblem), C.POINTER(SteInputs), C.POINTER(SteCandidates), C.POINTER(SteScores), C.c_void_p]),
     "ste_ukf_score_n_f64": (C.c_int, [C.POINTER(SteProblemN), C.POINTER(SteInputsN), C.POINTER(SteCandidates), C.POINTER(SteScores),
                                       C.c_void_p]),

@@ -17,7 +17,7 @@ the reference's own arithmetic (numpy fp64):
 from __future__ import annotations
 
 import ctypes as C
-from dataclasses import dataclass, field
+from dataclasses import dataclass, field, replace
 from typing import Dict, List, Optional, Sequence
 
 import numpy as np
@@ -34,6 +34,21 @@ def _as44(name: str, M) -> np.ndarray:
             "[lon, lat, SOG, COG] (the reference's update/rts_step hard-code state index 3 as heading)"
         )
     return np.ascontiguousarray(M)
+
+
+def track_planes(name: str, mats: Sequence, T: int) -> np.ndarray:
+    """``[16][T]`` row-major planes of one symmetric 4 x 4 matrix per track (the layout of ``SteInputs.R_tracks`` and
+    ``SteNoiseN.Q_tracks``), column ``i`` from ``mats[i]``.  ``ValueError`` for a wrong count; a wrong shape or an asymmetric
+    matrix raises as ``from_tracks(R=)`` does.  The kernels cannot check symmetry, so per-track matrices pass through here."""
+    if len(mats) != T:
+        raise ValueError(f"{name}: {len(mats)} matrices for {T} tracks (one 4 x 4 matrix per track)")
+    out = np.empty((16, T))
+    for i, M in enumerate(mats):
+        M = _as44(f"{name}[{i}]", M)
+        if not np.array_equal(M, M.T):
+            raise NotImplementedError(f"per-track {name} must be symmetric for the CUDA path ({name}[{i}] is not)")
+        out[:, i] = M.reshape(-1)
+    return out
 
 
 @dataclass
@@ -151,6 +166,9 @@ class TrackBatch:
     # take the next longest tracks): column j holds the caller's track order[j]; None = caller's order
     order: Optional[np.ndarray] = None
     _long_fraction: Optional[float] = field(default=None, repr=False, compare=False)
+    # per-track process noise (fleets mixing ship classes): row-major 4 x 4 planes replacing the filter's shared Q for
+    # each track in both passes (symmetric: from_tracks and with_noise check it; check() cannot without a synchronisation)
+    Q: Optional[torch.Tensor] = None  # [16][T]
 
     @property
     def n_tracks(self) -> int:
@@ -185,7 +203,8 @@ class TrackBatch:
                    ("cog_rate", self.cog_rate, (M, T), f64), ("upd_mask", self.upd_mask, (N, T), torch.uint8),
                    ("n_steps", self.n_steps, (T,), torch.int32), ("rate_repeat", self.rate_repeat, (T,), torch.int32),
                    ("P0", self.P0, (16, T), f64), ("R", self.R, (16, T), f64), ("noise_pred", self.noise_pred, (N, 4, T), f64),
-                   ("noise_upd", self.noise_upd, (M, 4, T), f64), ("noise_bwd", self.noise_bwd, (N, 4, T), f64)]
+                   ("noise_upd", self.noise_upd, (M, 4, T), f64), ("noise_bwd", self.noise_bwd, (N, 4, T), f64),
+                   ("Q", self.Q, (16, T), f64)]
         expect += [(f"z[{r}]", zr, (M, T), f64) for r, zr in enumerate(self.z)]
         for name, t, shape, dtype in expect:
             if t is None:
@@ -226,7 +245,7 @@ class TrackBatch:
         return float(((km > limit_km) & valid).sum()) / total if total else 0.0
 
     _TENSORS = ("x0", "dt", "sog_rate", "cog_rate", "upd_mask", "n_steps", "rate_repeat", "P0", "R",
-                "noise_pred", "noise_upd", "noise_bwd")
+                "noise_pred", "noise_upd", "noise_bwd", "Q")
 
     def _map(self, fn) -> "TrackBatch":
         kw = {name: (None if getattr(self, name) is None else fn(getattr(self, name))) for name in self._TENSORS}
@@ -265,6 +284,19 @@ class TrackBatch:
             t = getattr(self, name)
             total += 0 if t is None else t.numel() * t.element_size()
         return int(total)
+
+    def with_noise(self, Q: Optional[Sequence[np.ndarray]] = None, R: Optional[Sequence[np.ndarray]] = None) -> "TrackBatch":
+        """This tile with per-track noise: ``Q`` / ``R`` give one symmetric 4 x 4 matrix per ship in the caller's (ship)
+        order, checked as by :meth:`from_tracks`, and column j gets the matrix of ship ``order[j]``.  A set that is given
+        replaces the tile's own, one that is not keeps it; every other tensor is shared.  For tiles built on the device
+        (``FleetFixes.to_batch``, ``read_csv_fleet_device``, :meth:`from_synthetic`), which take no matrices themselves.
+        A per-track ``R`` selects the generic update, as :meth:`from_tracks` with ``R`` does."""
+        kw = {}
+        for name, mats in (("Q", Q), ("R", R)):
+            if mats is not None:
+                pl = track_planes(name, mats, self.n_tracks)
+                kw[name] = torch.from_numpy(np.ascontiguousarray(pl if self.order is None else pl[:, self.order])).to(self.device)
+        return replace(self, **kw)
 
     # ------------------------------------------------------------------ #
     @classmethod
@@ -327,6 +359,7 @@ class TrackBatch:
         smoother: bool = True,
         sort_by_length: bool = True,
         R: Optional[Sequence[np.ndarray]] = None,
+        Q: Optional[Sequence[np.ndarray]] = None,
     ):
         """Pack ``ShipTrack``-like objects (attributes ``dts, z, sog_rate, cog_rate``) with their step
         grids ``dt_arrays`` (what ``run(nsteps, dt, ship_track)`` receives).
@@ -336,7 +369,9 @@ class TrackBatch:
         as long as its work, not as its longest track times its width.  ``TrackBatch.order`` records
         the permutation and ``TrackResults.track(i)`` undoes it - ``i`` is always the caller's index,
         and every track's numbers are bit-identical to the unsorted packing.  ``R``: one symmetric
-        4 x 4 measurement covariance per track (instead of the filter's shared one).
+        4 x 4 measurement covariance per track (instead of the filter's shared one).  ``Q``: one symmetric 4 x 4
+        process noise matrix per track, in the caller's order, used by both passes instead of the filter's shared one:
+        each track equals a filter built with its own ``Q``.  ``ValueError`` for a wrong count of either.
 
         Raises ``IndexError`` where the reference would: more matched observation times than
         observations (``kalman_filter.py:101-108``) or a smoother rate index past the repeated rate
@@ -345,6 +380,7 @@ class TrackBatch:
         T = len(tracks)
         if T == 0:
             raise ValueError("empty batch")
+        Qt = None if Q is None else track_planes("Q", Q, T)
         dt_arrays = [np.asarray(d, dtype=np.float64).reshape(-1) for d in dt_arrays]
         order = length_order([len(d) for d in dt_arrays]) if sort_by_length else None
         if order is not None:
@@ -386,6 +422,8 @@ class TrackBatch:
             if not np.array_equal(Rt.reshape(4, 4, T), Rt.reshape(4, 4, T).transpose(1, 0, 2)):
                 raise NotImplementedError("per-track R must be symmetric for the CUDA path")
             kw["R"] = up(Rt)
+        if Qt is not None:
+            kw["Q"] = up(Qt if order is None else Qt[:, order])
         if noise is not None:
             npred = np.zeros((max(N, 1), 4, T))
             nupd = np.zeros((M, 4, T))
@@ -700,7 +738,11 @@ class BatchedUKF:
         p, i, o = self._problem(b), self._inputs(b), self._outputs(res)
         res.filtered_by = id(b)
         with torch.cuda.device(b.device):
-            if res.nis is None:
+            if b.Q is not None:
+                innov = None if res.nis is None else C.byref(innovation_planes(res))
+                nat.check(self._lib.ste_ukf_forward_noise_f64(C.byref(p), C.byref(i), C.byref(self._noise(b)), innov, C.byref(o),
+                                                              nat.current_stream()))
+            elif res.nis is None:
                 nat.check(self._lib.ste_ukf_forward_f64(C.byref(p), C.byref(i), C.byref(o), nat.current_stream()))
             else:
                 nat.check(self._lib.ste_ukf_forward_innov_f64(C.byref(p), C.byref(i), C.byref(innovation_planes(res)), C.byref(o),
@@ -712,7 +754,16 @@ class BatchedUKF:
         self._check_filtered(b, res)
         p, i, o = self._problem(b), self._inputs(b), self._outputs(res)
         with torch.cuda.device(b.device):
-            nat.check(self._lib.ste_urtss_backward_f64(C.byref(p), C.byref(i), C.byref(o), nat.current_stream()))
+            if b.Q is not None:
+                nat.check(self._lib.ste_urtss_backward_noise_f64(C.byref(p), C.byref(i), C.byref(self._noise(b)), C.byref(o),
+                                                                 nat.current_stream()))
+            else:
+                nat.check(self._lib.ste_urtss_backward_f64(C.byref(p), C.byref(i), C.byref(o), nat.current_stream()))
+
+    @staticmethod
+    def _noise(b: TrackBatch) -> nat.SteNoiseN:
+        """The per-track process noise of ``b`` (the n = 4 passes take a per-track ``R`` in ``SteInputs.R_tracks``)."""
+        return nat.SteNoiseN(nat.ptr(b.Q), None)
 
     @staticmethod
     def _check_filtered(b: TrackBatch, res: TrackResults) -> None:
@@ -728,9 +779,12 @@ class BatchedUKF:
         resident on every SM together.  Bit-identical to ``forward(fwd_batch, fwd_res);
         backward(bwd_batch, bwd_res)``, and on B200 ~13 % slower than those two launches (two
         instruction streams per SM overflow the instruction cache).  The two result sets must be distinct.
-        The fused launch writes no innovation statistics: ``fwd_res`` with innovation planes raises ``ValueError``."""
+        The fused launch writes no innovation statistics and takes no per-track ``Q``: ``fwd_res`` with innovation planes,
+        or a tile with ``TrackBatch.Q``, raises ``ValueError``."""
         if fwd_res.nis is not None:
             raise ValueError("the fused pass writes no innovation statistics: filter tiles with innovation planes with forward()")
+        if fwd_batch.Q is not None or bwd_batch.Q is not None:
+            raise ValueError("the fused pass takes no per-track Q: run tiles with TrackBatch.Q with forward() / backward()")
         self._check_rows(fwd_batch)
         self._check_shapes(fwd_batch, fwd_res)
         self._check_shapes(bwd_batch, bwd_res, smoother=True)
@@ -764,6 +818,8 @@ class BatchedUKF:
             if fused:
                 raise ValueError("choose one of fused=True and partition=...")
             return self._run_many_partitioned(batches, results, partition)
+        if fused and any(b.Q is not None for b in batches):
+            raise ValueError("the fused pass takes no per-track Q: run tiles with TrackBatch.Q with forward() / backward()")
         if not fused:
             for b, r in zip(batches, results):
                 self.forward(b, r)
@@ -915,10 +971,12 @@ class BatchedUKF:
 
         Candidates whose ``R`` selects the position-only update and those that need the generic one are launched
         apart; each launch covers up to ``STE_MAX_CANDIDATES`` candidates (asynchronous on the current stream).  A tile
-        with its own per-track ``R`` raises ``ValueError``: the candidates replace it."""
+        with its own per-track ``R`` or ``Q`` raises ``ValueError``: the candidates replace them."""
         b.check()
         if b.R is not None:
             raise ValueError("TrackBatch.R: a tile with per-track measurement noise cannot be scored (the candidates replace R)")
+        if b.Q is not None:
+            raise ValueError("TrackBatch.Q: a tile with per-track process noise cannot be scored (the candidates replace Q)")
         if self.model.gating and b.noise_upd is not None:
             raise NotImplementedError("gating with measurement noise tapes (data-dependent draw count)")
         m = self.model

@@ -277,7 +277,7 @@ class TrackBatchN:
         matrix per ship, in the caller's (ship) order, checked as by :meth:`from_tracks`; column j gets the matrix of
         ship ``b.order[j]``."""
         b.check()
-        for name in ("P0", "R", "noise_pred", "noise_upd", "noise_bwd"):
+        for name in ("P0", "R", "Q", "noise_pred", "noise_upd", "noise_bwd"):
             if getattr(b, name) is not None:
                 raise ValueError(f"TrackBatch.{name} is 4-state data; build the five-state tile with TrackBatchN.from_tracks")
         dev, T, N = b.device, b.n_tracks, b.max_steps

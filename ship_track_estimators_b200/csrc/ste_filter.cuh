@@ -670,6 +670,9 @@ STE_DEV void urtss_moments_impl(const double (&xf)[4], const double *Q, double d
     }
 }
 
+// PER_Q: a clone of its own for callers whose Q lives in thread-local memory (a track's own Q), so that the clone
+// the other callers share keeps reading Q from the kernel parameters
+template <bool PER_Q = false>
 STE_COLD void urtss_moments_cold(const double *xf_in, const double *Q, double dt, double dtR, double sog_rate,
                                  double cog_rate, double *s1_out, double *Pb_out, Scratch sc) {
     double xf[4], s1[4], Pb[10];
@@ -682,6 +685,7 @@ STE_COLD void urtss_moments_cold(const double *xf_in, const double *Q, double dt
     for (int k = 0; k < 10; ++k) Pb_out[k] = Pb[k];
 }
 
+template <bool PER_Q = false>
 STE_DEV void urtss_moments(const double (&xf)[4], const double (&Pf)[10], const double *Q, double dt,
                            double sog_rate, double cog_rate, double (&s1)[4], double (&Pb)[10], int &status,
                            const Scratch &sc) {
@@ -698,7 +702,7 @@ STE_DEV void urtss_moments(const double (&xf)[4], const double (&Pf)[10], const 
         double xt[4], st[4], Pt[10];
 #pragma unroll
         for (int r = 0; r < 4; ++r) xt[r] = xf[r];
-        urtss_moments_cold(xt, Q, dt, dtR, sog_rate, cog_rate, st, Pt, sc);
+        urtss_moments_cold<PER_Q>(xt, Q, dt, dtR, sog_rate, cog_rate, st, Pt, sc);
 #pragma unroll
         for (int r = 0; r < 4; ++r) s1[r] = st[r];
 #pragma unroll

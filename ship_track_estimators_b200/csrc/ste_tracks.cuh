@@ -99,8 +99,11 @@ STE_DEV bool any_nonfinite(const double (&x)[4], const double (&P)[10]) {
 // SCORE: the scoring form - candidate `cand` of `sa` supplies Q and R, nothing is stored per step (no states, no
 // smoother tape, no gating planes: the robustification itself still runs) and the statistics of the updates are summed
 // in update order, then written once per track into the candidate's row of sa->scores.
+// PER_Q: the track's own process noise `q_track` (row-major 4x4, thread-local: forward_track loads it once, before the
+// time loop) replaces the launch's Q.  Every read of Q (the predict's moments, the scaling of the noise tape) goes through
+// Qm(), so such a track is bit-identical to a launch whose shared Q is its own.
 // ------------------------------------------------------------------------------------------ //
-template <bool POS_ONLY, bool GATING, bool INNOV = false, bool SCORE = false>
+template <bool POS_ONLY, bool GATING, bool INNOV = false, bool SCORE = false, bool PER_Q = false>
 struct ForwardTrack {
     const KernelArgs &a;
     const SteInnovations *iv;
@@ -122,15 +125,17 @@ struct ForwardTrack {
     bool consistent = true, upd_next = false;
     double loglik_sum = 0.0, nis_sum = 0.0;   // SCORE: sums over the updates so far
     int dof_sum = 0;
+    const double *const qt;   // PER_Q: the track's own Q
 
     STE_DEV ForwardTrack(const KernelArgs &args, int track, const Scratch &scratch, const SteInnovations *innov = nullptr,
-                         const KernelArgsScore *score = nullptr, int candidate = 0)
+                         const KernelArgsScore *score = nullptr, int candidate = 0, const double *q_track = nullptr)
         : a(args), iv(innov), sa(score), cand(candidate), t(track), sc(scratch), ld(args.prob.ld),
-          packed((args.prob.flags & STE_FLAG_PACKED_COV) != 0) {}
+          packed((args.prob.flags & STE_FLAG_PACKED_COV) != 0), qt(q_track) {}
 
-    // the process and measurement noise of the run: the tile's, or (SCORE) the candidate's
+    // the process and measurement noise of the run: the tile's, (SCORE) the candidate's or (PER_Q) the track's own Q
     STE_DEV const double *Qm() const {
         if constexpr (SCORE) return sa->Q[cand];
+        else if constexpr (PER_Q) return qt;
         else return a.prob.Q;
     }
     STE_DEV const double *Rm() const {
@@ -285,10 +290,16 @@ struct ForwardTrack {
     }
 };
 
-template <bool POS_ONLY, bool GATING, bool INNOV = false, bool SCORE = false>
+template <bool POS_ONLY, bool GATING, bool INNOV = false, bool SCORE = false, bool PER_Q = false>
 STE_DEV void forward_track(const KernelArgs &a, const int t, const Scratch &sc, const SteInnovations *iv = nullptr,
-                           const KernelArgsScore *sa = nullptr, int cand = 0) {
-    ForwardTrack<POS_ONLY, GATING, INNOV, SCORE> f(a, t, sc, iv, sa, cand);
+                           const KernelArgsScore *sa = nullptr, int cand = 0, const double *q_planes = nullptr) {
+    // PER_Q: the track's Q from the planes q_planes [16][ld] (the layout of SteInputs.P0 / R_tracks)
+    double Qt[PER_Q ? 16 : 1];
+    if constexpr (PER_Q) {
+#pragma unroll
+        for (int k = 0; k < 16; ++k) Qt[k] = q_planes[k * a.prob.ld + t];
+    }
+    ForwardTrack<POS_ONLY, GATING, INNOV, SCORE, PER_Q> f(a, t, sc, iv, sa, cand, PER_Q ? Qt : nullptr);
     f.begin();
 #if defined(STE_STEP_SYNC) && defined(__CUDA_ARCH__)
     // experiment: the warps of a block start every step together (instruction-cache locality); ragged lengths are safe,
@@ -306,6 +317,9 @@ STE_DEV void forward_track(const KernelArgs &a, const int t, const Scratch &sc, 
 
 // ------------------------------------------------------------------------------------------ //
 // Backward smoother: UnscentedKalmanFilter.rts_step (unscented.py:267-351).
+// PER_Q: the track's own Q (planes as in ForwardTrack) wherever the step reads Q - the scaling of the noise tape, the
+// speed / course blocks of the predicted covariance rebuilt from the tape, and the recomputed moments.  The forward pass
+// put the same track's Q into the tape's position block, so both passes must be given the same planes.
 // ------------------------------------------------------------------------------------------ //
 STE_DEV void prefetch_l2(const void *p) {
 #if defined(__CUDA_ARCH__)
@@ -315,6 +329,7 @@ STE_DEV void prefetch_l2(const void *p) {
 #endif
 }
 
+template <bool PER_Q = false>
 struct BackwardTrack {
     const KernelArgs &a;
     const int t;
@@ -326,9 +341,15 @@ struct BackwardTrack {
     // but step 0: state 0 is the PRIOR (kalman_filter.py:76-81), which the filter never predicted
     // from (it predicted from the prior's update), so its statistics do not exist.
     bool use_stats = false, bad = false;
+    const double *const qt;   // PER_Q: the track's own Q
 
-    STE_DEV BackwardTrack(const KernelArgs &args, int track, const Scratch &scratch)
-        : a(args), t(track), sc(scratch), ld(args.prob.ld), packed((args.prob.flags & STE_FLAG_PACKED_COV) != 0) {}
+    STE_DEV BackwardTrack(const KernelArgs &args, int track, const Scratch &scratch, const double *q_track = nullptr)
+        : a(args), t(track), sc(scratch), ld(args.prob.ld), packed((args.prob.flags & STE_FLAG_PACKED_COV) != 0), qt(q_track) {}
+
+    STE_DEV const double *Qm() const {
+        if constexpr (PER_Q) return qt;
+        else return a.prob.Q;
+    }
 
     STE_DEV void begin() {
         nt = a.in.n_steps ? min_(a.in.n_steps[t], a.prob.max_steps) : a.prob.max_steps;
@@ -369,7 +390,7 @@ struct BackwardTrack {
         if (a.in.noise_bwd) {
 #pragma unroll
             for (int r = 0; r < 4; ++r)
-                e[r] = a.in.noise_bwd[((int64_t)step * 4 + r) * ld + t] * sqrt(a.prob.Q[r * 5]);
+                e[r] = a.in.noise_bwd[((int64_t)step * 4 + r) * ld + t] * sqrt(Qm()[r * 5]);
         }
         bool done = false;
 #ifndef STE_BWD_PREFETCH
@@ -379,7 +400,7 @@ struct BackwardTrack {
         // pulling the NEXT step's 29 lines towards L2 now, without registers, turns its DRAM round trip into an L2 hit.
         if (STE_BWD_PREFETCH && use_stats && step > STE_BWD_PREFETCH) prefetch_stats_step(step - STE_BWD_PREFETCH);   // distance in steps
         if (use_stats && step > 0)
-            done = urtss_step_from_stats(mf, cf, packed, a.out.smooth_stats + ((int64_t)step * kStatsPlanes) * ld + t, ld, a.prob.Q,
+            done = urtss_step_from_stats(mf, cf, packed, a.out.smooth_stats + ((int64_t)step * kStatsPlanes) * ld + t, ld, Qm(),
                                          e, xs, Ps, status, sc, (unsigned)a.prob.reserved);
         if (!done) {
             double xf[4], s1[4], Pb[10];
@@ -401,7 +422,7 @@ struct BackwardTrack {
                         for (int j = i; j < 4; ++j) prefetch_l2(cf + (cov_plane(packed, i, j) - cov_planes(packed)) * ld);
                     prefetch_l2(a.in.dt + (int64_t)(step - 1) * ld + t);
                 }
-                urtss_moments(xf, Pf, a.prob.Q, dt, sr, cr, s1, Pb, status, sc);
+                urtss_moments<PER_Q>(xf, Pf, Qm(), dt, sr, cr, s1, Pb, status, sc);
             }
             double Pf[10];   // again (L2-resident) rather than held across the sigma-point loop
             load_cov(cf, ld, packed, Pf);
@@ -417,8 +438,14 @@ struct BackwardTrack {
     }
 };
 
-STE_DEV void backward_track(const KernelArgs &a, const int t, const Scratch &sc) {
-    BackwardTrack g(a, t, sc);
+template <bool PER_Q = false>
+STE_DEV void backward_track(const KernelArgs &a, const int t, const Scratch &sc, const double *q_planes = nullptr) {
+    double Qt[PER_Q ? 16 : 1];   // as forward_track
+    if constexpr (PER_Q) {
+#pragma unroll
+        for (int k = 0; k < 16; ++k) Qt[k] = q_planes[k * a.prob.ld + t];
+    }
+    BackwardTrack<PER_Q> g(a, t, sc, PER_Q ? Qt : nullptr);
     g.begin();
 #pragma unroll 1
     for (int step = g.nt - 1; step >= 0; --step) g.step(step);

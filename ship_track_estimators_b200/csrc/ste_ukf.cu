@@ -41,14 +41,25 @@ constexpr int kThreads = STE_THREADS;
 struct KernelArgsInnov : KernelArgs {
     SteInnovations innov;
 };
-template <bool INNOV> struct ForwardArgs { using type = KernelArgs; };
+// PER_Q: every track has its own process noise (ste_ukf_forward_noise_f64 / ste_urtss_backward_noise_f64).  The plane
+// pointer travels in a parameter block read only by the PER_Q instantiations, after everything the others read; `innov`
+// is read only by the forward instantiations that write the statistics.
+struct KernelArgsQ : KernelArgsInnov {
+    const double *Q_tracks;   // [16][ld] row-major per-track Q
+};
+template <bool INNOV, bool PER_Q = false> struct ForwardArgs { using type = KernelArgs; };
 template <> struct ForwardArgs<true> { using type = KernelArgsInnov; };
+template <bool INNOV> struct ForwardArgs<INNOV, true> { using type = KernelArgsQ; };
 
-template <bool POS_ONLY, bool GATING, bool INNOV = false>
-__global__ void __launch_bounds__(kThreads, STE_FWD_MIN_BLOCKS) ukf_forward_kernel(const __grid_constant__ typename ForwardArgs<INNOV>::type a) {
+template <bool POS_ONLY, bool GATING, bool INNOV = false, bool PER_Q = false>
+__global__ void __launch_bounds__(kThreads, STE_FWD_MIN_BLOCKS) ukf_forward_kernel(const __grid_constant__ typename ForwardArgs<INNOV, PER_Q>::type a) {
     extern __shared__ double scratch[];   // kScratchSlotsFwd * kThreads doubles (62 KB: opt-in size)
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
-    if constexpr (INNOV) {
+    if constexpr (PER_Q) {
+        if (t < a.prob.n_tracks)
+            forward_track<POS_ONLY, GATING, INNOV, false, true>(a, t, Scratch{scratch + threadIdx.x, kThreads}, INNOV ? &a.innov : nullptr,
+                                                                nullptr, 0, a.Q_tracks);
+    } else if constexpr (INNOV) {
         if (t < a.prob.n_tracks) forward_track<POS_ONLY, GATING, true>(a, t, Scratch{scratch + threadIdx.x, kThreads}, &a.innov);
     } else {
         if (t < a.prob.n_tracks) forward_track<POS_ONLY, GATING>(a, t, Scratch{scratch + threadIdx.x, kThreads});
@@ -65,13 +76,17 @@ __global__ void __launch_bounds__(kThreads, STE_FWD_MIN_BLOCKS) ukf_score_kernel
     if (t < a.prob.n_tracks) forward_track<POS_ONLY, GATING, false, true>(a, t, Scratch{scratch + threadIdx.x, kThreads}, nullptr, &a, blockIdx.y);
 }
 
-// TAPE: the launch has a statistics tape (same code either way; only the register budget differs)
-template <bool TAPE>
+// TAPE: the launch has a statistics tape (same code either way; only the register budget differs).  PER_Q: as the forward.
+template <bool TAPE, bool PER_Q = false>
 __global__ void __launch_bounds__(kThreads, TAPE ? STE_BWD_MIN_BLOCKS : STE_BWD_RECOMPUTE_MIN_BLOCKS)
-urtss_backward_kernel(const __grid_constant__ KernelArgs a) {
+urtss_backward_kernel(const __grid_constant__ typename ForwardArgs<false, PER_Q>::type a) {
     extern __shared__ double scratch[];   // kScratchSlotsBwd * kThreads doubles (46 KB: opt-in size)
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t < a.prob.n_tracks) backward_track(a, t, Scratch{scratch + threadIdx.x, kThreads});
+    if constexpr (PER_Q) {
+        if (t < a.prob.n_tracks) backward_track<true>(a, t, Scratch{scratch + threadIdx.x, kThreads}, a.Q_tracks);
+    } else {
+        if (t < a.prob.n_tracks) backward_track(a, t, Scratch{scratch + threadIdx.x, kThreads});
+    }
 }
 
 // Co-resident passes: ONE launch whose blocks take one of two roles - forward filter of tile a or backward smoother
@@ -890,20 +905,20 @@ static int validate_innovations(const SteInnovations *innov) {
 }
 
 extern "C++" {
-template <bool POS_ONLY, bool GATING, bool INNOV>
-static int launch_forward(const typename ForwardArgs<INNOV>::type &a, cudaStream_t s) {
+template <bool POS_ONLY, bool GATING, bool INNOV, bool PER_Q>
+static int launch_forward(const typename ForwardArgs<INNOV, PER_Q>::type &a, cudaStream_t s) {
     const dim3 grid((a.prob.n_tracks + kThreads - 1) / kThreads), block(kThreads);
     const size_t smem = sizeof(double) * kScratchSlotsFwd * kThreads;
-    if (cudaFuncSetAttribute(ukf_forward_kernel<POS_ONLY, GATING, INNOV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+    if (cudaFuncSetAttribute(ukf_forward_kernel<POS_ONLY, GATING, INNOV, PER_Q>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
         return check_launch("cudaFuncSetAttribute(ukf_forward_kernel)");
-    ukf_forward_kernel<POS_ONLY, GATING, INNOV><<<grid, block, smem, s>>>(a);
+    ukf_forward_kernel<POS_ONLY, GATING, INNOV, PER_Q><<<grid, block, smem, s>>>(a);
     return check_launch("ukf_forward_kernel");
 }
 
-template <bool INNOV>
-static int launch_forward(bool pos, bool gating, const typename ForwardArgs<INNOV>::type &a, cudaStream_t s) {
-    if (pos) return gating ? launch_forward<true, true, INNOV>(a, s) : launch_forward<true, false, INNOV>(a, s);
-    return gating ? launch_forward<false, true, INNOV>(a, s) : launch_forward<false, false, INNOV>(a, s);
+template <bool INNOV, bool PER_Q = false>
+static int launch_forward(bool pos, bool gating, const typename ForwardArgs<INNOV, PER_Q>::type &a, cudaStream_t s) {
+    if (pos) return gating ? launch_forward<true, true, INNOV, PER_Q>(a, s) : launch_forward<true, false, INNOV, PER_Q>(a, s);
+    return gating ? launch_forward<false, true, INNOV, PER_Q>(a, s) : launch_forward<false, false, INNOV, PER_Q>(a, s);
 }
 }  // extern "C++"
 
@@ -923,6 +938,29 @@ int ste_ukf_forward_innov_f64(const SteProblem *prob, const SteInputs *in, const
     static_cast<KernelArgs &>(a) = kernel_args(prob, in, out);
     a.innov = *innov;
     return launch_forward<true>(pos, gating, a, s);
+}
+
+// the n = 4 passes' per-track noise: Q_tracks only (a per-track R travels in SteInputs.R_tracks)
+static int validate_noise4(const SteNoiseN *noise) {
+    if (noise && noise->R_tracks)
+        return fail(STE_ERR_INVALID_ARG, "n = 4: a per-track R travels in SteInputs.R_tracks, not SteNoiseN.R_tracks");
+    return STE_OK;
+}
+
+int ste_ukf_forward_noise_f64(const SteProblem *prob, const SteInputs *in, const SteNoiseN *noise, const SteInnovations *innov,
+                              SteOutputs *out, void *stream) {
+    if (int rc = validate_noise4(noise)) return rc;
+    if (!noise || !noise->Q_tracks) return ste_ukf_forward_innov_f64(prob, in, innov, out, stream);
+    if (int rc = validate_forward(prob, in, out)) return rc;
+    if (int rc = validate_innovations(innov)) return rc;
+    if (prob->n_tracks == 0) return STE_OK;
+    const bool gating = (prob->flags & STE_FLAG_GATING) != 0, pos = position_only(*prob);
+    KernelArgsQ a{};
+    static_cast<KernelArgs &>(a) = kernel_args(prob, in, out);
+    if (innov) a.innov = *innov;
+    a.Q_tracks = noise->Q_tracks;
+    cudaStream_t s = (cudaStream_t)stream;
+    return innov ? launch_forward<true, true>(pos, gating, a, s) : launch_forward<false, true>(pos, gating, a, s);
 }
 
 // ------------------------------------------------------------------------------------------ //
@@ -992,17 +1030,35 @@ int ste_ukf_score_f64(const SteProblem *prob, const SteInputs *in, const SteCand
     return gating ? launch_score<false, true>(a, cand->n_cand, s) : launch_score<false, false>(a, cand->n_cand, s);
 }
 
+extern "C++" {
+template <bool PER_Q>
+static int launch_backward(const typename ForwardArgs<false, PER_Q>::type &a, cudaStream_t s) {
+    const dim3 grid((a.prob.n_tracks + kThreads - 1) / kThreads), block(kThreads);
+    const size_t smem = sizeof(double) * kScratchSlotsBwd * kThreads;
+    auto kernel = a.out.smooth_stats ? urtss_backward_kernel<true, PER_Q> : urtss_backward_kernel<false, PER_Q>;
+    if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+        return check_launch("cudaFuncSetAttribute(urtss_backward_kernel)");
+    kernel<<<grid, block, smem, s>>>(a);
+    return check_launch("urtss_backward_kernel");
+}
+}  // extern "C++"
+
 int ste_urtss_backward_f64(const SteProblem *prob, const SteInputs *in, SteOutputs *out, void *stream) {
     if (int rc = validate_backward(prob, in, out)) return rc;
     if (prob->n_tracks == 0) return STE_OK;
-    const KernelArgs a = kernel_args(prob, in, out);
-    const dim3 grid((prob->n_tracks + kThreads - 1) / kThreads), block(kThreads);
-    const size_t smem = sizeof(double) * kScratchSlotsBwd * kThreads;
-    auto kernel = out->smooth_stats ? urtss_backward_kernel<true> : urtss_backward_kernel<false>;
-    if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-        return check_launch("cudaFuncSetAttribute(urtss_backward_kernel)");
-    kernel<<<grid, block, smem, (cudaStream_t)stream>>>(a);
-    return check_launch("urtss_backward_kernel");
+    return launch_backward<false>(kernel_args(prob, in, out), (cudaStream_t)stream);
+}
+
+int ste_urtss_backward_noise_f64(const SteProblem *prob, const SteInputs *in, const SteNoiseN *noise, SteOutputs *out,
+                                 void *stream) {
+    if (int rc = validate_noise4(noise)) return rc;
+    if (!noise || !noise->Q_tracks) return ste_urtss_backward_f64(prob, in, out, stream);
+    if (int rc = validate_backward(prob, in, out)) return rc;
+    if (prob->n_tracks == 0) return STE_OK;
+    KernelArgsQ a{};
+    static_cast<KernelArgs &>(a) = kernel_args(prob, in, out);
+    a.Q_tracks = noise->Q_tracks;
+    return launch_backward<true>(a, (cudaStream_t)stream);
 }
 
 extern "C++" {

@@ -4,11 +4,16 @@ Every candidate is scored on the device by ``BatchedUKF.score`` / ``BatchedUKFN.
 (candidate, track) pair that sums the Gaussian log-likelihood of each fix under its one-step prediction
 (``performance_metrics.innovation_metrics`` of a run with that candidate, without the run's states).  The largest
 summed log-likelihood is the maximum-likelihood choice, for the whole fleet or for each track on its own; the per-track
-choice is what ``TrackBatchN.from_tracks(Q=..., R=...)`` takes.
+choice is what ``TrackBatchN.from_tracks(Q=..., R=...)`` takes at n = 5, and ``TrackBatch.from_tracks(Q=..., R=...)`` or
+``TrackBatch.with_noise(Q=..., R=...)`` at n = 4.  At n = 4 a per-track ``R`` selects the generic update (as
+``TrackBatch.R`` always does), so a grid over ``Q`` alone keeps a position-only filter on its fast update.
 
     grid = noise_grid(Q, R, q_scales=(0.5, 1, 2), r_scales=(0.25, 0.5, 1, 2, 4))
     fit = fit_noise(engine, TrackBatchN.fleet_tiles(tracks, dts), grid, per="track")
     tiles = TrackBatchN.fleet_tiles(tracks, dts, Q=fit["Q"], R=fit["R"])
+
+    fit = fit_noise(ukf, tile, noise_grid(Q, R, q_scales=(0.25, 0.5, 1, 2, 4), r_scales=(1,)), per="track")   # n = 4
+    res = ukf.run(tile.with_noise(Q=fit["Q"]))
 """
 from __future__ import annotations
 
@@ -60,7 +65,9 @@ def fit_noise(engine, tiles, candidates: Sequence, per: str = "fleet") -> Dict[s
     Returns, in the caller's track order:
       ``loglik``   ``[C]`` fleet sums (``per="fleet"``) or the ``[C][n_tracks]`` table (``per="track"``);
       ``best``     the chosen candidate index, or one per track;
-      ``Q``, ``R`` the chosen matrices, or one list entry per track (what ``from_tracks(Q=, R=)`` takes);
+      ``Q``, ``R`` the chosen matrices, or one list entry per track (what ``TrackBatchN.from_tracks(Q=, R=)`` takes
+                   at n = 5, and ``TrackBatch.from_tracks(Q=, R=)`` / ``TrackBatch.with_noise(Q=, R=)`` at n = 4, where a
+                   per-track ``R`` selects the generic update);
       ``excluded`` the tracks with a non-finite score under some candidate (left out of the fleet sums).
     """
     tiles = [tiles] if hasattr(tiles, "n_tracks") else list(tiles)
